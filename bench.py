@@ -13,7 +13,10 @@ enabled, reference batch composition of 31 chains per early-exit group) of 4096 
 `precisions`: both MLP arithmetics measured the same way; the top-level `value` / `dtype` are the fp32-accurate path's.
 `parity_checked`: one early-exit group of the timed launch re-run on the CPU oracle after the timed region.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|bf16]
+`--dump-outputs DIR`: the sampled assignments, SAT flags and latch steps of the last timed run as .npy files; the inputs
+(formula, weights, Philox seeds) depend only on the arguments, so two builds can be compared output for output.
+
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|bf16] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -324,9 +327,32 @@ def parity_check(ctx, precision, unit, n, clauses, batch, chains, wts, chain_off
                         inside.mean() >= 0.99 and ((got > 0) == (want > 0))[same].mean() >= 0.97))}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, n_vars, chain_offset, packed, is_sat, latch_step, sat_any_step):
+    """Write what dsat_sample_fetch hands a caller after a run as DIR/<name>.npy: the sampled assignment of every chain
+    (0/1 per variable, x1 first), its SAT flag, the denoising step at which it was first satisfied (-1 = never) and the
+    any-step SAT flag, all float32, plus the global index of each chain (float64).  Above DUMP_BYTES in all, a fixed
+    seeded sample of the chains is written instead, so that two builds can still be compared chain for chain."""
+    chains = len(packed)
+    rows = np.arange(chains)
+    per_chain = 4 * (n_vars + 3) + 8
+    if chains * per_chain > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(chains, DUMP_BYTES // per_chain, replace=False))
+    bits = np.unpackbits(packed[rows].astype("<u8").view(np.uint8).reshape(len(rows), -1), axis=1, bitorder="little")
+    arrays = {"assignment": bits[:, :n_vars].astype(np.float32), "is_sat": is_sat[rows].astype(np.float32),
+              "latch_step": latch_step[rows].astype(np.float32), "sat_any_step": sat_any_step[rows].astype(np.float32),
+              "chain": (chain_offset + rows).astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def measure_precision(ctx, precision, args, world, rank, local_rank, unit, batch, chains, chain_offset, barrier, dist, torch, pk):
     """`value` of one precision: W warm-up + K timed whole reverse-diffusion runs, everything resident, CUDA events on the
-    launching stream, max over ranks; then (rank 0) the per-class device time of four rounds for the roofline."""
+    launching stream, max over ranks; then (rank 0) the per-class device time of four rounds for the roofline.  With
+    --dump-outputs, rank 0 writes the headline precision's results of the last timed run."""
     from diffusionsat_b200 import _lib
     ctx.set_precision(_lib.PRECISIONS[precision])
     ctx.set_graph(unit, chains=chains, group_graphs=batch)
@@ -346,6 +372,8 @@ def measure_precision(ctx, precision, args, world, rank, local_rank, unit, batch
     launches = ctx.launch_count() - launches0
     barrier()
     clock_info = clocks.stop()
+    if args.dump_outputs and precision == args.precision and rank == 0:
+        dump_outputs(args.dump_outputs, unit.n_vars, chain_offset, *ctx.sample_fetch())
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -718,7 +746,14 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-message-pass", action="store_true")
     ap.add_argument("--skip-trained", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="n100: write the results of the last timed run (headline precision) as DIR/<name>.npy; under "
+                         "several GPUs only rank 0's chains (chain.npy holds their global indices)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "n100"):
+        ap.error("--dump-outputs writes the outputs of the n100 config of --impl ours")
     # Only the JSON line may reach stdout: libraries (NCCL's version banner under torchrun, for one) write there too, so
     # file descriptor 1 points at stderr while the benchmark runs and is restored for the final print.
     sys.stdout.flush()

@@ -4,8 +4,6 @@ import ctypes
 import os
 import re
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -36,12 +34,15 @@ def test_library_exports_every_declared_symbol(dsat_lib):
 
 
 def test_no_cpu_fallback_without_gpu(dsat_lib):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    from diffusionsat_b200 import _lib
-    with pytest.raises(_lib.DsatError, match="no CPU fallback"):
-        _lib.Context(0)
+    """Creating a context without a CUDA device raises; on a machine with GPUs the child process is shown none."""
+    import subprocess
+    import sys
+    code = ("from diffusionsat_b200 import _lib\n"
+            "try:\n    _lib.Context(0)\nexcept _lib.DsatError as exc:\n    print(exc)\n")
+    proc = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                          stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=300)
+    assert proc.returncode == 0, proc.stderr[-2000:]
+    assert "no CPU fallback" in proc.stdout
 
 
 def test_product_code_never_imports_the_oracle():

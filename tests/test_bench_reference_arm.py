@@ -46,3 +46,29 @@ def test_per_kernel_roofline_of_a_recorded_bench_line():
                                      1369.7, 6552.3)
     assert set(bf16) == {"query_out", "lit_3", "clause_2", "update_3", "output_2", "pairnorm_clause", "pairnorm_var"}
     assert bench.per_kernel_roofline({}, n_rows, m_rows, "fp32", 1369.7, 6552.3) == {}
+
+
+def test_dump_outputs_unpacks_the_packed_assignments(tmp_path, monkeypatch):
+    """--dump-outputs: packed 64-bit words (x1 = bit 0 of word 0) come out as one 0/1 float32 row per chain; above the size
+    cap the same seeded chains are written every time, with their global indices."""
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(3)
+    chains, n_vars = 300, 100
+    bits = rng.integers(0, 2, (chains, n_vars))
+    packed = np.zeros((chains, 2), dtype=np.uint64)
+    for v in range(n_vars):
+        packed[:, v // 64] |= bits[:, v].astype(np.uint64) << np.uint64(v % 64)
+    latch = rng.integers(-1, 32, chains).astype(np.int32)
+    outs = (rng.integers(0, 2, chains).astype(np.uint8), latch, (latch >= 0).astype(np.uint8))
+    bench.dump_outputs(str(tmp_path / "all"), n_vars, 0, packed, *outs)
+    got = {f[:-4]: np.load(str(tmp_path / "all" / f)) for f in os.listdir(str(tmp_path / "all"))}
+    assert set(got) == {"assignment", "is_sat", "latch_step", "sat_any_step", "chain"}
+    assert got["assignment"].dtype == np.float32 and np.array_equal(got["assignment"], bits)
+    assert np.array_equal(got["latch_step"], latch) and np.array_equal(got["chain"], np.arange(chains))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * (4 * (n_vars + 3) + 8))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), n_vars, 1000, packed, *outs)
+    chain = np.load(str(tmp_path / "a" / "chain.npy"))
+    assert len(chain) == 100 and np.array_equal(chain, np.load(str(tmp_path / "b" / "chain.npy")))
+    assert np.array_equal(np.load(str(tmp_path / "a" / "assignment.npy")), bits[chain.astype(np.int64) - 1000])

@@ -282,3 +282,32 @@ def test_batch_tensors_match_the_reference_create_adj_matrices(tag):
     back = G.unit_graph_from_reference_coo(idx, shp, vg, cg)
     for name in ("cl_rowptr", "cl_lit", "lit_rowptr", "lit_clause", "var_seg", "clause_seg"):
         np.testing.assert_array_equal(getattr(back, name), getattr(union, name), err_msg=name)
+
+
+def test_host_mirrors_match_the_stored_differential_cases():
+    """A fixed, seeded draw from the input grammars of the differential fuzz tests (DIMACS token soup, VariableAssignment
+    cases, chi-square dict pairs with differing key sets or sums) and the outcome of every case, so that those edge cases
+    are checked where the original project is not at hand.  The file's `source` says which implementation produced the
+    outcomes (make_differential_golden.py: the original's classes where DIFFUSIONSAT_REFERENCE is set, else the mirrors)."""
+    import importlib.util
+    import math
+    from diffusionsat_b200.uniformity import chi_square_likelihood
+    here = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    spec = importlib.util.spec_from_file_location("make_differential_golden", os.path.join(here, "make_differential_golden.py"))
+    gen = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(gen)
+    gold = json.load(open(os.path.join(here, "differential_golden.json")))
+    assert gold["cases"] == json.loads(json.dumps(gen.draw_cases()))          # the stored inputs are the generator's draw
+    got = gen.outcomes(DimacsFile, VariableAssignment, chi_square_likelihood, gold["cases"])
+    want = gold["outcomes"]
+    for kind in ("dimacs", "assignment"):
+        for case, g, w in zip(gold["cases"][kind], got[kind], want[kind]):
+            assert json.loads(json.dumps(g)) == w, (kind, case)
+    for case, g, w in zip(gold["cases"]["chi_square"], got["chi_square"], want["chi_square"]):
+        assert g[0] == w[0], case
+        if g[0] == "error" or w[1] is None or g[1] is None:
+            assert g[1] == w[1], case
+        else:
+            assert math.isclose(g[1], w[1], rel_tol=1e-12, abs_tol=1e-300), case
+    assert {k: len(v) for k, v in want.items()} == {k: len(v) for k, v in got.items()} == {"dimacs": 300, "assignment": 120,
+                                                                                           "chi_square": 120}
