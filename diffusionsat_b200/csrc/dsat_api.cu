@@ -151,11 +151,6 @@ struct dsat_ctx {
     bool use_smem_gather = true;
     // fp32-accurate tensor-core path (dsat_mlp_x3.cuh): MLP inputs live as hi/lo bf16 planes [2][rows][ld]
     DevBuf<__nv_bfloat16> VROWp, CROWp, SPREp, H1p, H2p;
-    // layer-per-launch variants of the clause and update MLPs (hidden planes through HBM, deep rings instead of a hidden
-    // region in shared memory): clause 1, clause 2, update 1, update 2, update 3
-    DevBuf<__nv_bfloat16> CHp, U1p, U2p;
-    x3::X3Mlp x3s[5];
-    bool split_clause = false, split_update = false;
     DevBuf<__nv_bfloat16> wx[12];       // stacked hi/lo K-major weights [2N, K64] per reference layer
     int wx_k64[12] = {0}, wx_n[12] = {0};
     x3::X3Mlp x3[7];                    // query, lit layer 1, lit layer 2, lit layer 3, clause, update, output
@@ -495,7 +490,6 @@ void release_buffers(dsat_ctx* c) {
     c->O1b.drop();
     c->has_tc_buffers = false;
     c->VROWp.drop(); c->CROWp.drop(); c->SPREp.drop(); c->H1p.drop(); c->H2p.drop();
-    c->CHp.drop(); c->U1p.drop(); c->U2p.drop();
     c->has_x3_buffers = false;
 #endif
     c->has_buffers = false;
@@ -518,7 +512,6 @@ void free_buffers(dsat_ctx* c) {
     c->O1b.release();
     c->has_tc_buffers = false;
     c->VROWp.release(); c->CROWp.release(); c->SPREp.release(); c->H1p.release(); c->H2p.release();
-    c->CHp.release(); c->U1p.release(); c->U2p.release();
     c->has_x3_buffers = false;
 #endif
     c->has_buffers = false;
@@ -627,9 +620,8 @@ int ensure_x3_buffers(dsat_ctx* c) {
         }
         for (; i < x3::MAX_LAYERS; ++i) f.map_w[i] = f.map_w[0];
         if (getenv("DSAT_PLAN_LOG"))
-            fprintf(stderr, "[dsat] x3 mlp %d: smem %d B, hidden blocks 2 x %d, input ring %d, weight ring %d x %d B, epilogue warps %d, "
-                    "staging in hidden %d, cta pair %d, groups %d\n", which, f.smem_bytes, p.h_blocks, p.a_slots, p.w_slots, p.w_slot_bytes,
-                    p.epi_warps, p.stage_in_h, p.pair, p.n_groups);
+            fprintf(stderr, "[dsat] x3 mlp %d: smem %d B, input ring %d, weight ring %d x %d B, epilogue warps %d, cta pair %d, groups %d\n",
+                    which, f.smem_bytes, p.a_slots, p.w_slots, p.w_slot_bytes, p.epi_warps, p.pair, p.n_groups);
         return true;
     };
     const size_t vplane = Nt * c->ldv(), cplane = Mt * c->ldc(), splane = Nt * F, hplane = Nt * c->HL;
@@ -656,44 +648,6 @@ int ensure_x3_buffers(dsat_ctx* c) {
     else ok = false;
     ok = ok && build(XO, c->SPREp.p, splane, c->Nt, F, F,
                      {{10, OP_O1, 0, tc::TC_LRELU}, {11, OP_O2, 0, tc::TC_LINEAR}}, 1, x3::OUT_F32, c->LOGITS.p, nullptr, DSAT_LOGIT_PAD);
-    {   // Layer-per-launch variants (DSAT_X3_SPLIT=<mask>: bit 0 clause MLP, bit 1 update MLP; default 1).  The whole-MLP
-        // clause kernel keeps 128 KB of hidden hi/lo planes in shared memory and has 96 KB of rings left for 192 KB of input
-        // and 266 KB of weights per tile: its issue warp waits half of the time.  As two single-layer launches the hidden
-        // planes make a round trip through HBM (+2.9 GB per round) but both launches run at 82-87 % of the measured copy
-        // rate: 0.73 + 0.60 ms against 1.46 ms.  The update MLP gains nothing (0.53 against 0.52 ms) and stays fused.
-        static const int split_mask = getenv("DSAT_X3_SPLIT") ? atoi(getenv("DSAT_X3_SPLIT")) : 1;
-        c->split_clause = c->split_update = false;
-        if (ok && (split_mask & 1)) {
-            const size_t chplane = Mt * c->HC;
-            CK_CUDA(c, c->CHp.alloc(2 * chplane));
-            x3::X3Mlp keep_c = c->x3[XC];
-            bool k = build(XC, c->CROWp.p, cplane, c->Mt, F + 2 * Q, c->ldc(), {{5, OP_C1, 0, tc::TC_LRELU}}, 1, x3::OUT_SPLIT,
-                           c->CHp.p, c->CHp.p + chplane, c->HC);
-            c->x3s[0] = c->x3[XC];
-            k = k && build(XC, c->CHp.p, chplane, c->Mt, c->HC, c->HC, {{6, OP_C2, 0, tc::TC_LINEAR}}, 1, x3::OUT_F32,
-                           c->COUT.p, nullptr, Q + F);
-            c->x3s[1] = c->x3[XC];
-            c->x3[XC] = keep_c;
-            c->split_clause = k;
-        }
-        if (ok && (split_mask & 2)) {
-            const size_t uplane = Nt * c->HU;
-            CK_CUDA(c, c->U1p.alloc(2 * uplane));
-            CK_CUDA(c, c->U2p.alloc(2 * uplane));
-            x3::X3Mlp keep_u = c->x3[XU];
-            bool k = build(XU, c->VROWp.p, vplane, c->Nt, F + DSAT_AUX_PAD + 3 * Q, c->ldv(), {{7, OP_U1, 0, tc::TC_LRELU}}, 1,
-                           x3::OUT_SPLIT, c->U1p.p, c->U1p.p + uplane, c->HU);
-            c->x3s[2] = c->x3[XU];
-            k = k && build(XU, c->U1p.p, uplane, c->Nt, c->HU, c->HU, {{8, OP_U2, 0, tc::TC_LRELU}}, 1, x3::OUT_SPLIT,
-                           c->U2p.p, c->U2p.p + uplane, c->HU);
-            c->x3s[3] = c->x3[XU];
-            k = k && build(XU, c->U2p.p, uplane, c->Nt, c->HU, c->HU, {{9, OP_U3, 0, tc::TC_LINEAR}}, 1, x3::OUT_F32,
-                           c->UOUT.p, nullptr, F);
-            c->x3s[4] = c->x3[XU];
-            c->x3[XU] = keep_u;
-            c->split_update = k;
-        }
-    }
     c->x3_ready = ok;
     if (!ok) { c->err = "the fp32-accurate tensor-core path supports feature_maps = query_maps <= 128 (hidden widths <= 256 or 512)"; return DSAT_ERR_UNSUPPORTED; }
     c->has_x3_buffers = true;
@@ -1068,13 +1022,7 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
     // clause_update MLP                                                          (:258-261)
     if (x3p) {
 #ifdef DSAT_WITH_TCGEN05
-        if (c->split_clause) {
-            for (int k = 0; k < 2; ++k) {
-                prof_mark(c, k == 0 ? OP_C1 : OP_C2);
-                CK_CUDA(c, x3::launch_x3(c->x3s[k], c->device, c->sm_count, c->stream));
-                c->launches++;
-            }
-        } else if ((rc = run_x3(c, XC, OP_C2))) return rc;
+        if ((rc = run_x3(c, XC, OP_C2))) return rc;
 #endif
     } else if (!tcp) {
         if ((rc = run_linear(c, OP_C1, c->CROW.p, ldc, c->CH.p, c->HC, Mt, EPI_LRELU))) return rc;
@@ -1154,13 +1102,7 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
     // update_gate MLP                                                            (:277-278)
     if (x3p) {
 #ifdef DSAT_WITH_TCGEN05
-        if (c->split_update) {
-            for (int k = 0; k < 3; ++k) {
-                prof_mark(c, k == 0 ? OP_U1 : k == 1 ? OP_U2 : OP_U3);
-                CK_CUDA(c, x3::launch_x3(c->x3s[2 + k], c->device, c->sm_count, c->stream));
-                c->launches++;
-            }
-        } else if ((rc = run_x3(c, XU, OP_U3))) return rc;
+        if ((rc = run_x3(c, XU, OP_U3))) return rc;
 #endif
     } else if (!tcp) {
         if ((rc = run_linear(c, OP_U1, c->VROW.p, ldv, c->U1.p, c->HU, Nt, EPI_LRELU))) return rc;
@@ -2057,7 +1999,7 @@ int dsat_profile_fused(dsat_ctx* c, int which, long long* counters16) {
     return DSAT_ERR_UNSUPPORTED;
 #else
     CK_CUDA(c, cudaSetDevice(c->device));
-    if (use_x3(c)) {    // the seven x3 launches (query, lit 1, lit 2, lit 3, clause, update, output): 8 counters, see dsat_mlp_x3.cuh
+    if (use_x3(c)) {    // the seven x3 launches (query, lit 1, lit 2, lit 3, clause, update, output): 9 counters, see dsat_mlp_x3.cuh
         int rc = ensure_x3_buffers(c);
         if (rc) return rc;
         DevBuf<long long> d;
@@ -2376,22 +2318,8 @@ int dsat_debug_mlp(dsat_ctx* c, int which) {
         switch (which) {
             case 0: rc = run_x3(c, XQ, OP_Q2); break;
             case 1: rc = run_x3(c, XL1, OP_V1); if (!rc) rc = run_x3(c, XL2, OP_L2); if (!rc) rc = run_x3(c, XL3, OP_L3); break;
-            case 2:
-                if (c->split_clause) {
-                    for (int k = 0; k < 2 && !rc; ++k) {
-                        CK_CUDA(c, x3::launch_x3(c->x3s[k], c->device, c->sm_count, c->stream));
-                        c->launches++;
-                    }
-                } else rc = run_x3(c, XC, OP_C2);
-                break;
-            case 3:
-                if (c->split_update) {
-                    for (int k = 0; k < 3 && !rc; ++k) {
-                        CK_CUDA(c, x3::launch_x3(c->x3s[2 + k], c->device, c->sm_count, c->stream));
-                        c->launches++;
-                    }
-                } else rc = run_x3(c, XU, OP_U3);
-                break;
+            case 2: rc = run_x3(c, XC, OP_C2); break;
+            case 3: rc = run_x3(c, XU, OP_U3); break;
             default: rc = run_x3(c, XO, OP_O2); break;
         }
     } else if (use_tc(c) && c->precision == DSAT_BF16 && c->fused_ready && c->use_fused) {

@@ -233,6 +233,57 @@ __device__ __forceinline__ void umma_bf16_kblock_elect_cg2(uint32_t tmem_d, uint
         "@q tcgen05.mma.cta_group::2.kind::f16 [%0], a3, b3, %3, t;\n"
         "}\n" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate_first) : "memory");
 }
+// A operand in TENSOR memory (the tcgen05.mma [a_tmem] form; B from shared memory as above): 16-bit A elements sit two
+// per 32-bit column, row r of A in lane r (cta_group::2: each CTA's 128 rows in its own tensor memory, same column).  The
+// x3 hidden epilogue stores the hi and lo planes interleaved per 32 K values: columns [32j, 32j+16) hold the hi plane of
+// K in [32j, 32j+32), [32j+16, 32j+32) the lo plane.  So k-step k of a plane starts at column 32 (k/2) + 8 (k%2), and
+// the four k-steps of a K block of 64 at +0, +8, +32, +40 from the block's column 64 kb.
+__device__ __forceinline__ uint32_t tmem_a_kstep(int k) { return (uint32_t)(32 * (k >> 1) + 8 * (k & 1)); }
+template <bool PAIR>
+__device__ __forceinline__ void umma_bf16_ts_elect(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (PAIR) {
+        asm volatile(
+            "{\n"
+            ".reg .pred p, q;\n"
+            "setp.ne.b32 p, %4, 0;\n"
+            "elect.sync _|q, 0xffffffff;\n"
+            "@q tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n"
+            "}\n" ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
+    } else {
+        asm volatile(
+            "{\n"
+            ".reg .pred p, q;\n"
+            "setp.ne.b32 p, %4, 0;\n"
+            "elect.sync _|q, 0xffffffff;\n"
+            "@q tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n"
+            "}\n" ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
+    }
+}
+// one full K block (four k-steps) of the [a_tmem] form, one election
+template <bool PAIR>
+__device__ __forceinline__ void umma_bf16_ts_kblock_elect(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
+                                                          uint32_t accumulate_first) {
+#define DSAT_UMMA_TS_KBLOCK(CG)                                                              \
+    "{\n"                                                                                    \
+    ".reg .pred p, q, t;\n"                                                                  \
+    ".reg .b32 a1, a2, a3;\n"                                                                \
+    ".reg .b64 b1, b2, b3;\n"                                                                \
+    "setp.ne.b32 p, %4, 0;\n"                                                                \
+    "setp.eq.b32 t, 0, 0;\n"                                                                 \
+    "add.u32 a1, %1, 8;\n add.u32 a2, %1, 32;\n add.u32 a3, %1, 40;\n"                       \
+    "add.s64 b1, %2, 2;\n add.s64 b2, %2, 4;\n add.s64 b3, %2, 6;\n"                         \
+    "elect.sync _|q, 0xffffffff;\n"                                                          \
+    "@q tcgen05.mma.cta_group::" CG ".kind::f16 [%0], [%1], %2, %3, p;\n"                    \
+    "@q tcgen05.mma.cta_group::" CG ".kind::f16 [%0], [a1], b1, %3, t;\n"                    \
+    "@q tcgen05.mma.cta_group::" CG ".kind::f16 [%0], [a2], b2, %3, t;\n"                    \
+    "@q tcgen05.mma.cta_group::" CG ".kind::f16 [%0], [a3], b3, %3, t;\n"                    \
+    "}\n"
+    if constexpr (PAIR)
+        asm volatile(DSAT_UMMA_TS_KBLOCK("2") ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate_first) : "memory");
+    else
+        asm volatile(DSAT_UMMA_TS_KBLOCK("1") ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate_first) : "memory");
+#undef DSAT_UMMA_TS_KBLOCK
+}
 __device__ __forceinline__ void tcgen05_commit_elect(uint64_t* bar) {
     asm volatile(
         "{\n"

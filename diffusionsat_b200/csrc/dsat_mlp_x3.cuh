@@ -14,10 +14,12 @@
 //           weights     : per layer a stacked K-major array [2 N, K64] (rows [0,N) = hi, [N,2N) = lo)
 //   shared  input ring  : 16 KB blocks; a K block of the input occupies two consecutive slots (hi, lo)
 //           weight ring : slots of N x 64 (PAIR: N/2 x 64) bf16; per K block first W_hi (multiplies A_hi and A_lo), then W_lo
-//           hidden      : the activations between layers never leave the SM: the epilogue warps write them as hi/lo
-//                         planes of K-major SWIZZLE_128B blocks that the next layer's MMAs read as A operand
 //   tensor  memory      : two accumulators of <= 256 columns; consecutive (tile, layer) steps alternate between them,
 //                         so the final epilogue of a tile drains while the next tile's first layer accumulates
+//           hidden      : the activations between layers never leave tensor memory: the epilogue warps read a hidden
+//                         accumulator, add bias + leaky relu, split, and store the hi/lo planes back into the columns they
+//                         read (tc::tmem_a_kstep has the layout); the next layer's MMAs take them as A operand from there
+//                         and accumulate into the other half
 //   warps               : 0 = TMA producer, 1 = MMA issuer (+ TMEM alloc), 2.. = 4 or 8 epilogue warps
 // A single wide layer (N > 256, the 512-wide layers of lit_query) runs as `n_groups` column groups of 256: the work
 // unit is (tile, group) and its output goes to global memory as fp32 rows or as hi/lo planes for the next launch.
@@ -31,10 +33,14 @@ constexpr int BLOCK_M = 128;
 constexpr int BLOCK_K = 64;
 constexpr int BLK_BYTES = BLOCK_M * BLOCK_K * 2;     // 16 KB
 constexpr int MAX_LAYERS = 3;
-constexpr int MAX_RING = 8;
+constexpr int MAX_RING = 12;                          // a whole tile of the clause MLP's input: 6 K blocks x 2 planes
 constexpr int TMEM_COLS = 512;
 constexpr int STAGE_ROW = 128 + 16;
-constexpr int BAR_BYTES = 512;
+// barrier block: 4 rings of mbarriers, tmem_full[2], tmem_empty[2], h_full[2], the TMEM address; then the early-exit bits
+constexpr int SKIP_UNITS = 1024;                      // units per CTA up to which early-exit skipping is evaluated
+constexpr int SKIP_OFF = 512;
+constexpr int BAR_BYTES = SKIP_OFF + SKIP_UNITS / 8;
+static_assert((4 * MAX_RING + 6) * 8 + 4 <= SKIP_OFF, "x3 barriers overlap the early-exit bits");
 constexpr int SMEM_LIMIT = 227 * 1024;
 
 enum OutMode : int { OUT_F32 = 0, OUT_SPLIT = 1 };
@@ -52,12 +58,11 @@ struct X3Params {
     int n_layers;
     X3Layer layer[MAX_LAYERS];
     int rows, n_tiles, n_groups, a_box_rows;
-    int h_blocks;          // 16 KB blocks per hidden plane (0 for a single layer)
     int a_slots, w_slots, w_slot_bytes;
-    int epi_warps, stage_in_h, smem_pad, bias_total, qmaps, pair;
+    int epi_warps, smem_pad, bias_total, qmaps, pair;
     int out_mode;          // OUT_F32: out0 = fp32 [rows, ld_out]; OUT_SPLIT: out0 / out1 = bf16 hi / lo planes [rows, ld_out]
     void* out0; void* out1; int ld_out;
-    long long* prof;       // optional [8] cycle counters of CTA 0's issue warp (nullptr = off)
+    long long* prof;       // optional [9] cycle counters of CTA 0's issue warp and first epilogue warp (nullptr = off)
     // early exit (reference model/query_sat.py:330-338): rows of chain c belong to early-exit group c / chains_per_group;
     // a work unit all of whose rows belong to finished groups is skipped by every warp role (nullptr = never skip)
     const int* done; int rows_per_chain, chains_per_group;
@@ -67,31 +72,23 @@ struct X3Params {
 __device__ __forceinline__ void split2(float v0, float v1, uint32_t& hi, uint32_t& lo) { split_bf16x2(v0, v1, hi, lo); }
 
 struct Epi {
-    uint32_t lane_addr, h_addr, bl_addr, stage_addr;
-    int N, epi, cpar, cstep, r, lane, qmaps, col0, h_plane_bytes;
+    uint32_t lane_addr, bl_addr, stage_addr;
+    int N, epi, cpar, cstep, lane, qmaps, col0;
     size_t row_first; int rows_left;
     void* out0; void* out1; int ld_out, out_mode;
 };
 
-// hidden layer: bias + leaky relu in fp32, split, both planes into the K-major SWIZZLE_128B blocks
+// hidden layer: bias + leaky relu in fp32, split, and both planes back into the 32 accumulator columns just read
+// (hi of K in [c, c+32) at columns [c, c+16), lo at [c+16, c+32), two bf16 per column, the lower K in the low half):
+// the A operand of the next layer's MMAs (tc::tmem_a_kstep).  Columns past N hold values of unused accumulator columns
+// and are never read as A: the next layer's K steps stop at its K <= N.
 __device__ __forceinline__ void epi_hidden(const Epi& e, const uint32_t (&raw)[32], int c) {
     float v[32];
     fm::bias_act_chunk(raw, e.bl_addr + 4u * (uint32_t)c, e.epi == tc::TC_LRELU, v);
-    const uint32_t blk = e.h_addr + (uint32_t)(c >> 6) * BLK_BYTES + (uint32_t)e.r * 128;
-    const int j0 = (c & 63) >> 3;
+    uint32_t w[32];
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        uint4 hi, lo;
-        split2(v[8 * q], v[8 * q + 1], hi.x, lo.x);
-        split2(v[8 * q + 2], v[8 * q + 3], hi.y, lo.y);
-        split2(v[8 * q + 4], v[8 * q + 5], hi.z, lo.z);
-        split2(v[8 * q + 6], v[8 * q + 7], hi.w, lo.w);
-        if (c + 8 * q < e.N) {
-            const uint32_t at = blk + (uint32_t)(((j0 + q) ^ (e.r & 7)) << 4);
-            fm::sts128(at, hi);
-            fm::sts128(at + (uint32_t)e.h_plane_bytes, lo);
-        }
-    }
+    for (int i = 0; i < 16; ++i) split2(v[2 * i], v[2 * i + 1], w[i], w[16 + i]);
+    fm::tmem_st_32cols(e.lane_addr + (uint32_t)c, w);
 }
 
 __device__ __forceinline__ void epi_final(const Epi& e, const uint32_t (&raw)[32], int c) {
@@ -141,20 +138,18 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     if ((int)(smem - smem_raw) > p.smem_pad) __trap();
-    const int h_plane_bytes = p.h_blocks * BLK_BYTES;
-    uint8_t* hid = smem;                                           // [2][h_blocks] blocks: hi plane, lo plane
-    uint8_t* a_ring = smem + 2 * (size_t)h_plane_bytes;
+    uint8_t* a_ring = smem;
     uint8_t* w_ring = a_ring + (size_t)p.a_slots * BLK_BYTES;
     uint8_t* stage_all = w_ring + (size_t)p.w_slots * p.w_slot_bytes;
-    uint8_t* tail = stage_all + (p.stage_in_h ? 0 : (size_t)p.epi_warps * 32 * STAGE_ROW);
+    uint8_t* tail = stage_all + (size_t)p.epi_warps * 32 * STAGE_ROW;
     uint64_t* a_full = reinterpret_cast<uint64_t*>(tail);          // [MAX_RING]
     uint64_t* a_empty = a_full + MAX_RING;
     uint64_t* w_full = a_empty + MAX_RING;
     uint64_t* w_empty = w_full + MAX_RING;
     uint64_t* tmem_full = w_empty + MAX_RING;                       // [2]
     uint64_t* tmem_empty = tmem_full + 2;                           // [2]
-    uint64_t* h_full = tmem_empty + 2;                              // [1]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(h_full + 1);
+    uint64_t* h_full = tmem_empty + 2;                              // [2]: hidden columns [0, 128), [128, 256)
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(h_full + 2);
     float* bias_s = reinterpret_cast<float*>(tail + BAR_BYTES);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -172,7 +167,7 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
             mbar_init(&w_full[s], NC); mbar_init(&w_empty[s], 1);
         }
         for (int b = 0; b < 2; ++b) { mbar_init(&tmem_full[b], 1); mbar_init(&tmem_empty[b], NC * p.epi_warps); }
-        mbar_init(h_full, NC * p.epi_warps);
+        for (int h = 0; h < 2; ++h) mbar_init(&h_full[h], NC * p.epi_warps);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_hi) : "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a_lo) : "memory");
@@ -211,8 +206,7 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
     // rings and the accumulator parities count PROCESSED units), and nobody should wait for an L2 round trip per unit on its
     // issue path: the flags of this CTA's units are evaluated once, by all threads, into shared memory (`done` is written by
     // an earlier kernel and constant during this one).  More than SKIP_UNITS units per CTA: no skipping in this launch.
-    constexpr int SKIP_UNITS = 1024;
-    uint32_t* skip_bits = reinterpret_cast<uint32_t*>(tail + 384);      // 128 spare bytes of the barrier block
+    uint32_t* skip_bits = reinterpret_cast<uint32_t*>(tail + SKIP_OFF);
     const bool skipping = p.done != nullptr && nt <= SKIP_UNITS;
     if (skipping) {
         for (int base = 32 * warp; base < nt; base += (int)blockDim.x) {      // one unit per thread, one 32-bit word per warp pass
@@ -279,9 +273,19 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
     } else if (warp == 1) {
         if (leader) {      // ================================ MMA issuer: whole warp converged, one elected lane issues
             int as = 0, ws = 0; uint32_t aph = 0, wph = 0;
-            long long t_wait_acc = 0, t_wait_h = 0, t_wait_a = 0, t_wait_w = 0;
+            long long t_wait_acc = 0, t_wait_h = 0, t_wait_a = 0, t_wait_w = 0, t_wait_read = 0;
             const long long t_begin = timing ? clock64() : 0;
             auto commit = [&](uint64_t* bar) { if constexpr (PAIR) tcgen05_commit_elect_cg2(bar); else tcgen05_commit_elect(bar); };
+            // hidden layers: A (hi or lo plane) from tensor memory at column ta
+            auto kblock_ts = [&](uint32_t acc, uint32_t ta, uint64_t db, uint32_t idesc, uint32_t accum, int ksteps, uint64_t* free_bar) {
+                if (ksteps == BLOCK_K / 16) {
+                    umma_bf16_ts_kblock_elect<PAIR>(acc, ta, db, idesc, accum);
+                } else {
+                    for (int k = 0; k < ksteps; ++k)
+                        umma_bf16_ts_elect<PAIR>(acc, ta + tmem_a_kstep(k), db + (uint64_t)(2 * k), idesc, (accum | (uint32_t)k) != 0);
+                }
+                if (free_bar) commit(free_bar);
+            };
             auto kblock = [&](uint32_t acc, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accum, int ksteps, uint64_t* free_bar) {
                 if (ksteps == BLOCK_K / 16) {
                     if (free_bar) {
@@ -306,41 +310,58 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
                 for (int l = 0; l < L; ++l) {
                     const int g = jp * L + l, buf = g & 1, use = g >> 1;
                     X3_WAIT(t_wait_acc, mbar_wait(&tmem_empty[buf], (uint32_t)((use & 1) ^ 1)));
-                    if (l > 0) X3_WAIT(t_wait_h, mbar_wait(h_full, (uint32_t)((jp * (L - 1) + (l - 1)) & 1)));
+                    // Step g - 1 of a hidden layer read its A operand from this half.  The PTX ISA orders tcgen05.mma pairs
+                    // only on the same accumulator, so the MMAs writing here wait until those reads have completed (the
+                    // commit on tmem_full of step g - 1; the issuer made the next commit to that barrier itself, so the
+                    // phase cannot have moved on).
+                    if (g > 0 && (l > 0 ? l - 1 : L - 1) > 0)
+                        X3_WAIT(t_wait_read, mbar_wait(&tmem_full[buf ^ 1], (uint32_t)(((g - 1) >> 1) & 1)));
+                    const uint32_t h_par = (uint32_t)((jp * (L - 1) + (l - 1)) & 1);
                     tcgen05_fence_after();
                     const int K = p.layer[l].K, N = p.layer[l].N;
                     const int kbs = (K + BLOCK_K - 1) / BLOCK_K;
                     const uint32_t idesc = make_idesc_bf16(PAIR ? 2 * BLOCK_M : BLOCK_M, N);
                     const uint32_t acc = tmem_base + (uint32_t)(buf * 256);
+                    const uint32_t hid = tmem_base + (uint32_t)((buf ^ 1) * 256);      // layer l - 1's activations
                     for (int kb = 0; kb < kbs; ++kb) {
                         const int ksteps = min(BLOCK_K / 16, (K - kb * BLOCK_K + 15) / 16);
-                        uint64_t da_hi, da_lo;
-                        int as_hi = 0, as_lo = 0;
                         if (l == 0) {
-                            as_hi = as;
+                            const int as_hi = as;
                             const uint32_t ph_hi = aph;
                             if (++as == p.a_slots) { as = 0; aph ^= 1; }
-                            as_lo = as;
+                            const int as_lo = as;
                             const uint32_t ph_lo = aph;
                             if (++as == p.a_slots) { as = 0; aph ^= 1; }
                             X3_WAIT(t_wait_a, mbar_wait(&a_full[as_hi], ph_hi));
                             X3_WAIT(t_wait_a, mbar_wait(&a_full[as_lo], ph_lo));
-                            da_hi = make_smem_desc_sw128(smem_u32(a_ring + (size_t)as_hi * BLK_BYTES));
-                            da_lo = make_smem_desc_sw128(smem_u32(a_ring + (size_t)as_lo * BLK_BYTES));
+                            const uint64_t da_hi = make_smem_desc_sw128(smem_u32(a_ring + (size_t)as_hi * BLK_BYTES));
+                            const uint64_t da_lo = make_smem_desc_sw128(smem_u32(a_ring + (size_t)as_lo * BLK_BYTES));
+                            X3_WAIT(t_wait_w, mbar_wait(&w_full[ws], wph));
+                            uint64_t db = make_smem_desc_sw128(smem_u32(w_ring + (size_t)ws * p.w_slot_bytes));
+                            kblock(acc, da_hi, db, idesc, kb != 0, ksteps, nullptr);        // x_hi * w_hi
+                            kblock(acc, da_lo, db, idesc, 1u, ksteps, &w_empty[ws]);        // x_lo * w_hi
+                            if (++ws == p.w_slots) { ws = 0; wph ^= 1; }
+                            X3_WAIT(t_wait_w, mbar_wait(&w_full[ws], wph));
+                            db = make_smem_desc_sw128(smem_u32(w_ring + (size_t)ws * p.w_slot_bytes));
+                            kblock(acc, da_hi, db, idesc, 1u, ksteps, &w_empty[ws]);        // x_hi * w_lo
+                            if (++ws == p.w_slots) { ws = 0; wph ^= 1; }
+                            commit(&a_empty[as_hi]); commit(&a_empty[as_lo]);
                         } else {
-                            da_hi = make_smem_desc_sw128(smem_u32(hid + (size_t)kb * BLK_BYTES));
-                            da_lo = make_smem_desc_sw128(smem_u32(hid + (size_t)h_plane_bytes + (size_t)kb * BLK_BYTES));
+                            const uint32_t ta_hi = hid + (uint32_t)(kb * BLOCK_K), ta_lo = ta_hi + 16;
+                            if ((kb & 1) == 0 && kb < 4) {      // K blocks 0-1 / 2-3: the epilogue releases 128 columns at a time
+                                X3_WAIT(t_wait_h, mbar_wait(&h_full[kb >> 1], h_par));
+                                tcgen05_fence_after();
+                            }
+                            X3_WAIT(t_wait_w, mbar_wait(&w_full[ws], wph));
+                            uint64_t db = make_smem_desc_sw128(smem_u32(w_ring + (size_t)ws * p.w_slot_bytes));
+                            kblock_ts(acc, ta_hi, db, idesc, kb != 0, ksteps, nullptr);     // x_hi * w_hi
+                            kblock_ts(acc, ta_lo, db, idesc, 1u, ksteps, &w_empty[ws]);     // x_lo * w_hi
+                            if (++ws == p.w_slots) { ws = 0; wph ^= 1; }
+                            X3_WAIT(t_wait_w, mbar_wait(&w_full[ws], wph));
+                            db = make_smem_desc_sw128(smem_u32(w_ring + (size_t)ws * p.w_slot_bytes));
+                            kblock_ts(acc, ta_hi, db, idesc, 1u, ksteps, &w_empty[ws]);     // x_hi * w_lo
+                            if (++ws == p.w_slots) { ws = 0; wph ^= 1; }
                         }
-                        X3_WAIT(t_wait_w, mbar_wait(&w_full[ws], wph));
-                        uint64_t db = make_smem_desc_sw128(smem_u32(w_ring + (size_t)ws * p.w_slot_bytes));
-                        kblock(acc, da_hi, db, idesc, kb != 0, ksteps, nullptr);        // x_hi * w_hi
-                        kblock(acc, da_lo, db, idesc, 1u, ksteps, &w_empty[ws]);        // x_lo * w_hi
-                        if (++ws == p.w_slots) { ws = 0; wph ^= 1; }
-                        X3_WAIT(t_wait_w, mbar_wait(&w_full[ws], wph));
-                        db = make_smem_desc_sw128(smem_u32(w_ring + (size_t)ws * p.w_slot_bytes));
-                        kblock(acc, da_hi, db, idesc, 1u, ksteps, &w_empty[ws]);        // x_hi * w_lo
-                        if (++ws == p.w_slots) { ws = 0; wph ^= 1; }
-                        if (l == 0) { commit(&a_empty[as_hi]); commit(&a_empty[as_lo]); }
                     }
                     commit(&tmem_full[buf]);
                 }
@@ -349,21 +370,19 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
 #undef X3_WAIT
             if (timing && lane == 0) {
                 p.prof[0] = clock64() - t_begin; p.prof[1] = t_wait_acc; p.prof[2] = t_wait_h; p.prof[3] = t_wait_a; p.prof[4] = t_wait_w;
+                p.prof[8] = t_wait_read;
             }
         }
     } else if (warp < 2 + p.epi_warps) {               // ================================ epilogue warps
         const int quad = warp & 3;
         Epi e;
-        e.r = quad * 32 + lane;
         e.lane = lane;
         e.cpar = (warp - 2) >> 2;
         e.cstep = 32 * (p.epi_warps >> 2);
         e.qmaps = p.qmaps;
         e.out0 = p.out0; e.out1 = p.out1; e.ld_out = p.ld_out; e.out_mode = p.out_mode;
-        e.h_plane_bytes = h_plane_bytes;
-        e.h_addr = smem_u32(hid);
         const uint32_t bias_addr0 = smem_u32(bias_s);
-        e.stage_addr = (p.stage_in_h ? smem_u32(hid) : smem_u32(stage_all)) + (uint32_t)(warp - 2) * (32 * STAGE_ROW);
+        e.stage_addr = smem_u32(stage_all) + (uint32_t)(warp - 2) * (32 * STAGE_ROW);
         long long t_wait_full = 0, t_hidden = 0, t_final = 0;
         int jp = -1;
         for (int j = 0; j < nt; ++j) {
@@ -385,6 +404,21 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
                 const long long t1 = timing ? clock64() : 0;
                 const uint32_t empty_addr = at_leader(&tmem_empty[buf]);
                 if (l + 1 < L) {
+                    // The planes are in tensor memory before the issuer hears of them, 128 columns at a time (h_full[0] once
+                    // this warp's chunks below column 128 are stored: the next layer's K blocks 0-1 start while the epilogue
+                    // works on the rest).  The accumulator half stays in use (as A) until the next layer's MMAs completed:
+                    // the arrival on tmem_empty only keeps its phases counting steps, the issuer orders the half's next
+                    // accumulation after those MMAs itself.
+                    bool low_done = false;
+                    auto release = [&](int h) {
+                        fm::tmem_st_wait();
+                        tcgen05_fence_before();
+                        __syncwarp();
+                        if (lane == 0) {
+                            if (h == 1) fm::arrive_addr<PAIR>(empty_addr);
+                            fm::arrive_addr<PAIR>(at_leader(&h_full[h]));
+                        }
+                    };
                     // two register buffers: chunk c + cstep is on its way out of TMEM while chunk c is processed
                     int c = 32 * e.cpar;
                     if (c < e.N) {
@@ -396,18 +430,18 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
                             const int c1 = c + e.cstep;
                             if (c1 < e.N) fm::tmem_ld_32cols_async(e.lane_addr + (uint32_t)c1, rb);
                             epi_hidden(e, ra, c);
+                            if (!low_done && c1 >= 128) { release(0); low_done = true; }
                             if (c1 >= e.N) break;
                             fm::tmem_ld_wait(rb);
                             c = c1 + e.cstep;
                             if (c < e.N) fm::tmem_ld_32cols_async(e.lane_addr + (uint32_t)c, ra);
                             epi_hidden(e, rb, c1);
+                            if (!low_done && c >= 128) { release(0); low_done = true; }
                             if (c >= e.N) break;
                         }
                     }
-                    tcgen05_fence_before();
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // st.shared -> visible to this CTA's MMAs
-                    __syncwarp();
-                    if (lane == 0) { fm::arrive_addr<PAIR>(empty_addr); fm::arrive_addr<PAIR>(at_leader(h_full)); }
+                    if (!low_done) release(0);
+                    release(1);
                     if (timing) t_hidden += clock64() - t1;
                 } else {
                     bool released = false;
@@ -424,9 +458,6 @@ x3_mlp_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constan
                         epi_final(e, ra, c);
                     }
                     if (!released) { tcgen05_fence_before(); fm::warp_arrive<PAIR>(empty_addr, lane); }
-                    // staging inside the hidden region: nobody may write the next hidden activations there while another
-                    // warp still reads back its staged output
-                    if (p.stage_in_h) asm volatile("bar.sync 1, %0;" ::"r"(epi_threads) : "memory");
                     if (timing) t_final += clock64() - t1;
                 }
                 if (timing) t_wait_full += t1 - t0;
@@ -462,53 +493,40 @@ inline bool plan_x3(X3Mlp& f) {
     X3Params& p = f.p;
     const int pad = fm::dyn_smem_pad();
     p.smem_pad = pad;
-    int bias_total = 0, max_n = 0, h_blocks = 0;
+    int bias_total = 0, max_n = 0;
     bool pair = f.pair_mode && p.rows > BLOCK_M;
     for (int l = 0; l < p.n_layers; ++l) {
         X3Layer& ly = p.layer[l];
         if (ly.N > 256 || ly.N % 16 || ly.K % 16) return false;
-        if (l + 1 < p.n_layers) h_blocks = max(h_blocks, (ly.N + 63) / 64);
+        if (l > 0 && ly.K > p.layer[l - 1].N) return false;     // a hidden layer's A: the columns layer l - 1 wrote
         ly.bias_off = bias_total;
         bias_total += (ly.n_total + 31) / 32 * 32;
         max_n = max(max_n, ly.N);
     }
     if (p.n_groups > 1 && p.n_layers != 1) return false;
     p.pair = pair ? 1 : 0;
-    p.h_blocks = h_blocks;
     p.bias_total = bias_total;
     p.n_tiles = ceil_div(p.rows, BLOCK_M);
     p.w_slot_bytes = ((pair ? max_n / 2 : max_n) * BLOCK_K * 2 + 1023) / 1024 * 1024;
     for (int ew : {8, 4}) {
         if (ew == 8 && f.four_epilogue_warps) continue;
-        const int stage_bytes = ew * 32 * STAGE_ROW;
-        const int in_h = 2 * h_blocks * BLK_BYTES >= stage_bytes;
-        const int fixed = pad + 2 * h_blocks * BLK_BYTES + (in_h ? 0 : stage_bytes) + BAR_BYTES + bias_total * 4;
+        const int fixed = pad + ew * 32 * STAGE_ROW + BAR_BYTES + bias_total * 4;
         int avail = SMEM_LIMIT - fixed;
         int a = 2, w = 2;
         if (avail < a * BLK_BYTES + w * p.w_slot_bytes) continue;
         avail -= a * BLK_BYTES + w * p.w_slot_bytes;
-        if (p.n_layers > 1) {
-            // MLPs with hidden layers have little shared memory left, and their first layer is bound by the latency of the
-            // input stream from HBM (clock64 breakdown at cfg2: the issue warp of the clause / update MLPs waited 36 / 40 %
-            // of its time for input with a 3 + 3 split; 4 + 2: clause 1.60 -> 1.48 ms, update 0.64 -> 0.54 ms).  The weights
-            // come from L2 and are the same for every tile: two slots suffice, the input ring takes the rest (up to a tile).
-            const int a_want = min(MAX_RING, 2 * ((p.layer[0].K + BLOCK_K - 1) / BLOCK_K));
-            while (a < a_want && avail >= BLK_BYTES) { ++a; avail -= BLK_BYTES; }
-            while (w < MAX_RING && avail >= p.w_slot_bytes) { ++w; avail -= p.w_slot_bytes; }
-        } else {
-            // single wide layers: grow the rings in turn (the input comes from HBM, the weights from L2: the input ring first)
-            while (true) {
-                bool grew = false;
-                if (a <= w && a < MAX_RING && avail >= BLK_BYTES) { ++a; avail -= BLK_BYTES; grew = true; }
-                else if (w < MAX_RING && avail >= p.w_slot_bytes) { ++w; avail -= p.w_slot_bytes; grew = true; }
-                else if (a < MAX_RING && avail >= BLK_BYTES) { ++a; avail -= BLK_BYTES; grew = true; }
-                if (!grew) break;
-            }
+        // grow the rings in turn, the input ring first (the input comes from HBM, the weights from L2)
+        while (true) {
+            bool grew = false;
+            if (a <= w && a < MAX_RING && avail >= BLK_BYTES) { ++a; avail -= BLK_BYTES; grew = true; }
+            else if (w < MAX_RING && avail >= p.w_slot_bytes) { ++w; avail -= p.w_slot_bytes; grew = true; }
+            else if (a < MAX_RING && avail >= BLK_BYTES) { ++a; avail -= BLK_BYTES; grew = true; }
+            if (!grew) break;
         }
         const int ea = env_int("DSAT_X3_A_SLOTS", 0), ewn = env_int("DSAT_X3_W_SLOTS", 0);
         if (ea >= 2 && ewn >= 2 && ea <= MAX_RING && ewn <= MAX_RING &&
             fixed + ea * BLK_BYTES + ewn * p.w_slot_bytes <= SMEM_LIMIT) { a = ea; w = ewn; }
-        p.a_slots = a; p.w_slots = w; p.epi_warps = ew; p.stage_in_h = in_h;
+        p.a_slots = a; p.w_slots = w; p.epi_warps = ew;
         f.smem_bytes = fixed + a * BLK_BYTES + w * p.w_slot_bytes;
         f.ready = true;
         return true;

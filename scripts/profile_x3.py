@@ -11,5 +11,6 @@ names = ["query", "lit1", "lit2", "lit3", "clause", "update", "output"]
 for w in range(7):
     c = ctx.profile_fused(w)
     tot = c[0] or 1
-    print("%-7s mma warp %9d cyc | waits: accumulator %4.1f%%  hidden %4.1f%%  input %4.1f%%  weights %4.1f%% | epilogue warp: tmem_full wait %4.1f%%  hidden epi %4.1f%%  final epi %4.1f%%"
-          % (names[w], tot, 100 * c[1] / tot, 100 * c[2] / tot, 100 * c[3] / tot, 100 * c[4] / tot, 100 * c[5] / tot, 100 * c[6] / tot, 100 * c[7] / tot))
+    # "A reads": the wait before accumulating into the half the previous hidden layer's MMAs read their A operand from
+    print("%-7s mma warp %9d cyc | waits: accumulator %4.1f%%  A reads %4.1f%%  hidden %4.1f%%  input %4.1f%%  weights %4.1f%% | epilogue warp: tmem_full wait %4.1f%%  hidden epi %4.1f%%  final epi %4.1f%%"
+          % (names[w], tot, 100 * c[1] / tot, 100 * c[8] / tot, 100 * c[2] / tot, 100 * c[3] / tot, 100 * c[4] / tot, 100 * c[5] / tot, 100 * c[6] / tot, 100 * c[7] / tot))
