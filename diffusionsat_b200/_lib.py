@@ -48,6 +48,7 @@ _SIGNATURES = {
     "dsat_get_precision": (C.c_int, [_vp]),
     "dsat_set_graph": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _i32p, _i32p, _i32p, _i32p, C.c_int, _i32p, _i32p,
                                  C.c_int, C.c_int]),
+    "dsat_set_batches": (C.c_int, [_vp, C.c_int, _i32p, _u64p]),
     "dsat_graph_build": (C.c_int, [C.c_int, C.c_int, C.c_longlong, _i32p, _i32p, _i32p, _i32p, _i32p, _i32p, _i32p]),
     "dsat_model_call": (C.c_int, [_vp, C.c_float, _f32p, _i32p, _f32p, C.c_int, C.c_uint64, C.c_uint64, _f32p, _i32p,
                                   _f32p]),
@@ -57,6 +58,7 @@ _SIGNATURES = {
     "dsat_sample_fetch": (C.c_int, [_vp, _u64p, _u8p, _i32p, _u8p]),
     "dsat_words_per_graph": (C.c_int, [_vp]),
     "dsat_hist_reduce": (C.c_int, [_vp, C.c_int, _u64p, C.POINTER(C.c_int64), C.c_int, _i32p, _i32p]),
+    "dsat_hist_reduce_segments": (C.c_int, [_vp, C.c_int, _i32p, _i32p, _u64p, C.POINTER(C.c_int64), C.c_int, _i32p, _i32p]),
     "dsat_spmm": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_int]),
     "dsat_profile_classes": (C.c_int, []),
     "dsat_profile_fused": (C.c_int, [_vp, C.c_int, C.POINTER(C.c_longlong)]),
@@ -205,6 +207,17 @@ class Context:
             _ptr(arrs[5], C.c_int32), int(chains), int(group_graphs)))
         self.graph, self.chains = g, int(chains)
         self.group_graphs = int(group_graphs) if group_graphs > 0 else g.n_graphs * int(chains)
+        self.batch_groups = None
+
+    def set_batches(self, group_seg, noise_base=None):
+        """Early-exit groups ``[group_seg[i], group_seg[i+1])`` of the bound graphs and, optionally, the Philox element of
+        variable 0 of every graph (``dsat_set_batches``); cleared by the next ``set_graph``."""
+        seg = np.ascontiguousarray(group_seg, dtype=np.int32)
+        base = None if noise_base is None else np.ascontiguousarray(noise_base, dtype=np.uint64)
+        if base is not None and base.shape != (self.total_graphs,):
+            raise ValueError("noise_base needs one entry per graph (%d), got %r" % (self.total_graphs, base.shape))
+        self._check(self._lib.dsat_set_batches(self._h, int(seg.shape[0]) - 1, _ptr(seg, C.c_int32), _ptr(base, C.c_uint64)))
+        self.batch_groups = int(seg.shape[0]) - 1
 
     # ------------------------------------------------------------------ properties
     @property
@@ -221,6 +234,8 @@ class Context:
 
     @property
     def n_groups(self) -> int:
+        if getattr(self, "batch_groups", None):
+            return self.batch_groups
         return -(-self.total_graphs // self.group_graphs)
 
     # ------------------------------------------------------------------------ calls
@@ -283,6 +298,25 @@ class Context:
         self._check(self._lib.dsat_hist_reduce(self._h, int(chain_limit), _ptr(keys, C.c_uint64),
                                                counts.ctypes.data_as(C.POINTER(C.c_int64)), cap, C.byref(k), C.byref(n_sat)))
         return keys[:k.value], counts[:k.value], int(n_sat.value)
+
+    def hist_reduce_segments(self, graph_seg, limits):
+        """``hist_reduce`` per segment ``[graph_seg[s], graph_seg[s+1])`` of the last run's graphs, counting the first
+        ``limits[s]`` of each: ``([(keys [K_s, words] uint64 ascending, counts [K_s] int64) per segment], n_sat)``."""
+        seg = np.ascontiguousarray(graph_seg, dtype=np.int32)
+        lim = np.ascontiguousarray(limits, dtype=np.int32)
+        n_seg = int(seg.shape[0]) - 1
+        if lim.shape != (n_seg,):
+            raise ValueError("one limit per segment (%d), got %r" % (n_seg, lim.shape))
+        words = int(self._lib.dsat_words_per_graph(self._h))
+        cap = int(np.minimum(lim, np.diff(seg)).clip(min=0).sum()) if n_seg > 0 else 0
+        keys = np.empty((max(cap, 1), words), dtype=np.uint64)
+        counts = np.empty(max(cap, 1), dtype=np.int64)
+        runs = np.zeros(n_seg + 1, dtype=np.int32)
+        n_sat = C.c_int32(0)
+        self._check(self._lib.dsat_hist_reduce_segments(self._h, n_seg, _ptr(seg, C.c_int32), _ptr(lim, C.c_int32),
+                                                        _ptr(keys, C.c_uint64), counts.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                        cap, _ptr(runs, C.c_int32), C.byref(n_sat)))
+        return [(keys[runs[s]:runs[s + 1]], counts[runs[s]:runs[s + 1]]) for s in range(n_seg)], int(n_sat.value)
 
     def spmm(self, direction: int, x_dev_ptr: int, y_dev_ptr: int, feat: int, dtype: int, chains: int):
         self._check(self._lib.dsat_spmm(self._h, int(direction), _vp(x_dev_ptr), _vp(y_dev_ptr), int(feat), int(dtype),

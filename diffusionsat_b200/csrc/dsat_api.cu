@@ -106,6 +106,11 @@ struct dsat_ctx {
     int n = 0, m = 0, nnz = 0, n_graphs = 0, chains = 0, group_graphs = 0, n_groups = 0, total_graphs = 0;
     int words = 0;
     int max_graph_vars = 0, max_graph_clauses = 0;      // largest formula of the unit (shared-memory PairNorm)
+    // variable early-exit groups and per-graph noise bases (dsat_set_batches); cleared by dsat_set_graph
+    bool has_batches = false, has_noise_base = false;
+    DevBuf<int> batch_seg, graph_group;  // [n_groups+1] group bounds, [total_graphs] group of each graph
+    DevBuf<int> row_graph;               // [Nt] graph of each variable row
+    DevBuf<unsigned long long> graph_elem0;   // [total_graphs] noise base of the graph minus its first row (mod 2^64)
     long long Nt = 0, Mt = 0;
     DevBuf<int> cl_rowptr, cl_lit, lit_rowptr, lit_clause, var_seg, clause_seg;
     DevBuf<float> deg_w, vdeg_w, rev_w;
@@ -132,7 +137,7 @@ struct dsat_ctx {
     DevBuf<unsigned char> BITS, LAST, LATCH, FINAL, is_sat, sat_any;
     DevBuf<unsigned long long> packed;
     // histogram reduction scratch (dsat_hist.cuh)
-    DevBuf<int> hist_idx, hist_run, hist_totals;
+    DevBuf<int> hist_idx, hist_run, hist_totals, hist_seg, hist_run_seg;
     DevBuf<unsigned long long> hist_keys, hist_counts;
     // injected noise staging
     DevBuf<float> inj_normals, inj_uniforms, inj_noisy;
@@ -255,11 +260,19 @@ UnitGraphDev graph_view(const dsat_ctx* c) {
     return g;
 }
 
-// rows of finished early-exit groups are skipped when the groups consist of whole chains (DSAT_SKIP_DONE=0 turns it off)
+// rows of finished early-exit groups are skipped when the groups consist of whole chains (DSAT_SKIP_DONE=0 turns it off).
+// Variable groups (dsat_set_batches) are not runs of whole chains: nothing is skipped, which changes no result.
 SkipInfo skip_info(const dsat_ctx* c) {
     static const bool off = getenv("DSAT_SKIP_DONE") && atoi(getenv("DSAT_SKIP_DONE")) == 0;
-    if (off || c->n_graphs <= 0 || c->group_graphs % c->n_graphs != 0) return SkipInfo{nullptr, 1};
+    if (off || c->has_batches || c->n_graphs <= 0 || c->group_graphs % c->n_graphs != 0) return SkipInfo{nullptr, 1};
     return SkipInfo{c->done.p, c->group_graphs / c->n_graphs};
+}
+
+// Philox element of local row 0 = chain_offset * n, or the per-graph bases bound by dsat_set_batches
+NoiseSource noise_source(const dsat_ctx* c, uint64_t seed, uint64_t element_offset, unsigned step) {
+    NoiseSource ns{seed, element_offset, step};
+    if (c->has_noise_base) { ns.row_graph = c->row_graph.p; ns.graph_elem0 = c->graph_elem0.p; }
+    return ns;
 }
 
 // buffers every precision uses: the fp32 outputs of the MLPs, the diffusion state and the per-graph bookkeeping
@@ -506,6 +519,7 @@ void free_buffers(dsat_ctx* c) {
     c->sat_now.release(); c->is_sat.release(); c->sat_any.release(); c->packed.release();
     c->inj_normals.release(); c->inj_uniforms.release(); c->inj_noisy.release(); c->inj_labels.release();
     c->hist_idx.release(); c->hist_run.release(); c->hist_totals.release(); c->hist_keys.release(); c->hist_counts.release();
+    c->hist_seg.release(); c->hist_run_seg.release();
 #ifdef DSAT_WITH_TCGEN05
     c->VROWb.release(); c->CROWb.release(); c->H1b.release(); c->H2b.release(); c->QSb.release(); c->LITb.release();
     c->CHb.release(); c->COUTb.release(); c->UOUTb.release(); c->U1b.release(); c->U2b.release(); c->SPREb.release();
@@ -1169,11 +1183,12 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
     head_kernel<<<c->total_graphs, 128, 0, c->stream>>>(g, c->total_graphs, c->group_graphs, c->LOGITS.p,
                                                          DSAT_LOGIT_PAD, c->labels.p, ls.t, ls.ts, ls.norm_plus,
                                                          c->done.p, c->OUT.p, c->BITS.p, c->graph_sat.p,
-                                                         c->graph_loss.p, c->graph_map.p, sp_tab, sp_cur);
+                                                         c->graph_loss.p, c->graph_map.p, sp_tab, sp_cur,
+                                                         c->has_batches ? c->graph_group.p : nullptr);
     LAUNCHED(c);
     group_finalize_kernel<<<(c->n_groups + 127) / 128, 128, 0, c->stream>>>(
         c->n_groups, c->group_graphs, c->total_graphs, round, c->graph_sat.p, c->graph_loss.p, c->done.p,
-        c->steps_taken.p, c->loss_sum.p, c->rounds_run.p);
+        c->steps_taken.p, c->loss_sum.p, c->rounds_run.p, c->has_batches ? c->batch_seg.p : nullptr);
     LAUNCHED(c);
     prof_mark(c, PROF_END);
     return DSAT_OK;
@@ -1327,6 +1342,7 @@ void dsat_destroy(dsat_ctx* c) {
     for (auto& w : c->wx) w.release();
 #endif
     c->cl_rowptr.release(); c->cl_lit.release(); c->lit_rowptr.release(); c->lit_clause.release();
+    c->batch_seg.release(); c->graph_group.release(); c->row_graph.release(); c->graph_elem0.release();
     c->var_seg.release(); c->clause_seg.release(); c->deg_w.release(); c->vdeg_w.release(); c->rev_w.release(); c->var_order.release();
     c->cl_idx16.release(); c->lit_idx16.release(); c->cl_idx16_vecs = c->lit_idx16_vecs = 0;
     c->cl_desc.release(); c->lit_desc.release(); c->lit_desc4.release();
@@ -1484,10 +1500,11 @@ int dsat_set_graph(dsat_ctx* c, int n_vars, int n_clauses, int nnz, const int32_
     const int group_new = group_graphs > 0 ? group_graphs : total_graphs_new;
     const bool same_shape = c->has_graph && c->n == n_vars && c->m == n_clauses && c->n_graphs == n_graphs &&
                             c->chains == n_chains && c->words == ceil_div(max_graph_vars, 64) &&
-                            c->group_graphs == group_new;
+                            c->group_graphs == group_new && !c->has_batches;
     if (!same_shape) release_buffers(c);
     c->generation++;        // the index arrays are re-allocated
     c->has_graph = false;               // set again at the end: an upload that fails half way leaves no graph bound
+    c->has_batches = c->has_noise_base = false;
     c->n = n_vars; c->m = n_clauses; c->nnz = nnz; c->n_graphs = n_graphs; c->chains = n_chains;
     c->total_graphs = n_graphs * n_chains;
     c->group_graphs = group_graphs > 0 ? group_graphs : c->total_graphs;
@@ -1579,6 +1596,61 @@ int dsat_set_graph(dsat_ctx* c, int n_vars, int n_clauses, int nnz, const int32_
 
 int dsat_words_per_graph(const dsat_ctx* c) { return c ? c->words : 0; }
 
+int dsat_set_batches(dsat_ctx* c, int n_groups, const int32_t* group_seg, const uint64_t* noise_base) {
+    if (!c) return DSAT_ERR_ARG;
+    CK_ARG(c, c->has_graph, "dsat_set_batches: bind a graph first");
+    const int G = c->total_graphs;
+    CK_ARG(c, n_groups > 0 && n_groups <= G && group_seg, "dsat_set_batches: bad group count or null group_seg");
+    CK_ARG(c, group_seg[0] == 0 && group_seg[n_groups] == G, "dsat_set_batches: groups do not cover the graphs of the context");
+    for (int i = 0; i < n_groups; ++i)
+        CK_ARG(c, group_seg[i + 1] > group_seg[i], "dsat_set_batches: empty or unordered group");
+    // host copies of the unit's graph segments: row range of every graph
+    std::vector<int> var_seg(c->n_graphs + 1);
+    CK_CUDA(c, cudaSetDevice(c->device));
+    CK_CUDA(c, cudaStreamSynchronize(c->stream));
+    CK_CUDA(c, dsat_memcpy_sync(var_seg.data(), c->var_seg.p, var_seg.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    auto row0 = [&](int gi) { return (uint64_t)(gi / c->n_graphs) * (uint64_t)c->n + (uint64_t)var_seg[gi % c->n_graphs]; };
+    if (noise_base)
+        for (int gi = 0; gi < G; ++gi) {
+            const uint64_t vars = (uint64_t)(var_seg[gi % c->n_graphs + 1] - var_seg[gi % c->n_graphs]);
+            CK_ARG(c, noise_base[gi] <= UINT64_MAX - vars, "dsat_set_batches: a graph's Philox elements would wrap around 2^64");
+        }
+    std::vector<int> group_of(G);
+    for (int i = 0; i < n_groups; ++i)
+        for (int gi = group_seg[i]; gi < group_seg[i + 1]; ++gi) group_of[gi] = i;
+    // everything validated: commit (every table a captured step reads may move, so the step is captured again)
+    c->generation++;
+    c->has_batches = c->has_noise_base = false;
+    CK_CUDA(c, c->batch_seg.alloc(n_groups + 1));
+    CK_CUDA(c, dsat_memcpy_sync(c->batch_seg.p, group_seg, (n_groups + 1) * sizeof(int), cudaMemcpyHostToDevice));
+    CK_CUDA(c, c->graph_group.alloc(G));
+    CK_CUDA(c, dsat_memcpy_sync(c->graph_group.p, group_of.data(), G * sizeof(int), cudaMemcpyHostToDevice));
+    if (noise_base) {
+        std::vector<int> rg((size_t)c->Nt);
+        std::vector<unsigned long long> e0(G);
+        for (int gi = 0; gi < G; ++gi) {
+            const uint64_t r0 = row0(gi), r1 = r0 + (uint64_t)(var_seg[gi % c->n_graphs + 1] - var_seg[gi % c->n_graphs]);
+            for (uint64_t r = r0; r < r1; ++r) rg[r] = gi;
+            e0[gi] = noise_base[gi] - r0;           // element of row r = e0 + r (mod 2^64)
+        }
+        CK_CUDA(c, c->row_graph.alloc(rg.size()));
+        CK_CUDA(c, dsat_memcpy_sync(c->row_graph.p, rg.data(), rg.size() * sizeof(int), cudaMemcpyHostToDevice));
+        CK_CUDA(c, c->graph_elem0.alloc(G));
+        CK_CUDA(c, dsat_memcpy_sync(c->graph_elem0.p, e0.data(), G * sizeof(unsigned long long), cudaMemcpyHostToDevice));
+    }
+    // per-group bookkeeping is sized by the group count
+    c->n_groups = n_groups;
+    if (c->has_buffers) {
+        CK_CUDA(c, c->done.alloc(n_groups));
+        CK_CUDA(c, c->steps_taken.alloc(n_groups));
+        CK_CUDA(c, c->rounds_run.alloc(n_groups));
+        CK_CUDA(c, c->loss_sum.alloc(n_groups));
+    }
+    c->has_batches = true;
+    c->has_noise_base = noise_base != nullptr;
+    return DSAT_OK;
+}
+
 // ---------------------------------------------------------------------------------- graph build (host)
 int dsat_graph_build(int n_vars, int n_clauses, long long nnz, const int32_t* lens, const int32_t* flat, int32_t* cl_rowptr,
                      int32_t* cl_lit, int32_t* lit_rowptr, int32_t* lit_clause, int32_t* bad_clause) {
@@ -1606,6 +1678,7 @@ int dsat_model_call(dsat_ctx* c, float noise_scale, const float* noisy_num, cons
                     int32_t* steps_taken, float* loss) {
     if (!c) return DSAT_ERR_ARG;
     CK_ARG(c, noisy_num && prediction_out && rounds >= 0, "dsat_model_call: null buffer or negative rounds");
+    CK_ARG(c, !c->has_noise_base || chain_offset == 0, "dsat_model_call: chain_offset must be 0 while noise bases are bound");
     CK_CUDA(c, cudaSetDevice(c->device));
     int rc = ensure_active_buffers(c);
     if (rc) return rc;
@@ -1620,7 +1693,7 @@ int dsat_model_call(dsat_ctx* c, float noise_scale, const float* noisy_num, cons
         CK_CUDA(c, c->inj_normals.alloc(Nt * 4 * rounds));
         CK_CUDA(c, c->inj_normals.upload(normals, Nt * 4 * rounds, c->stream));
     }
-    NoiseSource ns{seed, chain_offset * (uint64_t)c->n, 0u};
+    const NoiseSource ns = noise_source(c, seed, chain_offset * (uint64_t)c->n, 0u);
     if ((rc = begin_call(c, noise_scale, c->inj_noisy.p, nullptr, labels ? c->inj_labels.p : nullptr, false, ns))) return rc;
     const LossScalars ls = loss_scalars(noise_scale);
     for (int r = 0; r < rounds; ++r)
@@ -1662,7 +1735,7 @@ static StepParams step_params(int t, int n_steps, uint64_t seed, uint64_t elemen
 static int enqueue_step(dsat_ctx* c, const StepParams& sp, int n_rounds, const float* uniforms_dev, const int* labels_dev,
                         const float* normals_dev, const StepParams* sp_tab, const int* sp_cur) {
     const UnitGraphDev g = graph_view(c);
-    NoiseSource ns{sp.seed, sp.element_offset, sp.step};
+    const NoiseSource ns = noise_source(c, sp.seed, sp.element_offset, sp.step);
     int rc = begin_call(c, sp.noise_scale, nullptr, uniforms_dev, labels_dev, true, ns, sp_tab, sp_cur);
     if (rc) return rc;
     LossScalars ls; ls.t = sp.t; ls.ts = sp.ts; ls.norm_plus = sp.norm_plus;
@@ -1749,6 +1822,7 @@ static int sample_enqueue_impl(dsat_ctx* c, int n_steps, int n_rounds, uint64_t 
 int dsat_sample_enqueue(dsat_ctx* c, int n_steps, int n_rounds, uint64_t seed, uint64_t chain_offset) {
     if (!c) return DSAT_ERR_ARG;
     CK_ARG(c, n_steps > 0 && n_rounds >= 0, "dsat_sample: bad step or round count");
+    CK_ARG(c, !c->has_noise_base || chain_offset == 0, "dsat_sample: chain_offset must be 0 while noise bases are bound");
     CK_CUDA(c, cudaSetDevice(c->device));
     return sample_enqueue_impl(c, n_steps, n_rounds, seed, chain_offset, nullptr, nullptr, nullptr);
 }
@@ -1779,6 +1853,7 @@ int dsat_sample(dsat_ctx* c, int n_steps, int n_rounds, uint64_t seed, uint64_t 
                 uint8_t* sat_any_step) {
     if (!c) return DSAT_ERR_ARG;
     CK_ARG(c, n_steps > 0 && n_rounds >= 0, "dsat_sample: bad step or round count");
+    CK_ARG(c, !c->has_noise_base || chain_offset == 0, "dsat_sample: chain_offset must be 0 while noise bases are bound");
     CK_CUDA(c, cudaSetDevice(c->device));
     int rc = ensure_active_buffers(c);
     if (rc) return rc;
@@ -1832,6 +1907,56 @@ int dsat_hist_reduce(dsat_ctx* c, int chain_limit, uint64_t* keys_out, int64_t* 
         CK_CUDA(c, cudaStreamSynchronize(c->stream));
     }
     CK_ARG(c, totals[0] <= capacity, "dsat_hist_reduce: capacity too small (n_unique holds the required size)");
+    return DSAT_OK;
+}
+
+int dsat_hist_reduce_segments(dsat_ctx* c, int n_segments, const int32_t* graph_seg, const int32_t* limit, uint64_t* keys_out,
+                              int64_t* counts_out, int capacity, int32_t* seg_runs, int32_t* n_sat) {
+    if (!c) return DSAT_ERR_ARG;
+    CK_ARG(c, c->has_buffers, "dsat_hist_reduce_segments: nothing was sampled");
+    const int G = c->total_graphs, words = c->words;
+    CK_ARG(c, n_segments > 0 && graph_seg && limit && seg_runs, "dsat_hist_reduce_segments: bad segment count or null array");
+    CK_ARG(c, capacity >= 0 && (capacity == 0 || (keys_out && counts_out)), "dsat_hist_reduce_segments: null output");
+    CK_ARG(c, graph_seg[0] >= 0 && graph_seg[n_segments] <= G, "dsat_hist_reduce_segments: segments outside the context's graphs");
+    for (int s = 0; s < n_segments; ++s) {
+        CK_ARG(c, graph_seg[s + 1] >= graph_seg[s], "dsat_hist_reduce_segments: unordered segments");
+        CK_ARG(c, limit[s] >= 0, "dsat_hist_reduce_segments: negative limit");
+    }
+    CK_CUDA(c, cudaSetDevice(c->device));
+    std::vector<int> seg(G, -1);            // segment of each counted chain index (monotone), -1 outside every limit
+    for (int s = 0; s < n_segments; ++s) {
+        const int end = graph_seg[s] + std::min(limit[s], graph_seg[s + 1] - graph_seg[s]);
+        for (int gi = graph_seg[s]; gi < end; ++gi) seg[gi] = s;
+    }
+    const int n_pad = hist::next_pow2(G < 2 ? 2 : G);
+    CK_CUDA(c, c->hist_idx.alloc(n_pad));
+    CK_CUDA(c, c->hist_run.alloc(n_pad));
+    CK_CUDA(c, c->hist_totals.alloc(2));
+    CK_CUDA(c, c->hist_keys.alloc((size_t)G * words));
+    CK_CUDA(c, c->hist_counts.alloc(G));
+    CK_CUDA(c, c->hist_seg.alloc(G));
+    CK_CUDA(c, c->hist_run_seg.alloc(G));
+    CK_CUDA(c, cudaMemcpyAsync(c->hist_seg.p, seg.data(), G * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    CK_CUDA(c, hist::enqueue(c->stream, G, G, words, c->packed.p, c->is_sat.p, c->hist_idx.p, c->hist_run.p, c->hist_keys.p,
+                             c->hist_counts.p, c->hist_totals.p, &c->launches, c->hist_seg.p, c->hist_run_seg.p));
+    int totals[2] = {0, 0};
+    CK_CUDA(c, cudaMemcpyAsync(totals, c->hist_totals.p, sizeof(totals), cudaMemcpyDeviceToHost, c->stream));
+    CK_CUDA(c, cudaStreamSynchronize(c->stream));      // (also keeps `seg` alive until its upload has run)
+    const int K = totals[0];
+    std::vector<int> run_seg(K);
+    if (K > 0) CK_CUDA(c, dsat_memcpy_sync(run_seg.data(), c->hist_run_seg.p, K * sizeof(int), cudaMemcpyDeviceToHost));
+    for (int s = 0, u = 0; s <= n_segments; ++s) {      // runs come segment by segment
+        while (u < K && run_seg[u] < s) ++u;
+        seg_runs[s] = u;
+    }
+    if (n_sat) *n_sat = totals[1];
+    const int k = K < capacity ? K : capacity;
+    if (k > 0) {
+        CK_CUDA(c, cudaMemcpyAsync(keys_out, c->hist_keys.p, (size_t)k * words * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
+        CK_CUDA(c, cudaMemcpyAsync(counts_out, c->hist_counts.p, (size_t)k * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+        CK_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    CK_ARG(c, K <= capacity, "dsat_hist_reduce_segments: capacity too small (seg_runs[n_segments] holds the required size)");
     return DSAT_OK;
 }
 

@@ -355,14 +355,15 @@ head_kernel(UnitGraphDev g, int total_graphs, int group_graphs,
             float t, float ts, float norm_plus,
             const int* __restrict__ done, float* __restrict__ OUT, unsigned char* BITS,
             int* __restrict__ graph_sat, float* __restrict__ graph_loss, int* __restrict__ graph_map,
-            const StepParams* __restrict__ sp_tab = nullptr, const int* __restrict__ sp_cur = nullptr) {
+            const StepParams* __restrict__ sp_tab = nullptr, const int* __restrict__ sp_cur = nullptr,
+            const int* __restrict__ graph_group = nullptr) {     // early-exit group of each graph (variable groups), or null
     __shared__ float red[4][DSAT_LOGIT_MAPS];
     __shared__ int best_s;
     if (sp_tab) { const StepParams sp = sp_tab[*sp_cur]; t = sp.t; ts = sp.ts; norm_plus = sp.norm_plus; }
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int gid = blockIdx.x;
     if (gid >= total_graphs) return;
-    if (done[gid / group_graphs]) return;
+    if (done[graph_group ? __ldg(graph_group + gid) : gid / group_graphs]) return;
     const int chain = gid / g.n_graphs, lg = gid % g.n_graphs;
     const int v0 = __ldg(g.var_seg + lg), v1 = __ldg(g.var_seg + lg + 1);
     const size_t rowbase = (size_t)chain * g.n;
@@ -425,14 +426,16 @@ head_kernel(UnitGraphDev g, int total_graphs, int group_graphs,
 
 // Batch-global early exit (reference model/query_sat.py:330-338): a group (= one reference batch of
 // graphs) stops at the first round in which every one of its graphs is satisfied.  Also accumulates
-// the scalar loss of :311-315,323.
+// the scalar loss of :311-315,323.  Groups are runs of group_graphs graphs, or [group_seg[i], group_seg[i+1])
+// when variable groups are bound (reference batches of several formulas in one launch, dsat_set_batches).
 __global__ void group_finalize_kernel(int n_groups, int group_graphs, int total_graphs, int round,
                                       const int* __restrict__ graph_sat, const float* __restrict__ graph_loss,
-                                      int* done, int* steps_taken, float* loss_sum, int* rounds_run) {
+                                      int* done, int* steps_taken, float* loss_sum, int* rounds_run,
+                                      const int* __restrict__ group_seg = nullptr) {
     const int grp = blockIdx.x * blockDim.x + threadIdx.x;
     if (grp >= n_groups || done[grp]) return;
-    const int g0 = grp * group_graphs;
-    const int g1 = min(g0 + group_graphs, total_graphs);
+    const int g0 = group_seg ? __ldg(group_seg + grp) : grp * group_graphs;
+    const int g1 = group_seg ? __ldg(group_seg + grp + 1) : min(g0 + group_graphs, total_graphs);
     int all = 1;
     float ls = 0.f;
     for (int gi = g0; gi < g1; ++gi) { all &= graph_sat[gi]; ls += graph_loss[gi]; }
@@ -447,7 +450,16 @@ struct NoiseSource {
     unsigned long long seed;
     unsigned long long element_offset;   // global index of local row 0 (global_chain0 * n_unit)
     unsigned int step;
+    // per-graph noise bases (dsat_set_batches): row r draws element graph_elem0[row_graph[r]] + r, where graph_elem0 holds
+    // each graph's base minus its first row (mod 2^64); null = element_offset + r
+    const int* row_graph = nullptr;
+    const unsigned long long* graph_elem0 = nullptr;
 };
+
+__device__ __forceinline__ unsigned long long noise_element(const NoiseSource& ns, long long r) {
+    return ns.row_graph ? __ldg(ns.graph_elem0 + __ldg(ns.row_graph + r)) + (unsigned long long)r
+                        : ns.element_offset + (unsigned long long)r;
+}
 
 // Model-call start: aux columns [normal4 | noisy2 | noise_scale | 0 0 | pad], state = ones, labels.
 // If `uniforms_or_null`/X are given this is also the randomized rounding of the denoising step
@@ -475,14 +487,14 @@ __global__ void step_begin_kernel(long long n_rows, float noise_scale, float2* X
             // Gumbel-argmax over the two classes (the sampler the reference sketches in model/query_sat.py:15-28, hard instead
             // of soft): class k wins with probability x_k / (x_0 + x_1) -- the same distribution as floor(x_0 + U), but not
             // the same sample under the same uniform, so this mode is validated statistically only
-            const Philox4 p = noise_draw(ns.seed, ns.element_offset + r, ns.step, 0, STREAM_UNIFORM);
+            const Philox4 p = noise_draw(ns.seed, noise_element(ns, r), ns.step, 0, STREAM_UNIFORM);
             const float g0 = -logf(-logf(u32_to_unit_float(p.x) + 1e-20f) + 1e-20f);
             const float g1 = -logf(-logf(u32_to_unit_float(p.y) + 1e-20f) + 1e-20f);
             const float2 x = X[r];
             a = (logf(fmaxf(x.x, 1e-20f)) + g0 >= logf(fmaxf(x.y, 1e-20f)) + g1) ? 1.0f : 0.0f;
         } else {
             const float u = uniforms_in ? uniforms_in[r]
-                                        : u32_to_unit_float(noise_draw(ns.seed, ns.element_offset + r, ns.step, 0, STREAM_UNIFORM).x);
+                                        : u32_to_unit_float(noise_draw(ns.seed, noise_element(ns, r), ns.step, 0, STREAM_UNIFORM).x);
             a = floorf(X[r].x + u);
         }
         b = 1.0f - a;
@@ -513,7 +525,7 @@ __global__ void step_begin_kernel(long long n_rows, float noise_scale, float2* X
         for (int i = 4; i < 8; ++i) reinterpret_cast<__nv_bfloat162*>(auxb)[i] = z;
     }
     labels[r] = labels_in ? labels_in[r]
-                          : (int)(noise_draw(ns.seed, ns.element_offset + r, ns.step, 0, STREAM_LABEL).x & 1u);
+                          : (int)(noise_draw(ns.seed, noise_element(ns, r), ns.step, 0, STREAM_LABEL).x & 1u);
 }
 
 // Fresh N(0,1)[.,4] every round (reference model/query_sat.py:239).
@@ -533,7 +545,7 @@ __global__ void round_noise_kernel(long long n_rows, const float* __restrict__ n
     if (normals_in) {
         nrm = __ldg(reinterpret_cast<const float4*>(normals_in) + r);
     } else {
-        Philox4 p = noise_draw(ns.seed, ns.element_offset + r, ns.step, round, STREAM_NORMAL);
+        Philox4 p = noise_draw(ns.seed, noise_element(ns, r), ns.step, round, STREAM_NORMAL);
         box_muller(p.x, p.y, nrm.x, nrm.y);
         box_muller(p.z, p.w, nrm.z, nrm.w);
     }

@@ -24,7 +24,7 @@ import numpy as np
 
 from . import _lib
 from .dimacs import DimacsFile
-from .graph import MAX_NODES_PER_BATCH, build_unit_graph, chains_per_reference_batch
+from .graph import MAX_NODES_PER_BATCH, build_union_graph, build_unit_graph, chains_per_reference_batch, flatten_formula
 from .query_sat import QuerySAT, distribution_at_time, randomized_rounding_tf, t_power
 from .variable_assignment import VariableAssignment
 from .weights import init_weights, load_weights
@@ -34,6 +34,7 @@ test_rounds = 32
 diffusion_steps = 32
 test_unigen = False
 self_supervised = False
+ROWS_CAP = 900_000          # variable/clause rows per launch (~20 GB of activations at n=100)
 
 
 def reverse_distribution_step_theoretic(x, x0, t, t_increment):
@@ -120,6 +121,24 @@ def unpack_assignments(packed: np.ndarray, n_bits: int) -> list:
     """Packed little-endian 64-bit words [G, words] -> Python ints (x1 = bit 0), masked to n_bits."""
     from .dist import keys_to_ints
     return keys_to_ints(np.asarray(packed, dtype=np.uint64), n_bits)
+
+
+def chains_for_rate(batch: int, n_vars: int, n_clauses: int, still_needed: int, sat_rate: float | None = None) -> int:
+    """Chains of one formula's next launch: whole reference batches, as many as the samples still needed are expected to
+    take at the SAT rate seen so far (first launch: 50 %, at least four batches), at most ``ROWS_CAP`` rows of the larger
+    side."""
+    rate = max(sat_rate if sat_rate is not None else 0.5, 0.02)
+    batches = max(4, -(-int(still_needed / rate * 1.15 + 1) // batch))
+    cap = max(1, ROWS_CAP // max(n_clauses, n_vars, 1) // batch)
+    return batch * min(batches, cap)
+
+
+def check_literals(n_vars: int, clauses):
+    """VariableAssignment(clauses=...) sizes its vector by the largest literal (utils/VariableAssignment.py:34-36); for a
+    header that declares more variables the reference fails in assign_all_from_bit_list on the first sample -- raised here
+    before any GPU work."""
+    if n_vars > max((abs(l) for c in clauses for l in c), default=0):
+        raise IndexError("list assignment index out of range")
 
 
 def consume_batches(is_sat: np.ndarray, batch: int, still_needed: int, total: int, sat_total: int,
@@ -214,11 +233,7 @@ class DiffusionSampler:
         if self.chains_per_launch:
             n = max(b, (self.chains_per_launch // b) * b)
         else:
-            rate = max(sat_rate if sat_rate is not None else 0.5, 0.02)
-            batches = max(4, -(-int(still_needed / rate * 1.15 + 1) // b))
-            rows_cap = 900_000                              # variable/clause rows per launch (~20 GB of activations at n=100)
-            cap = max(1, rows_cap // max(len(self.clauses), self.n_vars, 1) // b)
-            n = b * min(batches, cap)
+            n = chains_for_rate(b, self.n_vars, len(self.clauses), still_needed, sat_rate)
             if self.ctx.graph is self.unit and n <= self.ctx.chains <= 2 * n:
                 n = self.ctx.chains                         # same shape as the previous launch: buffers and the captured step are kept
         if chains_left is not None:
@@ -239,11 +254,7 @@ class DiffusionSampler:
         """``samples()`` before the conversion to Python ints: ``(keys [K, words] uint64 ascending, counts [K] int64)``,
         the form ``dist.merge_histograms`` exchanges between GPUs."""
         from .dist import merge_tables
-        max_lit = max((abs(l) for c in self.clauses for l in c), default=0)
-        if self.n_vars > max_lit:
-            # VariableAssignment(clauses=...) sizes its vector by the largest literal (utils/VariableAssignment.py:34-36);
-            # the reference then fails in assign_all_from_bit_list on the first sample -- raised here before any GPU work
-            raise IndexError("list assignment index out of range")
+        check_literals(self.n_vars, self.clauses)
         tables = []
         total = sat_total = launched = 0
         still_needed = int(n_samples)
@@ -275,3 +286,171 @@ class DiffusionSampler:
         self.last_stats = {"total": total, "sat": sat_total, "chains_launched": launched, "distinct": int(len(counts))}
         print("success rate: ", sat_total / total if total else 0.0)
         return keys, counts
+
+
+class _Formula:
+    """One file of a MultiDiffusionSampler: its graph data, reference batch size and the progress of the current call."""
+
+    def __init__(self, filename, max_nodes_per_batch):
+        dimacs = DimacsFile(filename=filename)
+        dimacs.load()
+        self.n_vars = dimacs.number_of_vars()
+        self.clauses = dimacs.clauses()
+        self.flat = flatten_formula(self.n_vars, self.clauses)
+        self.batch_chains = chains_per_reference_batch(self.n_vars, len(self.clauses), max_nodes_per_batch)
+        self.words = -(-self.n_vars // 64)
+        self.launched_before = 0            # chains launched by earlier samples() calls
+        self.start(0)
+
+    def start(self, n_samples):
+        self.still_needed = int(n_samples)
+        self.total = self.sat_total = self.launched = 0
+        self.stopped = False
+        self.tables = []
+
+    @property
+    def active(self) -> bool:
+        return self.still_needed > 0 and not self.stopped
+
+    @property
+    def rows_per_chain(self) -> int:
+        return self.n_vars + len(self.clauses)
+
+    def next_chains(self) -> int:
+        return chains_for_rate(self.batch_chains, self.n_vars, len(self.clauses), self.still_needed,
+                               self.sat_total / self.total if self.total else None)
+
+
+def plan_launch(formulas, rows_cap: int = ROWS_CAP):
+    """``[(index, chains), ...]`` of the next launch: every active formula in file order with the chains its own
+    ``DiffusionSampler`` would launch, while the variable + clause rows stay within ``rows_cap``.  The first active formula
+    always goes; the first one that does not fit and every later one wait for the next launch."""
+    plan, rows = [], 0
+    for k, f in enumerate(formulas):
+        if not f.active:
+            continue
+        c = f.next_chains()
+        if plan and rows + c * f.rows_per_chain > rows_cap:
+            break
+        plan.append((k, c))
+        rows += c * f.rows_per_chain
+    return plan
+
+
+def launch_layout(formulas, plan, chain_offset: int):
+    """Graph layout of one launch, formula-major (all copies of the first planned formula, then the next ...):
+    ``(graph_seg [len(plan)+1], group_seg, noise_base [graphs] uint64)``.  Early-exit groups are runs of the formula's
+    reference batch size; copy j of formula k draws the noise of chain ``chain_offset + launched_k + j`` of its own sampler,
+    i.e. Philox elements from ``(chain_offset + launched_k + j) * n_k`` on."""
+    graph_seg, group_seg, bases = [0], [0], []
+    for k, c in plan:
+        f = formulas[k]
+        g0 = graph_seg[-1]
+        group_seg.extend(min(g0 + i, g0 + c) for i in range(f.batch_chains, c + f.batch_chains, f.batch_chains))
+        first = chain_offset + f.launched_before + f.launched
+        bases.append((np.arange(first, first + c, dtype=np.uint64)) * np.uint64(f.n_vars))
+        graph_seg.append(g0 + c)
+    noise_base = np.concatenate(bases) if bases else np.zeros(0, dtype=np.uint64)
+    return np.asarray(graph_seg, dtype=np.int32), np.asarray(group_seg, dtype=np.int32), noise_base
+
+
+class MultiDiffusionSampler:
+    """``DiffusionSampler.samples`` for many DIMACS files at once: each launch holds reference batches of every formula that
+    still needs samples (one disjoint-union graph, ``dsat_set_batches``), so a set of small formulas pays the fixed cost of
+    a 32 x 32-round run once per launch instead of once per formula.
+
+    For a fresh sampler ``samples(n)[k]`` equals ``DiffusionSampler(model_path, files[k], ...).samples(n_k)`` built with the
+    same ``seed``, ``chain_offset``, ``max_nodes_per_batch``, ``precision`` and ``sampling``: copy j of a formula draws the
+    noise of that sampler's chain j, forms the same early-exit groups, and the reference's stop rules are applied per
+    formula.  (Bit-identical when the formulas of a launch share the shared-memory PairNorm's thread count; see DESIGN.md.)
+    A formula that is done or has aborted gets no chains in later launches."""
+
+    _prepare_checkpoints = DiffusionSampler._prepare_checkpoints
+
+    def __init__(self, model_path, dimacs_filenames, *, device: int = 0, precision: str = "fp32", seed: int = 0,
+                 chain_offset: int = 0, max_nodes_per_batch: int = MAX_NODES_PER_BATCH, sampling: str = "inverse_cdf",
+                 verbose: bool = False, context=None):
+        self.verbose = verbose
+        print("model_path is ", model_path)
+        weights = self._prepare_checkpoints(model_path)
+        self.formulas = [_Formula(f, max_nodes_per_batch) for f in dimacs_filenames]
+        self.model = QuerySAT(optimizer=None, test_rounds=test_rounds, weights=weights, device=device,
+                              precision=precision, seed=seed, context=context,
+                              feature_maps=weights.feature_maps, query_maps=weights.query_maps)
+        self.ctx = self.model.ctx
+        self.ctx.set_sampling(sampling)
+        self.seed = int(seed)
+        self.chain_offset = int(chain_offset)
+        self.min_sat_rate = 0.005               # reference :261-263, per formula
+        self.last_stats = []
+
+    def reset_chains(self, chain_offset: int | None = None):
+        """Rewind every formula's chain counter (and optionally move the block of global chain ids)."""
+        for f in self.formulas:
+            f.launched_before = 0
+        if chain_offset is not None:
+            self.chain_offset = int(chain_offset)
+
+    def samples(self, n_samples):
+        """:param n_samples: correct samples per formula (one int for all, or one per file)
+        :return: one dict solution-as-int => count per file, in file order"""
+        from .dist import table_to_dict
+        return [table_to_dict(keys, counts, f.n_vars)
+                for f, (keys, counts) in zip(self.formulas, self.samples_table(n_samples))]
+
+    def samples_table(self, n_samples):
+        """``samples()`` before the conversion to Python ints: one ``(keys [K, words_k] uint64 ascending, counts [K] int64)``
+        per file, ``words_k = ceil(n_k / 64)``."""
+        from .dist import merge_tables
+        counts = [int(n_samples)] * len(self.formulas) if np.ndim(n_samples) == 0 else [int(n) for n in n_samples]
+        if len(counts) != len(self.formulas):
+            raise ValueError("n_samples: one count per file (%d), got %d" % (len(self.formulas), len(counts)))
+        for f, n in zip(self.formulas, counts):
+            check_literals(f.n_vars, f.clauses)
+            f.start(n)
+        while True:
+            plan = plan_launch(self.formulas)
+            if not plan:
+                break
+            self._launch(plan)
+        out, self.last_stats = [], []
+        for f in self.formulas:
+            f.launched_before += f.launched
+            keys, cnt = merge_tables(f.tables, f.words)
+            f.tables = []
+            out.append((keys, cnt))
+            self.last_stats.append({"total": f.total, "sat": f.sat_total, "chains_launched": f.launched,
+                                    "distinct": int(len(cnt)), "stopped_on_rate": f.stopped})
+            if self.verbose:
+                print("success rate: ", f.sat_total / f.total if f.total else 0.0)
+        return out
+
+    def _launch(self, plan):
+        graph_seg, group_seg, noise_base = launch_layout(self.formulas, plan, self.chain_offset)
+        unit = build_union_graph([self.formulas[k].flat for k, c in plan for _ in range(c)])
+        self.ctx.set_graph(unit, chains=1)
+        self.ctx.set_batches(group_seg, noise_base)
+        self.model._graph_key = None
+        self.ctx.sample_enqueue(diffusion_steps, test_rounds, seed=self.seed, chain_offset=0)
+        is_sat = self.ctx.sample_fetch_sat()
+        limits, consumed = [], []
+        for i, (k, c) in enumerate(plan):
+            f = self.formulas[k]
+            used, sat_used, stop = consume_batches(is_sat[graph_seg[i]:graph_seg[i + 1]], f.batch_chains, f.still_needed,
+                                                   f.total, f.sat_total, self.min_sat_rate)
+            if stop:
+                print("too many unsat samples; stopping diffusion")
+            limits.append(used)
+            consumed.append((f, used, sat_used, stop, c))
+        if any(sat_used for _, _, sat_used, _, _ in consumed):
+            tables, _ = self.ctx.hist_reduce_segments(graph_seg, limits)       # sort / unique / count per formula on the device
+            for (f, _, sat_used, _, _), (keys, counts) in zip(consumed, tables):
+                assert int(counts.sum()) == sat_used
+                if sat_used:
+                    f.tables.append((np.ascontiguousarray(keys[:, :f.words]), counts))
+        for f, used, sat_used, stop, c in consumed:
+            f.total += used
+            f.sat_total += sat_used
+            f.still_needed -= sat_used
+            f.launched += c
+            f.stopped = f.stopped or stop

@@ -97,6 +97,17 @@ int dsat_set_graph(dsat_ctx* ctx, int n_vars, int n_clauses, int nnz,
                    int n_graphs, const int32_t* var_seg, const int32_t* clause_seg,
                    int n_chains, int group_graphs);
 
+/* Reference batches of several formulas in one launch (a disjoint union bound by dsat_set_graph).
+ * Early-exit group i = graphs [group_seg[i], group_seg[i+1]) of the context's n_chains*n_graphs graphs (replaces
+ * group_graphs); if noise_base is not NULL, the Philox element of variable v (0-based inside its graph) of graph gi is
+ * noise_base[gi] + v, and dsat_sample / dsat_sample_enqueue / dsat_model_call then require chain_offset == 0.
+ * Validated before anything changes; cleared by the next dsat_set_graph.
+ * With noise_base[gi] = (c0 + j) * n_k for copy j of a formula of n_k variables, a copy draws exactly the noise of chain
+ * c0 + j of that formula bound alone, so its samples do not depend on which formulas share the launch.  The steps_taken /
+ * loss outputs of dsat_model_call have one entry per bound group.  Finished groups are not skipped (their results are
+ * the same either way). */
+int dsat_set_batches(dsat_ctx* ctx, int n_groups, const int32_t* group_seg, const uint64_t* noise_base);
+
 /* Host-only helper (no context, no device): the index arrays dsat_set_graph takes, from the signed 1-based literals of all
  * clauses laid end to end (lens[j] literals for clause j, sum = nnz; a disjoint union passes its formulas already shifted by
  * their variable offsets, data/dimac.py:165-170,239-241).  cl_rowptr [n_clauses+1], cl_lit [nnz] (codes 2*var+sign, inside a
@@ -149,6 +160,15 @@ int dsat_spmm(dsat_ctx* ctx, int direction, const void* x_dev, void* y_dev, int 
  * these tables is diffusionsat_b200/dist.py (NCCL all-gather of keys + reduce of counts). */
 int dsat_hist_reduce(dsat_ctx* ctx, int chain_limit, uint64_t* keys_out, int64_t* counts_out, int capacity,
                      int32_t* n_unique, int32_t* n_sat);
+
+/* dsat_hist_reduce per formula: segment s = graphs [graph_seg[s], graph_seg[s+1]), of which the first limit[s]
+ * count.  Keys ascend within a segment, segments in order; seg_runs[n_segments+1] = offsets of each segment's runs.
+ * Segments are ordered and lie inside the context's graphs; graphs outside every segment do not count.  keys_out has
+ * dsat_words_per_graph words per key (a formula with fewer variables has zero high words); *n_sat = satisfied graphs
+ * counted over all segments (may be NULL).  Returns DSAT_ERR_ARG with seg_runs[n_segments] = the required capacity
+ * when capacity is too small. */
+int dsat_hist_reduce_segments(dsat_ctx* ctx, int n_segments, const int32_t* graph_seg, const int32_t* limit,
+                              uint64_t* keys_out, int64_t* counts_out, int capacity, int32_t* seg_runs, int32_t* n_sat);
 
 #ifdef __cplusplus
 }
