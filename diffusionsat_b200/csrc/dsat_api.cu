@@ -119,14 +119,9 @@ struct dsat_ctx {
     int cl_idx16_vecs = 0, lit_idx16_vecs = 0, cl_col_off = 0, lit_col_off = 0, lit_ord_off = 0;
     DevBuf<int> cl_desc, lit_desc, lit_desc4;   // standalone segment sums: row descriptors in processing order (dsat_spmm.cuh);
                                                 // the literal side keeps a 2-int4 and a 4-int4 form (chosen per shape)
-    bool use_spmm_order = true;
     std::vector<int32_t> h_cl_rowptr, h_cl_lit, h_lit_rowptr, h_lit_clause;     // host copy of the bound graph (ensure_spmm_desc)
     std::vector<float> h_deg_w, h_rev_w;
     bool spmm_desc_ready = false;
-    int spmm_minb = 0, spmm_pf = -1;     // DSAT_SPMM_MINB / DSAT_SPMM_PF: 0 / -1 = per-shape default (spmm_plan)
-    int spmm_half = -1;                  // DSAT_SPMM_HALF=0|1: half the lanes per row (two chunks per lane), -1 = per-shape default
-    int spmm_lit_dw = 0;                 // DSAT_SPMM_LIT_DW=2|4: int4 per literal-side row descriptor, 0 = per-shape default
-    bool use_idx16 = true;               // stage the 16-bit adjacency in the shared-memory gathers (DSAT_IDX16=0 disables)
 
     // activations
     bool has_buffers = false;
@@ -152,8 +147,6 @@ struct dsat_ctx {
     // whole-MLP kernels (dsat_mlp_fused.cuh): query, literal, clause, update, output
     fm::FusedMlp fused[5];
     bool fused_ready = false;
-    bool use_fused = true;
-    bool use_smem_gather = true;
     // fp32-accurate tensor-core path (dsat_mlp_x3.cuh): MLP inputs live as hi/lo bf16 planes [2][rows][ld]
     DevBuf<__nv_bfloat16> VROWp, CROWp, SPREp, H1p, H2p;
     DevBuf<__nv_bfloat16> wx[12];       // stacked hi/lo K-major weights [2N, K64] per reference layer
@@ -173,7 +166,6 @@ struct dsat_ctx {
     cudaGraphExec_t step_graph = nullptr;
     long long generation = 0, step_graph_generation = -1;   // bumped whenever a pointer or plan baked into the graph changes
     int step_graph_rounds = -1, step_graph_precision = -1, step_launches = 0;
-    bool use_graph = true;
 
     int ldv() const { return F + DSAT_AUX_PAD + 3 * Q; }
     int ldc() const { return F + 2 * Q; }
@@ -227,9 +219,6 @@ cudaError_t configure_kernels_for_device() {
     opt_in(literal_gather_smem_kernel<128, true>); opt_in(literal_gather_smem_kernel<128, false>);
     opt_in(literal_gather_smem_kernel<64, true>); opt_in(literal_gather_smem_kernel<64, false>);
     opt_in(literal_gather_smem_kernel<32, true>); opt_in(literal_gather_smem_kernel<32, false>);
-    opt_in(clause_gather_smem_f32_kernel<128, true>); opt_in(clause_gather_smem_f32_kernel<128, false>);
-    opt_in(clause_gather_smem_f32_kernel<64, true>); opt_in(clause_gather_smem_f32_kernel<64, false>);
-    opt_in(clause_gather_smem_f32_kernel<32, true>); opt_in(clause_gather_smem_f32_kernel<32, false>);
     opt_in(clause_gather_smem_f32x2_kernel<128, true>); opt_in(clause_gather_smem_f32x2_kernel<128, false>);
     opt_in(clause_gather_smem_f32x2_kernel<64, true>); opt_in(clause_gather_smem_f32x2_kernel<64, false>);
     opt_in(clause_gather_smem_f32x2_kernel<32, true>); opt_in(clause_gather_smem_f32x2_kernel<32, false>);
@@ -260,11 +249,10 @@ UnitGraphDev graph_view(const dsat_ctx* c) {
     return g;
 }
 
-// rows of finished early-exit groups are skipped when the groups consist of whole chains (DSAT_SKIP_DONE=0 turns it off).
+// rows of finished early-exit groups are skipped when the groups consist of whole chains.
 // Variable groups (dsat_set_batches) are not runs of whole chains: nothing is skipped, which changes no result.
 SkipInfo skip_info(const dsat_ctx* c) {
-    static const bool off = getenv("DSAT_SKIP_DONE") && atoi(getenv("DSAT_SKIP_DONE")) == 0;
-    if (off || c->has_batches || c->n_graphs <= 0 || c->group_graphs % c->n_graphs != 0) return SkipInfo{nullptr, 1};
+    if (c->has_batches || c->n_graphs <= 0 || c->group_graphs % c->n_graphs != 0) return SkipInfo{nullptr, 1};
     return SkipInfo{c->done.p, c->group_graphs / c->n_graphs};
 }
 
@@ -399,7 +387,6 @@ int ensure_tc_buffers(dsat_ctx* c) {
             f.p.a_box_rows = c->a_box_rows[a_op];
             f.p.qmaps = Q;
             f.p.prof = nullptr;
-            f.p.dbg = getenv("DSAT_FM_DEBUG") ? atoi(getenv("DSAT_FM_DEBUG")) : 0;   // timing experiments only, results are garbage
             f.p.out = out;
             int i = 0;
             for (const L& l : layers) {
@@ -410,24 +397,13 @@ int ensure_tc_buffers(dsat_ctx* c) {
                 if (!tc::make_bf16_map(&f.map_wp[i], l.w, l.n, K64, K64, f.p.layer[i].box_rows / 2)) return false;
                 ++i;
             }
-            {   // input ring per MLP: DSAT_A_RING is a bit mask over (query, literal, clause, update, output)
-                static const int mask = getenv("DSAT_A_RING") ? atoi(getenv("DSAT_A_RING")) : 0x1d;
-                f.stream_input = ((mask >> which) & 1) != 0;
-                // CTA pair (cta_group::2) for the literal (split mode), clause and update MLPs: measured 4 %, 7 % and 9 % faster there,
-                // 2-5 % slower for the small query and output MLPs
-                static const int pair_mask = getenv("DSAT_PAIR_MODE") ? atoi(getenv("DSAT_PAIR_MODE")) : 0xe;
-                f.pair_mode = ((pair_mask >> which) & 1) != 0;
-                // ping-pong everywhere it fits.  The clause MLP as a single CTA is the exception: there the same shared memory buys
-                // a three-slot weight ring and a four-slot input ring for one tile at a time, 2 % faster than two tiles on
-                // two-slot rings; as a CTA pair (half-height weight slots: three of them next to three input slots) two tiles
-                // in flight are 4 % faster than one
-                static const bool pp_env = getenv("DSAT_PING_PONG") != nullptr;
-                static const int pp_mask = pp_env ? atoi(getenv("DSAT_PING_PONG")) : 0x1b;
-                f.ping_pong = ((pp_mask >> which) & 1) != 0 || (!pp_env && which == FC && f.pair_mode);
-                static const int split_on = getenv("DSAT_SPLIT_MODE") ? atoi(getenv("DSAT_SPLIT_MODE")) : 1;
-                f.split_step_bias = (split_on & 2) == 0;  // DSAT_SPLIT_MODE=3: split mode with the whole bias array in shared memory (two weight slots)
-                f.split_mode = split_on != 0;       // takes effect only where every hidden layer is 512 wide (the literal MLP)
-            }
+            // input ring for all but the literal MLP, which keeps its input resident (split mode where every hidden layer is
+            // 512 wide); two tiles in flight wherever they fit
+            f.stream_input = which != FL;
+            // CTA pair (cta_group::2) for the literal (split mode), clause and update MLPs: measured 4 %, 7 % and 9 % faster there,
+            // 2-5 % slower for the small query and output MLPs; the clause pair with two tiles in flight (half-height weight
+            // slots: three of them next to three input slots) measured 4 % faster than with one
+            f.pair_mode = which == FL || which == FC || which == FU;
             if (!fm::plan_fused(f)) return false;
             if (getenv("DSAT_PLAN_LOG"))
                 fprintf(stderr, "[dsat] fused mlp %d: smem %d B (pad %d), hidden blocks %d x%d, input ring %d, weight ring %d x %d B, "
@@ -593,7 +569,6 @@ int ensure_x3_buffers(dsat_ctx* c) {
     CK_CUDA(c, cudaMemsetAsync(c->CROWp.p, 0, c->CROWp.count * 2, c->stream));
     enum { XQ = 0, XL1, XL2, XL3, XC, XU, XO };
     struct L { int wi; int op; int bias_off; int epi; };        // wi = index into wx[] (reference layer order)
-    static const int pair_mask = getenv("DSAT_X3_PAIR") ? atoi(getenv("DSAT_X3_PAIR")) : 0x3e;   // all but query and output
     auto build = [&](int which, const __nv_bfloat16* a_hi, size_t a_plane, long long rows, int k, int lda,
                      std::initializer_list<L> layers, int n_groups, int out_mode, void* out0, void* out1, int ld_out) -> bool {
         x3::X3Mlp& f = c->x3[which];
@@ -611,9 +586,7 @@ int ensure_x3_buffers(dsat_ctx* c) {
             p.done = sk.done; p.chains_per_group = sk.chains_per_group;
             p.rows_per_chain = rows == c->Mt ? c->m : c->n;
         }
-        f.pair_mode = ((pair_mask >> which) & 1) != 0;
-        static const int epi4_mask = getenv("DSAT_X3_EPI4") ? atoi(getenv("DSAT_X3_EPI4")) : 0;
-        f.four_epilogue_warps = ((epi4_mask >> which) & 1) != 0;
+        f.pair_mode = which != XQ && which != XO;       // CTA pair for all but the query and output MLPs
         if (!tc::make_bf16_map(&f.map_a_hi, a_hi, rows, k, lda, p.a_box_rows)) return false;
         if (!tc::make_bf16_map(&f.map_a_lo, a_hi + a_plane, rows, k, lda, p.a_box_rows)) return false;
         int i = 0;
@@ -820,9 +793,7 @@ int run_fused(dsat_ctx* c, int which, int prof_class) {
 // returns false when they do not fit (the L2-gather kernels run instead).
 static int pick_slice_width(size_t table_rows, int Q, size_t* bytes_out, int budget_kb, int elt_bytes) {
     // budget_kb: shared memory per CTA we aim for (smaller slices -> more co-resident CTAs, so one CTA's staging
-    // overlaps the others' compute); DSAT_GATHER_KB overrides it for experiments
-    static const int env_kb = getenv("DSAT_GATHER_KB") ? atoi(getenv("DSAT_GATHER_KB")) : 0;
-    if (env_kb > 0) budget_kb = env_kb;
+    // overlaps the others' compute)
     const int widths[3] = {128, 64, 32};
     for (int pass = 0; pass < 2; ++pass)
         for (int w : widths) {
@@ -843,13 +814,13 @@ static bool idx_fits(size_t table_bytes, int idx_vecs) {
 
 
 bool launch_clause_gather_smem(dsat_ctx* c, const UnitGraphDev& g) {
-    if (c->n_graphs != 1 || !c->use_smem_gather) return false;
+    if (c->n_graphs != 1) return false;
     size_t bytes = 0;
     const int w = pick_slice_width((size_t)2 * c->n, c->Q, &bytes, 56);    // measured best at cfg2: 4 CTAs per SM
     if (!w) return false;
     dim3 grid((unsigned)c->chains, (unsigned)(c->Q / w));
     const int Q = c->Q;
-    const bool si = c->use_idx16 && idx_fits(bytes, g.cl_idx16_vecs);
+    const bool si = idx_fits(bytes, g.cl_idx16_vecs);
     const size_t smem = bytes + (si ? (size_t)g.cl_idx16_vecs * 16 : 0);
     auto launch = [&](auto kernel) -> bool {
         kernel<<<grid, 512, smem, c->stream>>>(g, Q, c->LITb.p, 2 * Q, c->QSb.p, 3 * Q, Q, c->CROWb.p, c->ldc(), c->F, skip_info(c));
@@ -861,13 +832,13 @@ bool launch_clause_gather_smem(dsat_ctx* c, const UnitGraphDev& g) {
 }
 
 bool launch_literal_gather_smem(dsat_ctx* c, const UnitGraphDev& g) {
-    if (c->n_graphs != 1 || !c->use_smem_gather) return false;
+    if (c->n_graphs != 1) return false;
     size_t bytes = 0;
     const int w = pick_slice_width((size_t)c->m, c->Q, &bytes, 112);
     if (!w) return false;
     dim3 grid((unsigned)c->chains, (unsigned)(c->Q / w));
     const int Q = c->Q, F = c->F;
-    const bool si = c->use_idx16 && idx_fits(bytes, g.lit_idx16_vecs);
+    const bool si = idx_fits(bytes, g.lit_idx16_vecs);
     const size_t smem = bytes + (si ? (size_t)g.lit_idx16_vecs * 16 : 0);
     auto launch = [&](auto kernel) -> bool {
         kernel<<<grid, 512, smem, c->stream>>>(g, Q, c->CROWb.p, c->ldc(), F + Q, c->COUTb.p, Q + F, c->QSb.p, 3 * Q, c->VROWb.p,
@@ -883,49 +854,38 @@ bool launch_literal_gather_smem(dsat_ctx* c, const UnitGraphDev& g) {
 #ifdef DSAT_WITH_TCGEN05
 // fp32 tables (fp32-accurate tensor-core path): outputs go to the hi/lo planes
 bool launch_clause_gather_smem_f32(dsat_ctx* c, const UnitGraphDev& g) {
-    if (c->n_graphs != 1 || !c->use_smem_gather) return false;
-    // DSAT_GATHER_F32_CL1=1: one table per CTA at twice the slice width (the literal side's default) instead of both tables
-    static const bool one_table = getenv("DSAT_GATHER_F32_CL1") && atoi(getenv("DSAT_GATHER_F32_CL1")) != 0;
+    if (c->n_graphs != 1) return false;
     size_t bytes = 0;
-    static const int budget = getenv("DSAT_GATHER_F32_KB_CL") ? atoi(getenv("DSAT_GATHER_F32_KB_CL")) : 110;
-    const int w = pick_slice_width((size_t)2 * c->n, c->Q, &bytes, budget, one_table ? 2 : 4);
+    const int w = pick_slice_width((size_t)2 * c->n, c->Q, &bytes, 110, 4);       // both fp32 tables per CTA
     // one CTA per SM cannot overlap its staging with another CTA's gather: measured slower than the L2 gather (uf250)
     if (!w || bytes > 112 * 1024) return false;
-    dim3 grid((unsigned)c->chains, (unsigned)((one_table ? 2 : 1) * (c->Q / w)));
+    dim3 grid((unsigned)c->chains, (unsigned)(c->Q / w));
     const int Q = c->Q;
-    const bool si = c->use_idx16 && idx_fits(bytes, g.cl_idx16_vecs);
+    const bool si = idx_fits(bytes, g.cl_idx16_vecs);
     const size_t smem = bytes + (si ? (size_t)g.cl_idx16_vecs * 16 : 0);
     const size_t cplane = (size_t)c->Mt * c->ldc();
     auto launch = [&](auto kernel) -> bool {
         kernel<<<grid, 512, smem, c->stream>>>(g, Q, c->LIT.p, 2 * Q, c->QS.p, 3 * Q, Q, c->CROWp.p, cplane, c->ldc(), c->F, skip_info(c));
         return true;
     };
-    if (one_table) {
-        if (w == 128) return si ? launch(clause_gather_smem_f32_kernel<128, true>) : launch(clause_gather_smem_f32_kernel<128, false>);
-        if (w == 64) return si ? launch(clause_gather_smem_f32_kernel<64, true>) : launch(clause_gather_smem_f32_kernel<64, false>);
-        return si ? launch(clause_gather_smem_f32_kernel<32, true>) : launch(clause_gather_smem_f32_kernel<32, false>);
-    }
     if (w == 128) return si ? launch(clause_gather_smem_f32x2_kernel<128, true>) : launch(clause_gather_smem_f32x2_kernel<128, false>);
     if (w == 64) return si ? launch(clause_gather_smem_f32x2_kernel<64, true>) : launch(clause_gather_smem_f32x2_kernel<64, false>);
     return si ? launch(clause_gather_smem_f32x2_kernel<32, true>) : launch(clause_gather_smem_f32x2_kernel<32, false>);
 }
 
 bool launch_literal_gather_smem_f32(dsat_ctx* c, const UnitGraphDev& g) {
-    if (c->n_graphs != 1 || !c->use_smem_gather) return false;
+    if (c->n_graphs != 1) return false;
     size_t bytes = 0;
-    static const int budget = getenv("DSAT_GATHER_F32_KB_LIT") ? atoi(getenv("DSAT_GATHER_F32_KB_LIT")) : 112;
-    const int w = pick_slice_width((size_t)c->m, c->Q, &bytes, budget, 2);          // one fp32 table per CTA
+    const int w = pick_slice_width((size_t)c->m, c->Q, &bytes, 112, 2);             // one fp32 table per CTA
     if (!w || bytes > 112 * 1024) return false;     // (as on the clause side: uf250's 1065 clause rows ran 1.39 ms against 1.09 ms)
     dim3 grid((unsigned)c->chains, (unsigned)(2 * (c->Q / w)));
     const int Q = c->Q, F = c->F;
-    const bool si = c->use_idx16 && idx_fits(bytes, g.lit_idx16_vecs);
+    const bool si = idx_fits(bytes, g.lit_idx16_vecs);
     const size_t smem = bytes + (si ? (size_t)g.lit_idx16_vecs * 16 : 0);
     const size_t cplane = (size_t)c->Mt * c->ldc(), vplane = (size_t)c->Nt * c->ldv();
-    // DSAT_GATHER_F32_PLANES=0: widen 4*clauses_loss to an fp32 table while staging instead of keeping hi / lo bf16 tables
-    static const int planes_tables = getenv("DSAT_GATHER_F32_PLANES") ? atoi(getenv("DSAT_GATHER_F32_PLANES")) : 1;
     auto launch = [&](auto kernel) -> bool {
         kernel<<<grid, 512, smem, c->stream>>>(g, Q, c->CROWp.p, cplane, c->ldc(), F + Q, c->COUT.p, Q + F, c->QS.p, 3 * Q,
-                                                c->VROWp.p, vplane, c->ldv(), F + DSAT_AUX_PAD, skip_info(c), planes_tables);
+                                                c->VROWp.p, vplane, c->ldv(), F + DSAT_AUX_PAD, skip_info(c));
         return true;
     };
     if (w == 128) return si ? launch(literal_gather_smem_f32_kernel<128, true>) : launch(literal_gather_smem_f32_kernel<128, false>);
@@ -939,8 +899,6 @@ bool launch_literal_gather_smem_f32(dsat_ctx* c, const UnitGraphDev& g) {
 template <int V>
 bool launch_pairnorm_smem(dsat_ctx* c, const int* seg, int rows_per_chain, int max_graph_rows, const float* src, int ld_src, int src_off,
                           __nv_bfloat16* state_hi, size_t state_plane, int ld_state, __nv_bfloat16* pre_hi, size_t pre_plane, int ld_pre) {
-    static const bool off = getenv("DSAT_PN_SMEM") && atoi(getenv("DSAT_PN_SMEM")) == 0;
-    if (off) return false;
     constexpr int F = 32 * V;
     // small graphs: several CTAs of 256 threads per SM; large ones: one CTA of 1024 threads
     const size_t row_bytes = (size_t)max_graph_rows * F * 4;
@@ -971,7 +929,7 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
     const size_t vplane = x3p ? (size_t)Nt * ldv : 0, cplane = x3p ? (size_t)Mt * ldc : 0;
     const SkipInfo skip = skip_info(c);
 #ifdef DSAT_WITH_TCGEN05
-    const bool fusedp = tcp && c->precision == DSAT_BF16 && c->fused_ready && c->use_fused;
+    const bool fusedp = tcp && c->precision == DSAT_BF16 && c->fused_ready;
     enum { XQ = 0, XL1, XL2, XL3, XC, XU, XO };
 #endif
     int rc;
@@ -1083,16 +1041,7 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
     prof_mark(c, PROF_NORM_CLAUSE);
     rc = dispatch_width(c, F, [&](auto v) {
         constexpr int V = decltype(v)::value;
-        int grid = c->total_graphs < c->sm_count * 8 ? c->total_graphs : c->sm_count * 8;
-        {   // both passes of a CTA should find their graph in L2: cap the graphs in flight at about half of L2
-            static const int l2_mb = getenv("DSAT_PN_L2_MB") ? atoi(getenv("DSAT_PN_L2_MB")) : 0;
-            if (l2_mb > 0) {
-                const double per_graph = (double)c->m / c->n_graphs * F * (tcp ? 2 : 4);
-                int cap = (int)(l2_mb * 1048576.0 / (per_graph > 1 ? per_graph : 1));
-                cap = cap < c->sm_count ? c->sm_count : cap;
-                if (grid > cap) grid = cap;
-            }
-        }
+        const int grid = c->total_graphs < c->sm_count * 8 ? c->total_graphs : c->sm_count * 8;
         if (x3p) {
 #ifdef DSAT_WITH_TCGEN05
             if (!launch_pairnorm_smem<V>(c, c->clause_seg.p, c->m, c->max_graph_clauses, c->COUT.p, Q + F, Q, crow_b(c), cplane, ldc,
@@ -1299,28 +1248,6 @@ int dsat_create(int device, dsat_ctx** out) {
     c->stream = c->own_stream;
     cudaEventCreate(&c->ev0);
     cudaEventCreate(&c->ev1);
-#ifdef DSAT_WITH_TCGEN05
-    {   // A/B switches for measurements: DSAT_FUSED_MLP=0, DSAT_SMEM_GATHER=0
-        const char* e = getenv("DSAT_FUSED_MLP");
-        if (e && e[0] == '0') c->use_fused = false;
-        e = getenv("DSAT_SPMM_ORDER");
-        if (e) c->use_spmm_order = e[0] != '0';
-        e = getenv("DSAT_SPMM_MINB");
-        if (e) c->spmm_minb = atoi(e);
-        e = getenv("DSAT_SPMM_PF");
-        if (e) c->spmm_pf = atoi(e);
-        e = getenv("DSAT_SPMM_LIT_DW");
-        if (e) c->spmm_lit_dw = atoi(e);
-        e = getenv("DSAT_SPMM_HALF");
-        if (e) c->spmm_half = atoi(e);
-        e = getenv("DSAT_IDX16");
-        if (e) c->use_idx16 = e[0] != '0';
-        e = getenv("DSAT_SMEM_GATHER");
-        if (e && e[0] == '0') c->use_smem_gather = false;
-        e = getenv("DSAT_GRAPH");
-        if (e && e[0] == '0') c->use_graph = false;
-    }
-#endif
     *out = c;
     return DSAT_OK;
 }
@@ -1771,7 +1698,7 @@ static int sample_enqueue_impl(dsat_ctx* c, int n_steps, int n_rounds, uint64_t 
     CK_CUDA(c, cudaMemsetAsync(c->sat_any.p, 0, c->sat_any.count, c->stream));
     const uint64_t element_offset = chain_offset * (uint64_t)c->n;
     const bool injected = uniforms_dev || labels_dev || normals_dev;
-    if (c->use_graph && !injected && !c->profiling) {
+    if (!injected && !c->profiling) {
         // One denoising step is captured once and replayed n_steps times: the ~12 launches per round are issued by the
         // graph executor back to back instead of one cudaLaunchKernel each (small formulas are launch-bound: 12.5 k launches
         // per run).  Everything that differs between steps lives in step_tab[*step_cur].
@@ -1961,45 +1888,32 @@ int dsat_hist_reduce_segments(dsat_ctx* c, int n_segments, const int32_t* graph_
 }
 
 // ------------------------------------------------------------------------------------------ SpMM
-// Instantiation of spmm_rows_kernel per shape: resident CTAs per SM (= register budget) and descriptor prefetch.
-// DSAT_SPMM_MINB=4|5|6|8 and DSAT_SPMM_PF=0|1 override the table for A/B runs.
-struct SpmmPlan { int min_blocks; bool prefetch; int desc_words; bool half_lanes; };
-static SpmmPlan spmm_plan(int forced_minb, int forced_pf, int forced_lit_dw, int forced_half, int row_bytes, bool bf16,
-                          int direction) {
-    // measured on the n = 10000 sweep (profiles/r2_spmm_variants.txt).  Clause side: registers for the gathers (no spills)
-    // and, for rows of >= 512 bytes, the prefetched descriptor; bf16 rows of >= 256 bytes run with half the lanes per row
-    // (twice the gathers in flight per warp).  Literal side: the twelve-entry descriptor for rows of <= 256 bytes, the plain
-    // 32-register kernel for 512-byte fp32 rows.
-    SpmmPlan p{8, false, direction == 0 ? SPMM_DW_CLAUSE : 2, false};
+// The spmm_rows_kernel instantiation of each (direction, dtype, row bytes), measured on the n = 10000 sweep
+// (profiles/r2_spmm_variants.txt).  Clause side: registers for the gathers (no spills) and, for fp32 rows of >= 512 bytes,
+// the prefetched descriptor; bf16 rows of >= 256 bytes run with half the lanes per row (twice the gathers in flight per
+// warp).  Literal side: the twelve-entry descriptor (desc4) for rows of <= 256 bytes, the plain 32-register kernel for
+// 512-byte fp32 rows, half the lanes for 512-byte bf16 rows.
+using SpmmKernel = void (*)(const int4*, const int*, int, int, int, const void*, void*);
+struct SpmmPlan { SpmmKernel kernel; bool desc4; bool half_lanes; };
+static SpmmPlan spmm_plan(int direction, bool bf16, int row_bytes) {
     if (direction == 0) {
         if (bf16) {
-            if (row_bytes == 128) p = {6, false, 2, false};
-            else p = {4, false, 2, true};
-        } else {
-            if (row_bytes == 256) p = {8, false, 2, false};
-            else if (row_bytes == 512) p = {5, true, 2, false};
-            else p = {4, true, 2, false};
+            if (row_bytes == 128) return {spmm_rows_kernel<128, true, 6>, false, false};
+            if (row_bytes == 256) return {spmm_rows_kernel<256, true, 4, false, 2, 8>, false, true};
+            return {spmm_rows_kernel<512, true, 4, false, 2, 16>, false, true};
         }
-    } else {
-        if (bf16) {
-            if (row_bytes <= 256) p = {5, false, 4, false};
-            else p = {4, false, 2, true};
-        } else {
-            if (row_bytes == 256) p = {6, false, 4, false};
-            else if (row_bytes == 512) p = {8, false, 2, false};
-            else p = {5, false, 2, false};
-        }
+        if (row_bytes == 256) return {spmm_rows_kernel<256, false, 8>, false, false};
+        if (row_bytes == 512) return {spmm_rows_kernel<512, false, 5, true>, false, false};
+        return {spmm_rows_kernel<1024, false, 4, true>, false, false};
     }
-    const bool forced_any = forced_minb == 4 || forced_minb == 5 || forced_minb == 6 || forced_minb == 8 || forced_pf == 0 ||
-                            forced_pf == 1 || forced_lit_dw == 2 || forced_lit_dw == 4;
-    if (forced_any) p.half_lanes = false;       // an A/B run names the full-lane instantiation unless DSAT_SPMM_HALF=1
-    if (forced_minb == 4 || forced_minb == 5 || forced_minb == 6 || forced_minb == 8) p.min_blocks = forced_minb;
-    if (forced_pf == 0 || forced_pf == 1) p.prefetch = forced_pf == 1;
-    if (direction == 1 && (forced_lit_dw == 2 || forced_lit_dw == 4)) p.desc_words = forced_lit_dw;
-    if (p.desc_words == 4) p.prefetch = false;
-    if (forced_half == 0 || forced_half == 1) p.half_lanes = forced_half == 1;
-    if (p.half_lanes && row_bytes <= 512) p.desc_words = 2;
-    return p;
+    if (bf16) {
+        if (row_bytes == 128) return {spmm_rows_kernel<128, true, 5, false, 4>, true, false};
+        if (row_bytes == 256) return {spmm_rows_kernel<256, true, 5, false, 4>, true, false};
+        return {spmm_rows_kernel<512, true, 4, false, 2, 16>, false, true};
+    }
+    if (row_bytes == 256) return {spmm_rows_kernel<256, false, 6, false, 4>, true, false};
+    if (row_bytes == 512) return {spmm_rows_kernel<512, false, 8>, false, false};
+    return {spmm_rows_kernel<1024, false, 5>, false, false};
 }
 
 // Row descriptors of the standalone segment sums (dsat_spmm.cuh), built on first use after dsat_set_graph.
@@ -2017,11 +1931,10 @@ static int ensure_spmm_desc(dsat_ctx* c) {
             for (int e = rowptr[j]; e < rowptr[j + 1]; ++e) mn = col[e] < mn ? col[e] : mn;
             key[j] = mn;
         }
-        if (c->use_spmm_order)
-            std::stable_sort(ord.begin(), ord.begin() + rows, [&](int a, int b) {
-                const int la = rowptr[a + 1] - rowptr[a], lb = rowptr[b + 1] - rowptr[b];
-                return la != lb ? la > lb : key[a] < key[b];
-            });
+        std::stable_sort(ord.begin(), ord.begin() + rows, [&](int a, int b) {
+            const int la = rowptr[a + 1] - rowptr[a], lb = rowptr[b + 1] - rowptr[b];
+            return la != lb ? la > lb : key[a] < key[b];
+        });
         const size_t w = 4 * (size_t)dw;
         std::vector<int> desc(w * (size_t)(rows > 0 ? rows : 1), 0);
         for (int p = 0; p < rows; ++p) {
@@ -2062,53 +1975,11 @@ int dsat_spmm(dsat_ctx* c, int direction, const void* x_dev, void* y_dev, int fe
         c->err = "feature width must be 64, 128 or 256";
         rc = DSAT_ERR_UNSUPPORTED;
     } else {
-        const SpmmPlan plan = spmm_plan(c->spmm_minb, c->spmm_pf, c->spmm_lit_dw, c->spmm_half, row_bytes, dtype == DSAT_BF16,
-                                        direction);
-        const int4* rowdesc = reinterpret_cast<const int4*>(direction == 0 ? c->cl_desc.p
-                                                            : plan.desc_words == 4 ? c->lit_desc4.p : c->lit_desc.p);
-        auto launch = [&](auto kernel) {
-            const int rows_per_block = GATHER_WARPS * (row_bytes >= 512 ? 1 : 512 / row_bytes) * (plan.half_lanes ? 2 : 1);
-            const int grid = gather_grid(kernel, (long long)chains * rows_out, rows_per_block, c->sm_count);
-            kernel<<<grid, GATHER_WARPS * 32, 0, c->stream>>>(rowdesc, colidx, rows_out, rows_in, chains, x_dev, y_dev);
-        };
-        auto by_shape = [&](auto minb, auto pf, auto dwc) {
-            constexpr int MB = decltype(minb)::value;
-            constexpr bool PF = decltype(pf)::value;
-            constexpr int DW = decltype(dwc)::value;
-            if (dtype == DSAT_BF16) {
-                if (row_bytes == 128) launch(spmm_rows_kernel<128, true, MB, PF, DW>);
-                else if (row_bytes == 256) launch(spmm_rows_kernel<256, true, MB, PF, DW>);
-                else launch(spmm_rows_kernel<512, true, MB, PF, DW>);
-            } else {
-                if (row_bytes == 256) launch(spmm_rows_kernel<256, false, MB, PF, DW>);
-                else if (row_bytes == 512) launch(spmm_rows_kernel<512, false, MB, PF, DW>);
-                else launch(spmm_rows_kernel<1024, false, MB, PF, DW>);
-            }
-        };
-        const int dw = plan.desc_words;
-        if (plan.half_lanes && row_bytes <= 512) {      // half the lanes per row, two chunks per lane, 64 registers
-            if (dtype == DSAT_BF16) {
-                if (row_bytes == 128) launch(spmm_rows_kernel<128, true, 4, false, 2, 4>);
-                else if (row_bytes == 256) launch(spmm_rows_kernel<256, true, 4, false, 2, 8>);
-                else launch(spmm_rows_kernel<512, true, 4, false, 2, 16>);
-            } else {
-                if (row_bytes == 256) launch(spmm_rows_kernel<256, false, 4, false, 2, 8>);
-                else launch(spmm_rows_kernel<512, false, 4, false, 2, 16>);
-            }
-            LAUNCHED(c);
-            return DSAT_OK;
-        }
-        auto by_pf = [&](auto minb) {
-            if (dw == 4) by_shape(minb, std::false_type{}, std::integral_constant<int, 4>{});
-            else if (plan.prefetch) by_shape(minb, std::true_type{}, std::integral_constant<int, 2>{});
-            else by_shape(minb, std::false_type{}, std::integral_constant<int, 2>{});
-        };
-        switch (plan.min_blocks) {
-            case 4: by_pf(std::integral_constant<int, 4>{}); break;
-            case 5: by_pf(std::integral_constant<int, 5>{}); break;
-            case 6: by_pf(std::integral_constant<int, 6>{}); break;
-            default: by_pf(std::integral_constant<int, 8>{}); break;
-        }
+        const SpmmPlan plan = spmm_plan(direction, dtype == DSAT_BF16, row_bytes);
+        const int4* rowdesc = reinterpret_cast<const int4*>(direction == 0 ? c->cl_desc.p : plan.desc4 ? c->lit_desc4.p : c->lit_desc.p);
+        const int rows_per_block = GATHER_WARPS * (row_bytes >= 512 ? 1 : 512 / row_bytes) * (plan.half_lanes ? 2 : 1);
+        const int grid = gather_grid(plan.kernel, (long long)chains * rows_out, rows_per_block, c->sm_count);
+        plan.kernel<<<grid, GATHER_WARPS * 32, 0, c->stream>>>(rowdesc, colidx, rows_out, rows_in, chains, x_dev, y_dev);
     }
     if (rc) return rc;
     LAUNCHED(c);
@@ -2447,7 +2318,7 @@ int dsat_debug_mlp(dsat_ctx* c, int which) {
             case 3: rc = run_x3(c, XU, OP_U3); break;
             default: rc = run_x3(c, XO, OP_O2); break;
         }
-    } else if (use_tc(c) && c->precision == DSAT_BF16 && c->fused_ready && c->use_fused) {
+    } else if (use_tc(c) && c->precision == DSAT_BF16 && c->fused_ready) {
         static const int cls[5] = {OP_Q2, OP_L3, OP_C2, OP_U3, OP_O2};
         rc = run_fused(c, which, cls[which]);
     } else if (use_tc(c)) {

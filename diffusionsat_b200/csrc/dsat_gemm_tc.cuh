@@ -140,17 +140,6 @@ __device__ __forceinline__ void mbar_arrive_at(uint32_t cluster_addr) {
     // (tcgen05.fence::before_thread_sync); nothing of it is read by threads of the other CTA
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-__device__ __forceinline__ void mbar_wait_cluster_scope(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_LOOP_CS:\n"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra WAIT_DONE_CS;\n"
-        "bra WAIT_LOOP_CS;\n"
-        "WAIT_DONE_CS:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
 // TMA load into THIS CTA's shared memory whose completion is signalled on a barrier given by its shared::cluster address
 __device__ __forceinline__ void tma_load_2d_cg2(void* smem_dst, const CUtensorMap* map, uint32_t bar_cluster_addr, int c0, int c1) {
     asm volatile(

@@ -434,9 +434,6 @@ literal_gather_smem_kernel(UnitGraphDev g, int Q,
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
     const int sub = lane / LPR, li = lane % LPR;
     const size_t cbase = (size_t)chain * g.m;
-#ifdef DSAT_GATHER_TRACE
-    const long long t_start = clock64();
-#endif
     if (ld_cl == W && ld_msg == W) {   // dense [m, W] tables (Q == W): constant row pitch
         stage_rows_async<T>(t_cl, CL4 + cbase * W + cl_off, g.m, W, W, tid, blockDim.x);
         stage_rows_async<T>(t_ms, MSG + cbase * W, g.m, W, W, tid, blockDim.x);
@@ -449,13 +446,7 @@ literal_gather_smem_kernel(UnitGraphDev g, int Q,
         for (int i = tid; i < g.lit_idx16_vecs; i += blockDim.x) d[i] = __ldg(reinterpret_cast<const uint4*>(g.lit_idx16) + i);
     }
     cp_async_wait_all();
-#ifdef DSAT_GATHER_TRACE
-    const long long t_staged = clock64();
-#endif
     __syncthreads();
-#ifdef DSAT_GATHER_TRACE
-    const long long t_sync = clock64();
-#endif
     // variables are taken in order of descending degree: the RPW rows of a pass then have similar entry counts (a
     // pass runs for its longest row), and the heaviest passes are dealt first
     for (int v0 = warp * RPW; v0 < g.n; v0 += nwarps * RPW) {
@@ -521,11 +512,6 @@ literal_gather_smem_kernel(UnitGraphDev g, int Q,
             reinterpret_cast<uint4*>(dst)[li] = pack8(grad);
         }
     }
-#ifdef DSAT_GATHER_TRACE
-    if (slice == 0 && (chain == 1500 || chain == 3000) && (tid == 0 || tid == 511))
-        printf("literal gather chain %d tid %d: stage %lld  wait %lld  gather %lld cycles\n", chain, tid, t_staged - t_start,
-               t_sync - t_staged, clock64() - t_sync);
-#endif
 }
 
 // ------------------------------------------------------------------ fp32 tables (fp32-accurate tensor-core path)
@@ -541,82 +527,6 @@ __device__ __forceinline__ void store_split4(__nv_bfloat16* dst_hi, size_t plane
     split_bf16x2(f[2], f[3], hi.y, lo.y);
     reinterpret_cast<uint2*>(dst_hi)[li] = hi;
     reinterpret_cast<uint2*>(dst_hi + plane)[li] = lo;
-}
-
-// One table per CTA: blockIdx.y = slice * 2 + role.  The two sums of a side are independent, so a CTA stages only ONE of
-// the two tables and can afford a slice twice as wide: the adjacency walk (index loads, address arithmetic) is amortised
-// over twice the features -- these kernels are issue-bound, not bandwidth-bound -- and the rows it fetches are twice as
-// long (512-byte segments on the clause side).
-//   clause side  role 0: table LIT -> clause_messages            role 1: table softplus pair -> 4*clauses_loss
-//   literal side role 0: table 4*clauses_loss -> variables_grad   role 1: table messages -> loss_pos | loss_neg
-template <int W, bool SI>
-__global__ void __launch_bounds__(512, 2)
-clause_gather_smem_f32_kernel(UnitGraphDev g, int Q,
-                              const float* __restrict__ LIT, int ld_lit,
-                              const float* __restrict__ SP, int ld_sp, int sp_off,
-                              __nv_bfloat16* __restrict__ OUT_HI, size_t out_plane, int ld_out, int out_off, SkipInfo skip = SkipInfo{nullptr, 1}) {
-    if (chain_done(skip, (int)blockIdx.x)) return;     // the whole CTA works on one chain
-    constexpr int LPR = W / 4, RPW = 32 / LPR;
-    extern __shared__ __align__(16) uint8_t gsm[];
-    float* tab = reinterpret_cast<float*>(gsm);
-    const unsigned short* s_idx = reinterpret_cast<const unsigned short*>(tab + (size_t)2 * g.n * W);
-    const int chain = blockIdx.x, slice = blockIdx.y >> 1, role = blockIdx.y & 1;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
-    const int sub = lane / LPR, li = lane % LPR;
-    const size_t vbase = (size_t)chain * g.n;
-    {
-        const float* src = role ? SP + sp_off : LIT;
-        const int ld = role ? ld_sp : ld_lit;
-        const int total = 2 * g.n * LPR;                    // (variable, sign, 16-byte piece)
-        for (int i = tid; i < total; i += blockDim.x) {
-            const int code = i / LPR, k = i % LPR, v = code >> 1, sgn = code & 1;
-            cp_async16(reinterpret_cast<uint4*>(tab + (size_t)code * W) + k,
-                       reinterpret_cast<const uint4*>(src + (vbase + v) * ld + sgn * Q + slice * W) + k);
-        }
-    }
-    if constexpr (SI) {
-        uint4* d = reinterpret_cast<uint4*>(const_cast<unsigned short*>(s_idx));
-        for (int i = tid; i < g.cl_idx16_vecs; i += blockDim.x) d[i] = __ldg(reinterpret_cast<const uint4*>(g.cl_idx16) + i);
-    }
-    cp_async_wait_all();
-    __syncthreads();
-    for (int j0 = warp * RPW; j0 < g.m; j0 += nwarps * RPW) {
-        const int j = j0 + sub;
-        const bool live = j < g.m;
-        int e0 = 0, e1 = 0;
-        if (live) {
-            if constexpr (SI) { e0 = s_idx[j]; e1 = s_idx[j + 1]; }
-            else { e0 = __ldg(g.cl_rowptr + j); e1 = __ldg(g.cl_rowptr + j + 1); }
-        }
-        Acc4 acc = {{0.f, 0.f, 0.f, 0.f}};
-        int e = e0;
-        for (; e + 3 <= e1; e += 3) {
-            const int c0 = SI ? (int)s_idx[g.cl_col_off + e] : __ldg(g.cl_lit + e);
-            const int c1 = SI ? (int)s_idx[g.cl_col_off + e + 1] : __ldg(g.cl_lit + e + 1);
-            const int c2 = SI ? (int)s_idx[g.cl_col_off + e + 2] : __ldg(g.cl_lit + e + 2);
-            DSAT_CHECK((unsigned)c0 < 2u * g.n && (unsigned)c1 < 2u * g.n && (unsigned)c2 < 2u * g.n && e + 3 <= g.nnz);
-            const float4 l0 = reinterpret_cast<const float4*>(tab + (size_t)c0 * W)[li];
-            const float4 l1 = reinterpret_cast<const float4*>(tab + (size_t)c1 * W)[li];
-            const float4 l2 = reinterpret_cast<const float4*>(tab + (size_t)c2 * W)[li];
-            acc4_add(acc, l0); acc4_add(acc, l1); acc4_add(acc, l2);
-        }
-        for (; e < e1; ++e) {
-            const int code = SI ? (int)s_idx[g.cl_col_off + e] : __ldg(g.cl_lit + e);
-            acc4_add(acc, reinterpret_cast<const float4*>(tab + (size_t)code * W)[li]);
-        }
-        if (live) {
-            float o[4];
-            if (role) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i) o[i] = 4.0f * expf(-acc.v[i]);
-            } else {
-                const float rw = __ldg(g.rev_w + j);
-#pragma unroll
-                for (int i = 0; i < 4; ++i) o[i] = acc.v[i] * rw;
-            }
-            store_split4(OUT_HI + ((size_t)chain * g.m + j) * ld_out + out_off + role * Q + slice * W, out_plane, li, o);
-        }
-    }
 }
 
 // Role 0 of the literal side with the hi / lo planes of 4*clauses_loss kept as TWO bf16 tables (the same bytes as one fp32
@@ -705,57 +615,32 @@ __device__ __forceinline__ void literal_grad_from_planes(const UnitGraphDev& g, 
     }
 }
 
+// One table per CTA: blockIdx.y = slice * 2 + role.  The two sums of the literal side are independent, so a CTA stages only
+// ONE of the two tables and can afford a slice twice as wide: the adjacency walk (index loads, address arithmetic) is
+// amortised over twice the features -- these kernels are issue-bound, not bandwidth-bound.
+//   role 0: tables 4*clauses_loss (hi / lo) -> variables_grad (literal_grad_from_planes)
+//   role 1: table messages -> loss_pos | loss_neg
 template <int W, bool SI>
 __global__ void __launch_bounds__(512, 2)
 literal_gather_smem_f32_kernel(UnitGraphDev g, int Q,
                                const __nv_bfloat16* __restrict__ CL4_HI, size_t cl_plane, int ld_cl, int cl_off,
                                const float* __restrict__ MSG, int ld_msg,
                                const float* __restrict__ QRY, int ld_q,
-                               __nv_bfloat16* __restrict__ OUT_HI, size_t out_plane, int ld_out, int out_off, SkipInfo skip = SkipInfo{nullptr, 1},
-                               int planes_as_tables = 1) {
+                               __nv_bfloat16* __restrict__ OUT_HI, size_t out_plane, int ld_out, int out_off, SkipInfo skip = SkipInfo{nullptr, 1}) {
     if (chain_done(skip, (int)blockIdx.x)) return;     // the whole CTA works on one chain
     constexpr int LPR = W / 4, RPW = 32 / LPR;
     extern __shared__ __align__(16) uint8_t gsm[];
-    float* tab = reinterpret_cast<float*>(gsm);
-    const unsigned short* s_idx = reinterpret_cast<const unsigned short*>(tab + (size_t)g.m * W);
-    const int chain = blockIdx.x, slice = blockIdx.y >> 1, role = blockIdx.y & 1;
-    if (role == 0 && planes_as_tables) {
+    const int chain = blockIdx.x, slice = blockIdx.y >> 1;
+    if ((blockIdx.y & 1) == 0) {
         literal_grad_from_planes<W, SI>(g, Q, CL4_HI, cl_plane, ld_cl, cl_off, QRY, ld_q, OUT_HI, out_plane, ld_out, out_off, gsm, chain, slice);
         return;
     }
+    float* tab = reinterpret_cast<float*>(gsm);
+    const unsigned short* s_idx = reinterpret_cast<const unsigned short*>(tab + (size_t)g.m * W);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
     const int sub = lane / LPR, li = lane % LPR;
     const size_t cbase = (size_t)chain * g.m;
-    if (role) {
-        stage_rows_async<float>(tab, MSG + cbase * ld_msg + slice * W, g.m, ld_msg, W, tid, blockDim.x);
-    } else {   // 4*clauses_loss = hi + lo, widened while staging (8 features per piece; four pieces in flight per thread)
-        constexpr int PPR = W / 8;
-        const int total = g.m * PPR;
-        const __nv_bfloat16* src = CL4_HI + cbase * ld_cl + cl_off + slice * W;
-        for (int i0 = tid; i0 < total; i0 += 4 * blockDim.x) {
-            uint4 hi[4], lo[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int i = i0 + u * blockDim.x;
-                if (i < total) {
-                    const __nv_bfloat16* p = src + (size_t)(i / PPR) * ld_cl + (i % PPR) * 8;
-                    hi[u] = ldg_stream(reinterpret_cast<const uint4*>(p));
-                    lo[u] = ldg_stream(reinterpret_cast<const uint4*>(p + cl_plane));
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int i = i0 + u * blockDim.x;
-                if (i < total) {
-                    float a[8], b[8];
-                    unpack8(hi[u], a); unpack8(lo[u], b);
-                    float4* d = reinterpret_cast<float4*>(tab + (size_t)(i / PPR) * W + (i % PPR) * 8);
-                    d[0] = make_float4(a[0] + b[0], a[1] + b[1], a[2] + b[2], a[3] + b[3]);
-                    d[1] = make_float4(a[4] + b[4], a[5] + b[5], a[6] + b[6], a[7] + b[7]);
-                }
-            }
-        }
-    }
+    stage_rows_async<float>(tab, MSG + cbase * ld_msg + slice * W, g.m, ld_msg, W, tid, blockDim.x);
     if constexpr (SI) {
         uint4* d = reinterpret_cast<uint4*>(const_cast<unsigned short*>(s_idx));
         for (int i = tid; i < g.lit_idx16_vecs; i += blockDim.x) d[i] = __ldg(reinterpret_cast<const uint4*>(g.lit_idx16) + i);
@@ -768,12 +653,8 @@ literal_gather_smem_f32_kernel(UnitGraphDev g, int Q,
         if (live) v = SI ? (int)s_idx[g.lit_ord_off + v0 + sub] : __ldg(g.var_order + v0 + sub);
         const size_t row = (size_t)chain * g.n + v;
         __nv_bfloat16* dst = OUT_HI + row * ld_out + out_off + slice * W;
-        float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
-        float vw = 0.f, dw[2] = {0.f, 0.f};
-        if (live) {
-            if (role) { dw[0] = __ldg(g.deg_w + 2 * v); dw[1] = __ldg(g.deg_w + 2 * v + 1); }
-            else { q = __ldg(reinterpret_cast<const float4*>(QRY + row * ld_q + slice * W) + li); vw = __ldg(g.vdeg_w + v); }
-        }
+        float dw[2] = {0.f, 0.f};
+        if (live) { dw[0] = __ldg(g.deg_w + 2 * v); dw[1] = __ldg(g.deg_w + 2 * v + 1); }
         Acc4 sum[2];
 #pragma unroll
         for (int sgn = 0; sgn < 2; ++sgn) {
@@ -800,23 +681,12 @@ literal_gather_smem_f32_kernel(UnitGraphDev g, int Q,
             sum[sgn] = acc;
         }
         if (!live) continue;
-        if (role) {
 #pragma unroll
-            for (int sgn = 0; sgn < 2; ++sgn) {
-                float o[4];
+        for (int sgn = 0; sgn < 2; ++sgn) {
+            float o[4];
 #pragma unroll
-                for (int i = 0; i < 4; ++i) o[i] = sum[sgn].v[i] * dw[sgn];
-                store_split4(dst + (1 + sgn) * Q, out_plane, li, o);
-            }
-        } else {
-            const float qv[4] = {q.x, q.y, q.z, q.w};
-            float grad[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float sg = sigmoid_f(qv[i]), sgn_ = sigmoid_f(-qv[i]);
-                grad[i] = (-sg * sum[0].v[i] + sgn_ * sum[1].v[i]) * vw;
-            }
-            store_split4(dst, out_plane, li, grad);
+            for (int i = 0; i < 4; ++i) o[i] = sum[sgn].v[i] * dw[sgn];
+            store_split4(dst + (1 + sgn) * Q, out_plane, li, o);
         }
     }
 }

@@ -41,9 +41,6 @@ constexpr int STAGE_ROW = 128 + 16;                        // bytes per staged r
 constexpr int BAR_BYTES = 512;
 constexpr int MAX_A_SLOTS = 8;
 constexpr int SMEM_LIMIT = 227 * 1024;
-#ifndef DSAT_EPI_SERIAL_HIDDEN
-#define DSAT_EPI_SERIAL_HIDDEN 0      // 1: hidden epilogues drain TMEM one chunk at a time (no second register buffer)
-#endif
 
 struct FmLayer {
     int K, N;              // multiples of 16; N <= 512
@@ -65,7 +62,6 @@ struct FmParams {
     int n_layers;
     FmLayer layer[MAX_LAYERS];
     int rows, n_tiles, a_box_rows, ah_blocks, slots, slot_bytes, two_bufs, qmaps;
-    int dbg;               // experiments only (DSAT_FM_DEBUG): bit 0 = epilogues do no work (results are garbage)
     int pair;              // CTA-pair mode (cluster of 2, cta_group::2): host-side flag, the kernel is a separate instantiation
     int pp;                // ping-pong: two tiles in flight (needs a_slots > 0 and two_bufs)
     int stage_in_h;        // the output staging of a tile aliases its (by then dead) hidden region, at byte offset stage_off
@@ -75,9 +71,8 @@ struct FmParams {
     int bias_total;        // floats in the shared bias array
     int smem_pad;          // bytes the plan reserved for aligning the dynamic shared memory base to 1024
     int epi_warps;         // 4 or 8 epilogue warps: with 8, two warps share a TMEM lane quadrant and alternate 32-column chunks
-    int step_bias;         // split mode: only the current step's biases are in shared memory (2 x 256 floats, staged per step):
-                           // the space of the whole bias array buys a third weight slot
-    int split;             // split mode (fused_mlp_split_kernel): 512-wide layers run as two 256-column steps, see below
+    int split;             // split mode (fused_mlp_split_kernel): 512-wide layers run as two 256-column steps, see below;
+                           // only the current step's biases are in shared memory (2 x 256 floats, staged per step)
     int n_steps;
     FmStep step[MAX_STEPS];
     TcOut out;
@@ -261,7 +256,6 @@ struct EpiCtx {           // loop-invariant scalars of one (tile, layer) epilogu
     int N, epi, cpar, cstep, r, lane, qmaps, stage_row;
     size_t row_first; int rows_left;
     void* ptr0; void* ptr1; int ld0, ld1, bf0, bf1, split;
-    bool skip;
 };
 
 template <bool HIDDEN>
@@ -333,11 +327,7 @@ __device__ __forceinline__ void warp_arrive(uint32_t addr, int lane) {
 template <bool HIDDEN, bool PAIR>
 __device__ __forceinline__ void epi_drain(const EpiCtx& e, uint32_t tmem_empty_addr) {
     bool released = false;
-    if (e.skip) {          // timing experiment: hand everything back without touching the accumulator
-        if (!HIDDEN) { tc::tcgen05_fence_before(); warp_arrive<PAIR>(tmem_empty_addr, e.lane); }
-        return;
-    }
-    if constexpr (!HIDDEN || DSAT_EPI_SERIAL_HIDDEN) {
+    if constexpr (!HIDDEN) {
 #pragma unroll 1
         for (int c = 32 * e.cpar; c < e.N; c += e.cstep) {
             uint32_t ra[32];
@@ -413,7 +403,6 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     // arrival from the leader's multicast commit.
     const uint32_t rank = PAIR ? cluster_rank() : 0u;
     const bool leader = rank == 0;
-    const bool pair_wait_cta_scope = (p.dbg & 2) == 0;      // DSAT_FM_DEBUG=2: the old cluster-scope waits everywhere
     constexpr int NC = PAIR ? 2 : 1;
     if (threadIdx.x == 0) {
         mbar_init(a_full, NC);
@@ -452,17 +441,10 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     tcgen05_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int n_layers = p.n_layers;
-    auto wait = [&](uint64_t* bar, uint32_t parity) {
-        if constexpr (PAIR) { if (pair_wait_cta_scope) mbar_wait(bar, parity); else mbar_wait_cluster_scope(bar, parity); }
-        else mbar_wait(bar, parity);
-    };
-    // Barriers completed by TMA transactions or tcgen05.commit order async-proxy work on both sides and need no cluster-scope
-    // acquire by the waiting thread; only the barriers the peer's epilogue THREADS arrive on (tmem_empty, h_full) do.  (With a
-    // cluster-scope try_wait on every ring slot the pair instantiation spent ~2 k cycles per k-block.)
-    auto wait_async = [&](uint64_t* bar, uint32_t parity) {
-        if constexpr (PAIR) { if (pair_wait_cta_scope) mbar_wait(bar, parity); else mbar_wait_cluster_scope(bar, parity); }
-        else mbar_wait(bar, parity);
-    };
+    // Every wait, in CTA-pair mode too, acquires at CTA scope: barriers completed by TMA transactions or tcgen05.commit order
+    // async-proxy work on both sides, and the peer's epilogue threads arrive on tmem_empty / h_full only for what this CTA's
+    // tensor core reads (tc::mbar_arrive_at).  (With a cluster-scope try_wait on every ring slot the pair instantiation
+    // spent ~2 k cycles per k-block.)
     // address of the barrier the leader's issue warp waits on (this CTA's own one when not paired)
     auto at_leader = [&](uint64_t* bar) -> uint32_t { return PAIR ? mapa_rank(smem_u32(bar), 0) : smem_u32(bar); };
     // This CTA's tiles are blockIdx.x + j * gridDim.x, j < nt.  All three roles walk the same sequence of
@@ -513,7 +495,7 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                         if (j0 + s >= nt) continue;
                         const int j = j0 + s, tile = tile_of(j);
                         if (l == 0 && p.a_slots == 0) {      // whole input tile into AH
-                            if (j > 0) DSAT_TIMED_WAIT(w0, wait_async(ah_free, (uint32_t)((j - 1) & 1)));   // tile j-1 no longer reads AH
+                            if (j > 0) DSAT_TIMED_WAIT(w0, mbar_wait(ah_free, (uint32_t)((j - 1) & 1)));   // tile j-1 no longer reads AH
                             expect(a_full, (uint32_t)(k0_blocks * p.a_box_rows) * (BLOCK_K * 2));
                             for (int kb = 0; kb < k0_blocks; ++kb) load_a_block(ah + (size_t)kb * AH_BLOCK_BYTES, a_full, kb, tile);
                         }
@@ -521,13 +503,13 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                         const int halves = (p.layer[l].N + 255) / 256;
                         for (int kb = 0; kb < kbs; ++kb) {
                             if (l == 0 && p.a_slots > 0) {     // input block kb of this tile into the input ring
-                                DSAT_TIMED_WAIT(w0, wait_async(&a_ring_empty[aslot], aphase ^ 1));
+                                DSAT_TIMED_WAIT(w0, mbar_wait(&a_ring_empty[aslot], aphase ^ 1));
                                 expect(&a_ring_full[aslot], (uint32_t)p.a_box_rows * (BLOCK_K * 2));
                                 load_a_block(a_ring + (size_t)aslot * AH_BLOCK_BYTES, &a_ring_full[aslot], kb, tile);
                                 if (++aslot == p.a_slots) { aslot = 0; aphase ^= 1; }
                             }
                             for (int h = 0; h < halves; ++h) {
-                                DSAT_TIMED_WAIT(w1, wait_async(&ring_empty[slot], phase ^ 1));
+                                DSAT_TIMED_WAIT(w1, mbar_wait(&ring_empty[slot], phase ^ 1));
                                 if constexpr (PAIR) {     // this CTA's half of the weight block: rows [h*256 + rank*bn/2, +bn/2) of W^T
                                     const int bn = min(256, p.layer[l].N - h * 256);
                                     expect(&ring_full[slot], (uint32_t)(bn / 2) * (BLOCK_K * 2));
@@ -555,10 +537,10 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                         if (j0 + s >= nt) continue;
                         const Step st = make_step(j0, s, l);
                         const int j = j0 + s;
-                        DSAT_TIMED_WAIT(w0, wait(&tmem_empty[st.buf], (uint32_t)((st.use & 1) ^ 1)));   // accumulator drained
+                        DSAT_TIMED_WAIT(w0, mbar_wait(&tmem_empty[st.buf], (uint32_t)((st.use & 1) ^ 1)));   // accumulator drained
                         const bool streamed = l == 0 && p.a_slots > 0;
-                        if (l == 0) { if (!streamed) DSAT_TIMED_WAIT(w1, wait_async(a_full, (uint32_t)(j & 1))); }
-                        else DSAT_TIMED_WAIT(w2, wait(&h_full[st.hidx], (uint32_t)(st.hcnt & 1)));
+                        if (l == 0) { if (!streamed) DSAT_TIMED_WAIT(w1, mbar_wait(a_full, (uint32_t)(j & 1))); }
+                        else DSAT_TIMED_WAIT(w2, mbar_wait(&h_full[st.hidx], (uint32_t)(st.hcnt & 1)));
                         tcgen05_fence_after();
                         const int K = p.layer[l].K, N = p.layer[l].N;
                         const int kbs = (K + BLOCK_K - 1) / BLOCK_K;
@@ -569,14 +551,14 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                         for (int kb = 0; kb < kbs; ++kb) {
                             // (no tcgen05 fence after the ring waits: TMA writes and MMA reads are both async-proxy accesses
                             //  ordered by the mbarrier; the fences that matter are the per-step ones above)
-                            if (streamed) { DSAT_TIMED_WAIT(w1, wait_async(&a_ring_full[aslot], aphase)); }
+                            if (streamed) { DSAT_TIMED_WAIT(w1, mbar_wait(&a_ring_full[aslot], aphase)); }
                             const uint64_t da = make_smem_desc_sw128(smem_u32(streamed ? a_ring + (size_t)aslot * AH_BLOCK_BYTES
                                                                                        : a_src + (size_t)kb * AH_BLOCK_BYTES));
                             const int ksteps = min(BLOCK_K / 16, (K - kb * BLOCK_K + 15) / 16);
                             for (int h = 0; h < halves; ++h) {
                                 const int bn = min(256, N - h * 256);
                                 const uint32_t idesc = make_idesc_bf16(PAIR ? 2 * BLOCK_M : BLOCK_M, bn);
-                                DSAT_TIMED_WAIT(w3, wait_async(&ring_full[slot], phase));
+                                DSAT_TIMED_WAIT(w3, mbar_wait(&ring_full[slot], phase));
                                 const uint64_t db = make_smem_desc_sw128(smem_u32(ring + (size_t)slot * p.slot_bytes));
                                 const long long t_i0 = timing ? clock64() : 0;
                                 const uint32_t acc_h = acc + (uint32_t)(h * 256);
@@ -614,7 +596,6 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         e.cstep = 32 * (p.epi_warps >> 2);
         e.stage_row = p.stage_row;
         e.qmaps = p.qmaps;
-        e.skip = (p.dbg & 1) != 0;
         e.ptr0 = p.out.ptr0; e.ptr1 = p.out.ptr1; e.ld0 = p.out.ld0; e.ld1 = p.out.ld1;
         e.bf0 = p.out.bf16_0; e.bf1 = p.out.bf16_1; e.split = p.out.split;
         const uint32_t bias_addr0 = smem_u32(bias_s);
@@ -632,7 +613,7 @@ fused_mlp_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                     e.N = p.layer[l].N; e.epi = p.layer[l].epi;
                     e.bl_addr = bias_addr0 + 4u * (uint32_t)p.layer[l].bias_off;
                     e.lane_addr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(st.buf * 256);
-                    DSAT_TIMED_WAIT(w0, wait_async(&tmem_full[st.buf], (uint32_t)(st.use & 1)));
+                    DSAT_TIMED_WAIT(w0, mbar_wait(&tmem_full[st.buf], (uint32_t)(st.use & 1)));
                     tcgen05_fence_after();
                     const long long t_epi0 = timing ? clock64() : 0;
                     const uint32_t empty_addr = at_leader(&tmem_empty[st.buf]);
@@ -745,10 +726,6 @@ fused_mlp_split_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
             asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
         }
     }
-    if (!p.step_bias && warp >= 2) {
-        for (int l = 0; l < p.n_layers; ++l)
-            for (int i = threadIdx.x - 64; i < p.layer[l].N; i += epi_threads) bias_s[p.layer[l].bias_off + i] = __ldg(p.layer[l].bias + i);
-    }
     tcgen05_fence_before();
     __syncthreads();
     if constexpr (PAIR) cluster_sync_all();              // both CTAs' barriers exist before any remote arrive
@@ -845,13 +822,11 @@ fused_mlp_split_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
         e.cstep = 32 * (p.epi_warps >> 2);
         e.stage_row = p.stage_row;
         e.qmaps = p.qmaps;
-        e.skip = (p.dbg & 1) != 0;
         e.ptr0 = p.out.ptr0; e.ptr1 = p.out.ptr1; e.ld0 = p.out.ld0; e.ld1 = p.out.ld1;
         e.bf0 = p.out.bf16_0; e.bf1 = p.out.bf16_1; e.split = p.out.split;
-        const uint32_t bias_addr0 = smem_u32(bias_s);
         const uint32_t stage_off = (uint32_t)(warp - 2) * (32 * p.stage_row);
         e.stage_addr = (p.stage_in_h ? smem_u32(ah) + (uint32_t)p.stage_off : smem_u32(stage_all)) + stage_off;
-        // step_bias: the biases of the step after this one travel from global memory into registers while this step
+        // the biases of the step after this one travel from global memory into registers while this step
         // is processed, and into one of two 256-float shared buffers at the start of their step
         const int et = (int)threadIdx.x - 64;
         float bnext[2] = {0.f, 0.f};
@@ -863,7 +838,7 @@ fused_mlp_split_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                 bnext[k] = i < s.N ? __ldg(p.layer[s.layer].bias + s.n0 + i) : 0.f;
             }
         };
-        if (p.step_bias && nt > 0) fetch_bias(0);
+        if (nt > 0) fetch_bias(0);
         for (int j = 0; j < nt; ++j) {
             const int tile = tile_of(j);
             e.row_first = (size_t)tile * BLOCK_M + quad * 32;
@@ -872,18 +847,15 @@ fused_mlp_split_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_c
                 const FmStep st = p.step[v];
                 const int g = j * nv + v, buf = g & 1, use = g >> 1;
                 e.N = st.N; e.epi = p.layer[st.layer].epi;
-                if (p.step_bias) {
-                    float* dst = bias_s + (g & 1) * 256;      // last read two steps ago; every warp passed the previous step's barrier since
+                float* dst = bias_s + (g & 1) * 256;      // last read two steps ago; every warp passed the previous step's barrier since
 #pragma unroll
-                    for (int k = 0; k < 2; ++k) {
-                        const int i = et + k * epi_threads;
-                        if (i < 256) dst[i] = bnext[k];
-                    }
-                    fetch_bias(v + 1 < nv ? v + 1 : 0);
-                    asm volatile("bar.sync 2, %0;" ::"r"(epi_threads) : "memory");
-                    e.bl_addr = smem_u32(dst);
-                } else
-                e.bl_addr = bias_addr0 + 4u * (uint32_t)(p.layer[st.layer].bias_off + st.n0);
+                for (int k = 0; k < 2; ++k) {
+                    const int i = et + k * epi_threads;
+                    if (i < 256) dst[i] = bnext[k];
+                }
+                fetch_bias(v + 1 < nv ? v + 1 : 0);
+                asm volatile("bar.sync 2, %0;" ::"r"(epi_threads) : "memory");
+                e.bl_addr = smem_u32(dst);
                 e.ah_addr = smem_u32(ah) + (uint32_t)(st.n0 >> 6) * AH_BLOCK_BYTES;
                 e.lane_addr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * 256);
                 mbar_wait(&tmem_full[buf], (uint32_t)(use & 1));
@@ -920,9 +892,6 @@ struct FusedMlp {
     int smem_bytes;
     CUtensorMap map_wp[MAX_LAYERS];     // weight maps with half-height boxes (CTA-pair mode: each CTA loads half a block)
     bool stream_input = false;      // request the input ring (FmParams::a_slots), set before plan_fused
-    bool ping_pong = false;         // request two tiles in flight (FmParams::pp); needs stream_input
-    bool split_step_bias = true;    // split mode stages biases per step (room for one more weight slot)
-    bool split_mode = false;        // request split mode (fused_mlp_split_kernel) for MLPs with 512-wide hidden layers
     bool pair_mode = false;         // request the CTA-pair instantiation: half-height weight slots (map_wp), clusters of 2
 };
 
@@ -952,17 +921,10 @@ inline int dyn_smem_pad() {
     return pad;
 }
 
-inline int pair_a_slots() {
-    static const int v = getenv("DSAT_PAIR_A_SLOTS") ? atoi(getenv("DSAT_PAIR_A_SLOTS")) : 4;
-    return v < 2 ? 2 : v;
-}
-
-inline int pair_pp_wmin() {
-    // half-height weight slots reserved before the input ring gets the rest (CTA pair + ping-pong): the update MLP measured
-    // 0.263 / 0.230 / 0.245 ms with 4 / 3 / 2 (input ring 2 / 3 / 4)
-    static const int v = getenv("DSAT_PAIR_PP_WMIN") ? atoi(getenv("DSAT_PAIR_PP_WMIN")) : 3;
-    return v < 2 ? 2 : v;
-}
+constexpr int PAIR_A_SLOTS = 4;     // input-ring cap of a CTA pair that streams one tile at a time
+// half-height weight slots reserved before the input ring gets the rest (CTA pair + ping-pong): the update MLP measured
+// 0.263 / 0.230 / 0.245 ms with 4 / 3 / 2 (input ring 2 / 3 / 4)
+constexpr int PAIR_PP_WMIN = 3;
 
 // shared-memory plan; returns false when the MLP does not fit
 inline bool plan_fused(FusedMlp& f) {
@@ -975,7 +937,6 @@ inline bool plan_fused(FusedMlp& f) {
     p.a_slots = 0;
     p.pp = 0;
     p.split = 0;
-    p.step_bias = 0;
     p.n_steps = 0;
     p.stage_in_h = 0;
     p.stage_off = 0;
@@ -1010,14 +971,14 @@ inline bool plan_fused(FusedMlp& f) {
         int h_blocks = 1;
         for (int l = 0; l + 1 < p.n_layers; ++l) h_blocks = max(h_blocks, (p.layer[l].N + 63) / 64);
         const int k0_blocks = (p.layer[0].K + 63) / 64;
-        if (f.ping_pong && p.two_bufs) {
+        if (p.two_bufs) {
             // two tiles in flight: two hidden regions; a tile's output staging aliases its own hidden region when it fits
             for (int ew : {8, 4}) {
                 const int h_bytes = h_blocks * AH_BLOCK_BYTES, stage_bytes = ew * 32 * p.stage_row;
                 const int in_h = stage_bytes <= h_bytes;
                 const int fixed = pad + 2 * h_bytes + (in_h ? 0 : stage_bytes) + BAR_BYTES + bias_total * 4;
                 // weight slots to reserve before the input ring gets the rest: four half-height ones in pair mode
-                int w_min = p.pair ? pair_pp_wmin() : 2;
+                int w_min = p.pair ? PAIR_PP_WMIN : 2;
                 if (SMEM_LIMIT - fixed - w_min * p.slot_bytes < 2 * AH_BLOCK_BYTES) w_min = 2;
                 int a_slots = (SMEM_LIMIT - fixed - w_min * p.slot_bytes) / AH_BLOCK_BYTES;
                 if (a_slots > 2 * k0_blocks) a_slots = 2 * k0_blocks;
@@ -1043,7 +1004,7 @@ inline bool plan_fused(FusedMlp& f) {
             if (a_slots > MAX_A_SLOTS) a_slots = MAX_A_SLOTS;
             // CTA pair: weight slots are half-height (as large as an input block) and the in-order producer never runs the
             // input ring further ahead than the weight ring lets it: the weight ring gets the larger share
-            if (p.pair && a_slots > pair_a_slots()) a_slots = pair_a_slots();
+            if (p.pair && a_slots > PAIR_A_SLOTS) a_slots = PAIR_A_SLOTS;
             fixed -= (w_min - 2) * p.slot_bytes;          // `fixed` below counts two weight slots
             if (a_slots >= 2 && a_slots >= (k0_blocks + 1) / 2) {
                 p.a_slots = a_slots;
@@ -1063,10 +1024,9 @@ inline bool plan_fused(FusedMlp& f) {
     // first k0 blocks, and the next hidden epilogue comes after this one in the same warps' program order.
     const int k0_blocks_res = (p.layer[0].K + 63) / 64;
     // split mode: every hidden layer exactly 512 wide (two accumulator halves, two h_full halves), output <= 256
-    bool split = f.split_mode && p.n_layers >= 2 && p.layer[p.n_layers - 1].N <= 256 && p.rows > 0;
+    bool split = p.n_layers >= 2 && p.layer[p.n_layers - 1].N <= 256 && p.rows > 0;
     for (int l = 0; l + 1 < p.n_layers; ++l) split = split && p.layer[l].N == 512;
-    const bool step_bias = split && f.split_step_bias;
-    const int bias_bytes = step_bias ? 2 * 256 * 4 : bias_total * 4;
+    const int bias_bytes = split ? 2 * 256 * 4 : bias_total * 4;
     for (int ew : {8, 4}) {     // prefer 8 epilogue warps when two ring slots still fit
         const int stage_bytes = ew * 32 * p.stage_row;
         const int in_h = p.n_layers > 1 && (blocks - k0_blocks_res) * AH_BLOCK_BYTES >= stage_bytes;
@@ -1095,7 +1055,6 @@ inline bool plan_fused(FusedMlp& f) {
                 }
                 p.n_steps = n;
                 p.split = 1;
-                p.step_bias = step_bias ? 1 : 0;
             }
             return true;
         }

@@ -482,11 +482,8 @@ struct X3Mlp {
     X3Params p;
     int smem_bytes = 0;
     bool pair_mode = false;     // request the CTA-pair instantiation
-    bool four_epilogue_warps = false;   // one epilogue warp per TMEM lane quadrant instead of two
     bool ready = false;
 };
-
-inline int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
 
 // shared-memory plan; returns false when the MLP does not fit
 inline bool plan_x3(X3Mlp& f) {
@@ -509,7 +506,6 @@ inline bool plan_x3(X3Mlp& f) {
     p.n_tiles = ceil_div(p.rows, BLOCK_M);
     p.w_slot_bytes = ((pair ? max_n / 2 : max_n) * BLOCK_K * 2 + 1023) / 1024 * 1024;
     for (int ew : {8, 4}) {
-        if (ew == 8 && f.four_epilogue_warps) continue;
         const int fixed = pad + ew * 32 * STAGE_ROW + BAR_BYTES + bias_total * 4;
         int avail = SMEM_LIMIT - fixed;
         int a = 2, w = 2;
@@ -523,9 +519,6 @@ inline bool plan_x3(X3Mlp& f) {
             else if (a < MAX_RING && avail >= BLK_BYTES) { ++a; avail -= BLK_BYTES; grew = true; }
             if (!grew) break;
         }
-        const int ea = env_int("DSAT_X3_A_SLOTS", 0), ewn = env_int("DSAT_X3_W_SLOTS", 0);
-        if (ea >= 2 && ewn >= 2 && ea <= MAX_RING && ewn <= MAX_RING &&
-            fixed + ea * BLK_BYTES + ewn * p.w_slot_bytes <= SMEM_LIMIT) { a = ea; w = ewn; }
         p.a_slots = a; p.w_slots = w; p.epi_warps = ew;
         f.smem_bytes = fixed + a * BLK_BYTES + w * p.w_slot_bytes;
         f.ready = true;

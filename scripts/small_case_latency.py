@@ -15,5 +15,5 @@ with contextlib.redirect_stdout(io.StringIO()):
     times = []
     for _ in range(3):
         t0 = time.perf_counter(); h = s.samples(256); times.append(time.perf_counter() - t0)
-print("%s: samples(256) n=30: cold %.3f s, warm %s s, %d chains launched per call, launches %d, graph %s" % (
-    prec, cold, ["%.3f" % t for t in times], s.last_stats["chains_launched"], s.ctx.launch_count(), os.environ.get("DSAT_GRAPH", "1")))
+print("%s: samples(256) n=30: cold %.3f s, warm %s s, %d chains launched per call, launches %d" % (
+    prec, cold, ["%.3f" % t for t in times], s.last_stats["chains_launched"], s.ctx.launch_count()))

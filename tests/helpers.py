@@ -6,8 +6,15 @@ from diffusionsat_b200 import synth, weights as W
 from oracle import querysat_oracle as O
 
 
-def make_weights(feature_maps=128, query_maps=128, seed=7, bias_scale=0.1):
-    return W.init_weights(feature_maps, query_maps, seed=seed, bias_scale=bias_scale)
+def make_weights(feature_maps=128, query_maps=128, seed=7, bias_scale=0.1, lit_hidden=None):
+    """Seeded weights; `lit_hidden` narrows the literal MLP's hidden layers (the C ABI takes any consistent widths)."""
+    wts = W.init_weights(feature_maps, query_maps, seed=seed, bias_scale=bias_scale)
+    if lit_hidden is not None:
+        for i in range(3):
+            k, b = wts.layers["lit_query/%d" % i]
+            k = k[:, :lit_hidden] if i == 0 else k[:lit_hidden, :lit_hidden] if i == 1 else k[:lit_hidden]
+            wts.layers["lit_query/%d" % i] = (np.ascontiguousarray(k), b[:lit_hidden] if i < 2 else b)
+    return wts
 
 
 def noise_for(n_rows, rounds, seed, steps=None):

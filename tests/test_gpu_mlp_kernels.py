@@ -8,13 +8,14 @@ restatement of reference model/mlp.py:42-50 (Dense = x @ kernel + bias, hidden a
   leaky relu on bf16 values, outputs); 2e-3 |want| + 2e-3 rms for at least 99 % of the elements (half a bf16 ulp), and
   one bf16 ulp (8e-3) for every element: an accumulator within rounding distance of a bf16 tie may round the other way.
 
-Sizes: n = 100, m = 428 (the bench formula's shape) with 700 chains: 547 variable tiles and 2341 clause tiles, so every
-persistent CTA (or CTA pair) loops over several tiles, rings wrap, and the last tile is partial.  The reference values
-are computed for rows drawn from the first, middle and last tiles and a random subset."""
-import os
-import subprocess
-import sys
-
+Shapes (SHAPES), each of which selects other kernel plans:
+* bench: n = 100, m = 428 (the bench formula's shape) with 700 chains: 547 variable tiles and 2341 clause tiles, so every
+  persistent CTA (or CTA pair) loops over several tiles, rings wrap, and the last tile is partial;
+* one_tile: n = 20 with one chain, at most 128 rows per MLP: the single-CTA instantiations (split, x3 and whole-MLP);
+* f128_q64: feature_maps 128, query_maps 64: the literal MLP through the resident-input fused_mlp_kernel (hidden 256);
+* lit_hidden_384 (bf16 only; the fp32-accurate kernels tile hidden widths of at most 256 or multiples of 256): hidden
+  layers wider than 256 columns without split mode.
+The reference values are computed for rows drawn from the first, middle and last tiles and a random subset."""
 import numpy as np
 import pytest
 
@@ -22,16 +23,21 @@ from diffusionsat_b200 import _lib, graph as G, synth
 from tests import helpers as H
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-F = Q = 128
-MLPS = {   # name -> (input buffer, input columns (None = all), output buffer, output columns)
-    "variables_query": ("VROW", F + 9, "QS", 3 * Q),
-    "lit_query": ("VROW", F + 9, "LIT", 2 * Q),
-    "clause_update": ("CROW", F + 2 * Q, "COUT", Q + F),
-    "update_gate": ("VROW", None, "UOUT", F),
-    "variables_output": ("SPRE", F, "LOGITS", 8),
+SHAPES = {   # name -> (variables, chains, feature_maps, query_maps, literal hidden width (None = 4 query_maps))
+    "bench": (100, 700, 128, 128, None),
+    "one_tile": (20, 1, 128, 128, None),
+    "f128_q64": (100, 70, 128, 64, None),
+    "lit_hidden_384": (100, 70, 128, 128, 384),
 }
+FP32_SHAPES = ("bench", "one_tile", "f128_q64")
+
+
+def mlps(F, Q):
+    """name -> (input buffer, output buffer, output columns)"""
+    return {"variables_query": ("VROW", "QS", 3 * Q), "lit_query": ("VROW", "LIT", 2 * Q),
+            "clause_update": ("CROW", "COUT", Q + F), "update_gate": ("VROW", "UOUT", F),
+            "variables_output": ("SPRE", "LOGITS", 8)}
 
 
 def sample_rows(rows, rng):
@@ -50,6 +56,7 @@ def softplus64(x):
 
 def reference_fp64(name, x, wts):
     """fp64 chain of one MLP on the reference's column order; x is in the kernels' packed row layout."""
+    F, Q = wts.feature_maps, wts.query_maps
     layers = wts.mlp(name)
     if name in ("variables_query", "lit_query"):
         h = x[:, :F + 9]
@@ -70,6 +77,7 @@ def reference_fp64(name, x, wts):
 def reference_bf16_chain(name, x, wts):
     """The same chain with bf16 rounding at the kernel's rounding points (dsat_mlp_fused.cuh)."""
     r = H.bf16_round
+    F, Q = wts.feature_maps, wts.query_maps
     layers = wts.mlp(name)
     if name in ("variables_query", "lit_query"):
         h = x[:, :F + 9]
@@ -92,16 +100,18 @@ def reference_bf16_chain(name, x, wts):
     return h
 
 
-def run_case(ctx, precision, chains=700, seed=0):
-    n_vars = 100
+def run_case(ctx, precision, shape, seed=0):
+    n_vars, chains, F, Q, lit_hidden = SHAPES[shape]
     _, clauses = synth.random_3sat(n_vars, seed=3)
-    wts = H.make_weights(seed=31 + seed, bias_scale=0.1)
+    if shape == "one_tile":
+        assert len(clauses) <= 128
+    wts = H.make_weights(F, Q, seed=31 + seed, bias_scale=0.1, lit_hidden=lit_hidden)
     ctx.set_model(wts)
     ctx.set_precision(precision)
     ctx.set_graph(G.build_unit_graph(n_vars, clauses), chains=chains, group_graphs=0)
     rng = np.random.default_rng(seed)
     checked = {}
-    for name, (src, _, dst, out_cols) in MLPS.items():
+    for name, (src, dst, out_cols) in mlps(F, Q).items():
         rows, ld = ctx.debug_dims(src)
         x = rng.standard_normal((rows, ld)).astype(np.float32)
         if src == "VROW":
@@ -117,50 +127,26 @@ def run_case(ctx, precision, chains=700, seed=0):
 
 @pytest.mark.parametrize("precision", ["fp32", "fp32_simt"])
 def test_fp32_mlp_kernels_elementwise(ctx, precision):
-    for name, (got, x, wts) in run_case(ctx, _lib.PRECISIONS[precision]).items():
-        want = reference_fp64(name, x, wts)
-        rms = float(np.sqrt(np.mean(want ** 2)))
-        bound = 2e-4 * np.abs(want) + 1e-4 * np.sqrt(np.mean(want ** 2, axis=1, keepdims=True))
-        bad = np.abs(got - want) > bound
-        assert not bad.any(), "%s (%s): %d of %d elements off, worst %.3e at value %.3e (rms %.3e)" % (
-            name, precision, int(bad.sum()), bad.size, float(np.abs(got - want).max()), float(want[np.unravel_index(np.argmax(np.abs(got - want)), want.shape)]), rms)
+    for shape in FP32_SHAPES:
+        for name, (got, x, wts) in run_case(ctx, _lib.PRECISIONS[precision], shape).items():
+            want = reference_fp64(name, x, wts)
+            rms = float(np.sqrt(np.mean(want ** 2)))
+            bound = 2e-4 * np.abs(want) + 1e-4 * np.sqrt(np.mean(want ** 2, axis=1, keepdims=True))
+            bad = np.abs(got - want) > bound
+            assert not bad.any(), "%s (%s, %s): %d of %d elements off, worst %.3e at value %.3e (rms %.3e)" % (
+                name, precision, shape, int(bad.sum()), bad.size, float(np.abs(got - want).max()),
+                float(want[np.unravel_index(np.argmax(np.abs(got - want)), want.shape)]), rms)
 
 
 def test_bf16_mlp_kernels_elementwise(ctx):
-    for name, (got, x, wts) in run_case(ctx, _lib.BF16).items():
-        want = reference_bf16_chain(name, x, wts)
-        rms = float(np.sqrt(np.mean(want ** 2)))
-        err = np.abs(got - want)
-        tight = err <= 2e-3 * np.abs(want) + 2e-3 * rms
-        loose = err <= 8e-3 * np.abs(want) + 8e-3 * rms
-        assert tight.mean() >= 0.99, "%s: only %.4f of the elements within half a bf16 ulp" % (name, tight.mean())
-        assert loose.all(), "%s: %d elements beyond one bf16 ulp, worst %.3e (rms %.3e)" % (name, int((~loose).sum()), float(err.max()), rms)
+    for shape in SHAPES:
+        for name, (got, x, wts) in run_case(ctx, _lib.BF16, shape).items():
+            want = reference_bf16_chain(name, x, wts)
+            rms = float(np.sqrt(np.mean(want ** 2)))
+            err = np.abs(got - want)
+            tight = err <= 2e-3 * np.abs(want) + 2e-3 * rms
+            loose = err <= 8e-3 * np.abs(want) + 8e-3 * rms
+            assert tight.mean() >= 0.99, "%s (%s): only %.4f of the elements within half a bf16 ulp" % (name, shape, tight.mean())
+            assert loose.all(), "%s (%s): %d elements beyond one bf16 ulp, worst %.3e (rms %.3e)" % (
+                name, shape, int((~loose).sum()), float(err.max()), rms)
 
-
-PLANS = {
-    "x3_no_pair": {"DSAT_X3_PAIR": "0"},
-    "x3_all_pair": {"DSAT_X3_PAIR": "127"},
-    "x3_shallow_rings": {"DSAT_X3_A_SLOTS": "2", "DSAT_X3_W_SLOTS": "2"},
-    "x3_four_epilogue_warps": {"DSAT_X3_EPI4": "127"},
-    "x3_whole_clause_mlp": {"DSAT_X3_SPLIT": "0"},
-    "x3_layer_per_launch_update": {"DSAT_X3_SPLIT": "3"},
-    "bf16_split_off": {"DSAT_SPLIT_MODE": "0"},
-    "bf16_cta_pair": {"DSAT_PAIR_MODE": "31", "DSAT_SPLIT_MODE": "0"},
-    "bf16_no_pair": {"DSAT_PAIR_MODE": "0"},
-    "bf16_one_tile_at_a_time": {"DSAT_PING_PONG": "0", "DSAT_A_RING": "0", "DSAT_PAIR_MODE": "0"},
-}
-
-
-@pytest.mark.parametrize("plan", sorted(PLANS))
-def test_mlp_kernels_under_other_plans(plan):
-    """The kernel plans are picked by environment switches read once per process: re-run the element-wise tests of this
-    file in a fresh process under every non-default plan."""
-    env = dict(os.environ)
-    env.update(PLANS[plan])
-    pick = "test_fp32_mlp_kernels_elementwise and fp32-" if plan.startswith("x3") else "test_bf16_mlp_kernels_elementwise"
-    if plan.startswith("x3"):
-        pick = "test_fp32_mlp_kernels_elementwise and not simt"
-    cmd = [sys.executable, "-m", "pytest", os.path.abspath(__file__), "-x", "-q", "-m", "gpu", "-k", pick, "-p", "no:cacheprovider"]
-    proc = subprocess.run(cmd, cwd=ROOT, env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
-    assert proc.returncode == 0, "plan %s (%s):\n%s" % (plan, PLANS[plan], proc.stdout[-3000:])
-    assert "1 passed" in proc.stdout

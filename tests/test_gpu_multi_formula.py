@@ -142,6 +142,26 @@ def test_union_groups_match_their_solo_runs_and_the_oracle(ctx, tmp_path):
         ctx.set_batches(group_seg, np.array(base, dtype=np.uint64))
 
 
+@pytest.mark.parametrize("precision", ["fp32", "bf16"])
+def test_skipping_finished_groups_changes_nothing(ctx, precision):
+    """Whole-chain groups bound with group_graphs skip the rows of finished groups; the same groups bound through
+    dsat_set_batches (no noise bases) compute every row.  Both runs give the same bits."""
+    n_vars, clauses, _ = synth.planted_3sat(24, seed=5)
+    chains, group, steps, rounds = 96, 3, 16, 32
+    unit = G.build_unit_graph(n_vars, clauses)
+    ctx.set_model(load_weights(FIXTURE))
+    ctx.set_precision(precision)
+    runs = []
+    for skip in (True, False):
+        ctx.set_graph(unit, chains=chains, group_graphs=group)
+        if not skip:
+            ctx.set_batches(np.arange(0, chains + 1, group))
+        runs.append(ctx.sample(steps, rounds, seed=13) + (ctx.debug_groups()["steps_taken"],))
+    assert (runs[0][-1] < rounds - 1).any(), "no group finished early: nothing was skipped"
+    for name, a, b in zip(("packed", "is_sat", "latch_step", "sat_any", "steps_taken"), *runs):
+        np.testing.assert_array_equal(a, b, err_msg=name)
+
+
 def test_segmented_histogram_equals_numpy(ctx):
     ctx.set_model(load_weights(FIXTURE))
     ctx.set_precision("bf16")
