@@ -37,13 +37,10 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if not force and not needs_build():
         return LIB_PATH
     # -compress-all: the fatbin's cubin is compressed whatever its size (by default nvcc left the 8.9 MB cubin of
-    # sm_100a SASS uncompressed, a 10.4 MB library instead of 3.8 MB)
+    # sm_100a SASS uncompressed, a 10.4 MB library instead of 3.8 MB).  No -lcuda: cuTensorMapEncodeTiled is resolved at
+    # run time (cudaGetDriverEntryPoint), so the library still loads on a machine without a driver (CPU test tier)
     cmd = [_nvcc(), "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
            "-Xcompiler", "-fPIC", "-shared", "-Xfatbin", "-compress-all"]
-    if os.path.exists(os.path.join(CSRC, "dsat_gemm_tc.cuh")):
-        # cuTensorMapEncodeTiled is resolved at run time (cudaGetDriverEntryPoint): no link against libcuda,
-        # so the library still loads on a machine without a driver (CPU test tier)
-        cmd += ["-DDSAT_WITH_TCGEN05"]
     if verbose:
         cmd += ["-Xptxas", "-v"]
     cmd += os.environ.get("DSAT_NVCC_FLAGS", "").split()      # e.g. -DDSAT_ASSERT for the debug build

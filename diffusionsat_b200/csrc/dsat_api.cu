@@ -20,11 +20,9 @@
 #include "dsat_graph_host.cuh"
 #include "dsat_norm_head.cuh"
 #include "dsat_hist.cuh"
-#ifdef DSAT_WITH_TCGEN05
 #include "dsat_gemm_tc.cuh"
 #include "dsat_mlp_fused.cuh"
 #include "dsat_mlp_x3.cuh"
-#endif
 
 using namespace dsat;
 
@@ -67,9 +65,7 @@ struct DevBuf {
 
 struct PackedLayer {          // one launched linear op
     DevBuf<float> w, b;
-#ifdef DSAT_WITH_TCGEN05
     DevBuf<__nv_bfloat16> w_bf16;   // [N, K] K-major copy for the tensor-core path
-#endif
     int K = 0, N = 0;
 };
 
@@ -85,11 +81,7 @@ struct dsat_ctx {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::string err;
     long long launches = 0;
-#ifdef DSAT_WITH_TCGEN05
     int precision = DSAT_F32_TC;        // default: fp32-accurate Dense layers on the tensor cores
-#else
-    int precision = DSAT_F32;
-#endif
     // per-class CUDA-event marks (dsat_profile_rounds)
     struct ProfMark { cudaEvent_t ev; int cls; };
     std::vector<ProfMark> prof;
@@ -137,7 +129,6 @@ struct dsat_ctx {
     // injected noise staging
     DevBuf<float> inj_normals, inj_uniforms, inj_noisy;
     DevBuf<int> inj_labels;
-#ifdef DSAT_WITH_TCGEN05
     // bf16 activations of the tensor-core path (A operands are fetched by TMA from these)
     DevBuf<__nv_bfloat16> VROWb, CROWb, H1b, H2b, QSb, LITb, CHb, COUTb, U1b, U2b, UOUTb, SPREb, O1b;
     CUtensorMap map_a[OP_COUNT];        // A operand of each linear op
@@ -154,7 +145,6 @@ struct dsat_ctx {
     x3::X3Mlp x3[7];                    // query, lit layer 1, lit layer 2, lit layer 3, clause, update, output
     bool has_x3_buffers = false;
     bool x3_ready = false;
-#endif
     bool has_simt_buffers = false;
     float last_noise_scale = 0.f;
     int sampling = DSAT_SAMPLE_INVERSE_CDF;
@@ -212,7 +202,6 @@ cudaError_t configure_kernels_for_device() {
     auto opt_in = [&](auto kernel) {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     };
-#ifdef DSAT_WITH_TCGEN05
     opt_in(clause_gather_smem_kernel<128, true>); opt_in(clause_gather_smem_kernel<128, false>);
     opt_in(clause_gather_smem_kernel<64, true>); opt_in(clause_gather_smem_kernel<64, false>);
     opt_in(clause_gather_smem_kernel<32, true>); opt_in(clause_gather_smem_kernel<32, false>);
@@ -229,7 +218,6 @@ cudaError_t configure_kernels_for_device() {
     if (e == cudaSuccess) e = fm::configure_fused_device();
     if (e == cudaSuccess) e = x3::configure_x3_device(0);
     if (e == cudaSuccess) e = tc::configure_tc_device();
-#endif
     if (e == cudaSuccess) configured.mark();
     return e;
 }
@@ -298,7 +286,7 @@ int ensure_common_buffers(dsat_ctx* c) {
     return DSAT_OK;
 }
 
-// + the fp32 row buffers and hidden activations of the CUDA-core path (the bf16 path mirrors the state there too)
+// + the fp32 row buffers and hidden activations of the CUDA-core path
 int ensure_buffers(dsat_ctx* c) {
     int rc = ensure_common_buffers(c);
     if (rc) return rc;
@@ -320,21 +308,12 @@ int ensure_buffers(dsat_ctx* c) {
     return DSAT_OK;
 }
 
-#ifdef DSAT_WITH_TCGEN05
 static int pick_slice_width(size_t table_rows, int Q, size_t* bytes_out, int budget_kb, int elt_bytes = 2);
-
-__global__ void mirror_cols_kernel(const float* __restrict__ src, int ld_src, __nv_bfloat16* __restrict__ dst, int ld_dst,
-                                   long long rows, int cols) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= rows * cols) return;
-    const long long r = i / cols; const int cc = (int)(i % cols);
-    dst[(size_t)r * ld_dst + cc] = __float2bfloat16_rn(src[(size_t)r * ld_src + cc]);
-}
 
 // bf16 activation buffers + the TMA descriptors of every A operand (they depend on the row counts)
 int ensure_tc_buffers(dsat_ctx* c) {
     if (c->has_tc_buffers) return DSAT_OK;
-    int rc = ensure_buffers(c);
+    int rc = ensure_common_buffers(c);
     if (rc) return rc;
     const size_t Nt = (size_t)c->Nt, Mt = (size_t)c->Mt;
     const int F = c->F, Q = c->Q;
@@ -458,7 +437,6 @@ int tc_pack_weights(dsat_ctx* c) {
     }
     return DSAT_OK;
 }
-#endif
 
 // Invalidate every activation buffer (shape or model changed).  The memory stays with the context and is reused by the next
 // ensure_*_buffers when it is large enough; dsat_destroy frees it (free_buffers).
@@ -473,14 +451,12 @@ void release_buffers(dsat_ctx* c) {
     c->sat_now.drop(); c->is_sat.drop(); c->sat_any.drop(); c->packed.drop();
     c->inj_normals.drop(); c->inj_uniforms.drop(); c->inj_noisy.drop(); c->inj_labels.drop();
     c->hist_idx.drop(); c->hist_run.drop(); c->hist_totals.drop(); c->hist_keys.drop(); c->hist_counts.drop();
-#ifdef DSAT_WITH_TCGEN05
     c->VROWb.drop(); c->CROWb.drop(); c->H1b.drop(); c->H2b.drop(); c->QSb.drop(); c->LITb.drop();
     c->CHb.drop(); c->COUTb.drop(); c->UOUTb.drop(); c->U1b.drop(); c->U2b.drop(); c->SPREb.drop();
     c->O1b.drop();
     c->has_tc_buffers = false;
     c->VROWp.drop(); c->CROWp.drop(); c->SPREp.drop(); c->H1p.drop(); c->H2p.drop();
     c->has_x3_buffers = false;
-#endif
     c->has_buffers = false;
     c->has_simt_buffers = false;
 }
@@ -496,14 +472,12 @@ void free_buffers(dsat_ctx* c) {
     c->inj_normals.release(); c->inj_uniforms.release(); c->inj_noisy.release(); c->inj_labels.release();
     c->hist_idx.release(); c->hist_run.release(); c->hist_totals.release(); c->hist_keys.release(); c->hist_counts.release();
     c->hist_seg.release(); c->hist_run_seg.release();
-#ifdef DSAT_WITH_TCGEN05
     c->VROWb.release(); c->CROWb.release(); c->H1b.release(); c->H2b.release(); c->QSb.release(); c->LITb.release();
     c->CHb.release(); c->COUTb.release(); c->UOUTb.release(); c->U1b.release(); c->U2b.release(); c->SPREb.release();
     c->O1b.release();
     c->has_tc_buffers = false;
     c->VROWp.release(); c->CROWp.release(); c->SPREp.release(); c->H1p.release(); c->H2p.release();
     c->has_x3_buffers = false;
-#endif
     c->has_buffers = false;
     c->has_simt_buffers = false;
 }
@@ -525,7 +499,6 @@ void prof_mark(dsat_ctx* c, int cls) {
     c->prof_used++;
 }
 
-#ifdef DSAT_WITH_TCGEN05
 // ------------------------------------------------------------------ fp32-accurate tensor-core path (x3)
 // Stacked hi/lo K-major copies [2N, K64] of the twelve reference layers, cut out of the packed fp32 operators.
 int x3_pack_weights(dsat_ctx* c) {
@@ -554,6 +527,9 @@ int x3_pack_weights(dsat_ctx* c) {
     return DSAT_OK;
 }
 
+// the seven x3 launches, slots of dsat_ctx::x3
+enum { XQ = 0, XL1, XL2, XL3, XC, XU, XO };
+
 int ensure_x3_buffers(dsat_ctx* c) {
     if (c->has_x3_buffers) return DSAT_OK;
     int rc = ensure_common_buffers(c);
@@ -567,7 +543,6 @@ int ensure_x3_buffers(dsat_ctx* c) {
     CK_CUDA(c, c->H2p.alloc(2 * Nt * c->HL));
     CK_CUDA(c, cudaMemsetAsync(c->VROWp.p, 0, c->VROWp.count * 2, c->stream));
     CK_CUDA(c, cudaMemsetAsync(c->CROWp.p, 0, c->CROWp.count * 2, c->stream));
-    enum { XQ = 0, XL1, XL2, XL3, XC, XU, XO };
     struct L { int wi; int op; int bias_off; int epi; };        // wi = index into wx[] (reference layer order)
     auto build = [&](int which, const __nv_bfloat16* a_hi, size_t a_plane, long long rows, int k, int lda,
                      std::initializer_list<L> layers, int n_groups, int out_mode, void* out0, void* out1, int ld_out) -> bool {
@@ -647,7 +622,6 @@ int run_x3(dsat_ctx* c, int which, int prof_class) {
     c->launches++;
     return DSAT_OK;
 }
-#endif
 
 int run_linear(dsat_ctx* c, int op, const float* A, int lda, float* Y, int ldy, long long rows, int epi) {
     prof_mark(c, op);
@@ -690,24 +664,17 @@ LossScalars loss_scalars(float noise_scale) {
     return s;
 }
 
-#ifdef DSAT_WITH_TCGEN05
 static inline bool use_tc(const dsat_ctx* c) { return c->precision == DSAT_BF16 || c->precision == DSAT_BF16_UNFUSED; }
 static inline bool use_x3(const dsat_ctx* c) { return c->precision == DSAT_F32_TC; }
+// the variable rows in the active precision: fp32 on the CUDA cores, bf16 (hi plane) on the tensor-core paths
+static inline float* vrow_f(dsat_ctx* c) { return c->precision == DSAT_F32 ? c->VROW.p : nullptr; }
 static inline __nv_bfloat16* vrow_b(dsat_ctx* c) { return use_tc(c) ? c->VROWb.p : use_x3(c) ? c->VROWp.p : nullptr; }
 static inline __nv_bfloat16* crow_b(dsat_ctx* c) { return use_tc(c) ? c->CROWb.p : use_x3(c) ? c->CROWp.p : nullptr; }
-#else
-static inline bool use_tc(const dsat_ctx*) { return false; }
-static inline bool use_x3(const dsat_ctx*) { return false; }
-static inline __nv_bfloat16* vrow_b(dsat_ctx*) { return nullptr; }
-static inline __nv_bfloat16* crow_b(dsat_ctx*) { return nullptr; }
-#endif
 
 // buffers of the active precision
 int ensure_active_buffers(dsat_ctx* c) {
-#ifdef DSAT_WITH_TCGEN05
     if (use_tc(c)) return ensure_tc_buffers(c);
     if (use_x3(c)) return ensure_x3_buffers(c);
-#endif
     return ensure_buffers(c);
 }
 
@@ -720,11 +687,11 @@ int begin_call(dsat_ctx* c, float noise_scale, const float* noisy_dev, const flo
     c->last_noise_scale = noise_scale;
     step_begin_kernel<<<(unsigned)((Nt + threads - 1) / threads), threads, 0, c->stream>>>(
         Nt, noise_scale, use_x ? c->X.p : nullptr, noisy_dev, uniforms_dev, labels_dev, c->labels.p,
-        x3p ? nullptr : c->VROW.p, c->ldv(), c->F, vrow_b(c), ns, vplane, sp_tab, sp_cur, c->sampling == DSAT_SAMPLE_GUMBEL ? 1 : 0);
+        vrow_f(c), c->ldv(), c->F, vrow_b(c), ns, vplane, sp_tab, sp_cur, c->sampling == DSAT_SAMPLE_GUMBEL ? 1 : 0);
     LAUNCHED(c);
     {   // variables_state = ones, clauses_state = ones (reference model/query_sat.py:141,148)
         long long tot;
-        if (!x3p) {
+        if (vrow_f(c)) {
             tot = Nt * (c->F / 4);
             fill_cols_kernel<<<(unsigned)((tot + threads - 1) / threads), threads, 0, c->stream>>>(
                 c->VROW.p, c->ldv(), Nt, c->F / 4, 1.0f);
@@ -733,8 +700,7 @@ int begin_call(dsat_ctx* c, float noise_scale, const float* noisy_dev, const flo
             fill_cols_kernel<<<(unsigned)((tot + threads - 1) / threads), threads, 0, c->stream>>>(
                 c->CROW.p, c->ldc(), c->Mt, c->F / 4, 1.0f);
             LAUNCHED(c);
-        }
-        if (use_tc(c) || x3p) {
+        } else {
             tot = Nt * (c->F / 8);
             fill_cols_bf16_kernel<<<(unsigned)((tot + threads - 1) / threads), threads, 0, c->stream>>>(
                 vrow_b(c), c->ldv(), Nt, c->F / 8, 1.0f);
@@ -762,7 +728,6 @@ int begin_call(dsat_ctx* c, float noise_scale, const float* noisy_dev, const flo
     return DSAT_OK;
 }
 
-#ifdef DSAT_WITH_TCGEN05
 // one tensor-core linear op; out0/out1 describe where the output columns go
 int run_linear_tc(dsat_ctx* c, int op, long long rows, int epi, void* p0, int ld0, bool bf0,
                   void* p1 = nullptr, int ld1 = 0, bool bf1 = false, int split = 0) {
@@ -777,18 +742,14 @@ int run_linear_tc(dsat_ctx* c, int op, long long rows, int epi, void* p0, int ld
     c->launches++;
     return DSAT_OK;
 }
-#endif
 
-#ifdef DSAT_WITH_TCGEN05
 int run_fused(dsat_ctx* c, int which, int prof_class) {
     prof_mark(c, prof_class);
     CK_CUDA(c, fm::launch_fused(c->fused[which], c->sm_count, c->stream));
     c->launches++;
     return DSAT_OK;
 }
-#endif
 
-#ifdef DSAT_WITH_TCGEN05
 // Shared-memory staged gathers (small formulas): pick the widest feature slice whose two tables fit;
 // returns false when they do not fit (the L2-gather kernels run instead).
 static int pick_slice_width(size_t table_rows, int Q, size_t* bytes_out, int budget_kb, int elt_bytes) {
@@ -849,9 +810,7 @@ bool launch_literal_gather_smem(dsat_ctx* c, const UnitGraphDev& g) {
     if (w == 64) return si ? launch(literal_gather_smem_kernel<64, true>) : launch(literal_gather_smem_kernel<64, false>);
     return si ? launch(literal_gather_smem_kernel<32, true>) : launch(literal_gather_smem_kernel<32, false>);
 }
-#endif
 
-#ifdef DSAT_WITH_TCGEN05
 // fp32 tables (fp32-accurate tensor-core path): outputs go to the hi/lo planes
 bool launch_clause_gather_smem_f32(dsat_ctx* c, const UnitGraphDev& g) {
     if (c->n_graphs != 1) return false;
@@ -892,9 +851,7 @@ bool launch_literal_gather_smem_f32(dsat_ctx* c, const UnitGraphDev& g) {
     if (w == 64) return si ? launch(literal_gather_smem_f32_kernel<64, true>) : launch(literal_gather_smem_f32_kernel<64, false>);
     return si ? launch(literal_gather_smem_f32_kernel<32, true>) : launch(literal_gather_smem_f32_kernel<32, false>);
 }
-#endif
 
-#ifdef DSAT_WITH_TCGEN05
 // PairNorm with the graph resident in shared memory (split-plane path); false when a graph does not fit
 template <int V>
 bool launch_pairnorm_smem(dsat_ctx* c, const int* seg, int rows_per_chain, int max_graph_rows, const float* src, int ld_src, int src_off,
@@ -916,58 +873,80 @@ bool launch_pairnorm_smem(dsat_ctx* c, const int* seg, int rows_per_chain, int m
                                                                 state_hi, state_plane, ld_state, pre_hi, pre_plane, ld_pre, skip_info(c));
     return true;
 }
-#endif
+
+// One MLP in the active precision: 0 variables_query (VROW -> QS), 1 lit_query (VROW -> LIT), 2 clause_update
+// (CROW -> COUT), 3 update_gate (VROW -> UOUT), 4 variables_output (SPRE -> LOGITS).  On the per-layer paths the query and
+// literal MLPs share their first layer (OP_V1, both halves in one launch): `v1_done` says it has already run.
+// Each launch is profiled under the last linear op it runs.
+int run_mlp(dsat_ctx* c, int which, bool v1_done = false) {
+    const long long Nt = c->Nt, Mt = c->Mt;
+    const int F = c->F, Q = c->Q, ldh1 = c->ldh1();
+    int rc = DSAT_OK;
+    if (use_x3(c)) {
+        switch (which) {
+            case 0: return run_x3(c, XQ, OP_Q2);
+            case 1: if ((rc = run_x3(c, XL1, OP_V1)) || (rc = run_x3(c, XL2, OP_L2))) return rc;
+                    return run_x3(c, XL3, OP_L3);
+            case 2: return run_x3(c, XC, OP_C2);
+            case 3: return run_x3(c, XU, OP_U3);
+            default: return run_x3(c, XO, OP_O2);
+        }
+    }
+    if (c->precision == DSAT_BF16 && c->fused_ready) {
+        static const int cls[5] = {OP_Q2, OP_L3, OP_C2, OP_U3, OP_O2};
+        return run_fused(c, which, cls[which]);
+    }
+    if (use_tc(c)) {
+        if (which <= 1 && !v1_done && (rc = run_linear_tc(c, OP_V1, Nt, tc::TC_LRELU, c->H1b.p, ldh1, true))) return rc;
+        switch (which) {
+            case 0: return run_linear_tc(c, OP_Q2, Nt, tc::TC_QUERY, c->QSb.p, 3 * Q, true);
+            case 1: if ((rc = run_linear_tc(c, OP_L2, Nt, tc::TC_LRELU, c->H2b.p, c->HL, true))) return rc;
+                    return run_linear_tc(c, OP_L3, Nt, tc::TC_LINEAR, c->LITb.p, 2 * Q, true);
+            case 2: if ((rc = run_linear_tc(c, OP_C1, Mt, tc::TC_LRELU, c->CHb.p, c->HC, true))) return rc;
+                    return run_linear_tc(c, OP_C2, Mt, tc::TC_LINEAR, c->COUTb.p, Q + F, true);
+            case 3: if ((rc = run_linear_tc(c, OP_U1, Nt, tc::TC_LRELU, c->U1b.p, c->HU, true)) ||
+                        (rc = run_linear_tc(c, OP_U2, Nt, tc::TC_LRELU, c->U2b.p, c->HU, true))) return rc;
+                    return run_linear_tc(c, OP_U3, Nt, tc::TC_LINEAR, c->UOUTb.p, F, true);
+            default: if ((rc = run_linear_tc(c, OP_O1, Nt, tc::TC_LRELU, c->O1b.p, c->HO, true))) return rc;
+                     return run_linear_tc(c, OP_O2, Nt, tc::TC_LINEAR, c->LOGITS.p, DSAT_LOGIT_PAD, false);
+        }
+    }
+    const int ldv = c->ldv(), ldc = c->ldc();
+    if (which <= 1 && !v1_done && (rc = run_linear(c, OP_V1, c->VROW.p, ldv, c->H1.p, ldh1, Nt, EPI_LRELU))) return rc;
+    switch (which) {
+        case 0: return run_linear(c, OP_Q2, c->H1.p, ldh1, c->QS.p, 3 * Q, Nt, EPI_QUERY);
+        case 1: if ((rc = run_linear(c, OP_L2, c->H1.p + c->HQ, ldh1, c->H2.p, c->HL, Nt, EPI_LRELU))) return rc;
+                return run_linear(c, OP_L3, c->H2.p, c->HL, c->LIT.p, 2 * Q, Nt, EPI_LINEAR);
+        case 2: if ((rc = run_linear(c, OP_C1, c->CROW.p, ldc, c->CH.p, c->HC, Mt, EPI_LRELU))) return rc;
+                return run_linear(c, OP_C2, c->CH.p, c->HC, c->COUT.p, Q + F, Mt, EPI_LINEAR);
+        case 3: if ((rc = run_linear(c, OP_U1, c->VROW.p, ldv, c->U1.p, c->HU, Nt, EPI_LRELU)) ||
+                    (rc = run_linear(c, OP_U2, c->U1.p, c->HU, c->U2.p, c->HU, Nt, EPI_LRELU))) return rc;
+                return run_linear(c, OP_U3, c->U2.p, c->HU, c->UOUT.p, F, Nt, EPI_LINEAR);
+        default: if ((rc = run_linear(c, OP_O1, c->SPRE.p, F, c->O1.p, c->HO, Nt, EPI_LRELU))) return rc;
+                 return run_linear(c, OP_O2, c->O1.p, c->HO, c->LOGITS.p, DSAT_LOGIT_PAD, Nt, EPI_LINEAR);
+    }
+}
 
 // One message-passing round (reference model/query_sat.py:225-348).
 int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, LossScalars ls,
               const StepParams* sp_tab = nullptr, const int* sp_cur = nullptr) {
     const long long Nt = c->Nt, Mt = c->Mt;
-    const int F = c->F, Q = c->Q, ldv = c->ldv(), ldc = c->ldc(), ldh1 = c->ldh1();
+    const int F = c->F, Q = c->Q, ldv = c->ldv(), ldc = c->ldc();
     const UnitGraphDev g = graph_view(c);
     const bool tcp = use_tc(c);
     const bool x3p = use_x3(c);
     const size_t vplane = x3p ? (size_t)Nt * ldv : 0, cplane = x3p ? (size_t)Mt * ldc : 0;
     const SkipInfo skip = skip_info(c);
-#ifdef DSAT_WITH_TCGEN05
-    const bool fusedp = tcp && c->precision == DSAT_BF16 && c->fused_ready;
-    enum { XQ = 0, XL1, XL2, XL3, XC, XU, XO };
-#endif
     int rc;
     {
         const int threads = 256;
         prof_mark(c, PROF_NOISE);
         round_noise_kernel<<<(unsigned)((Nt + threads - 1) / threads), threads, 0, c->stream>>>(
-            Nt, normals_dev, x3p ? nullptr : c->VROW.p, ldv, F, vrow_b(c), ns, (unsigned)round, vplane, sp_tab, sp_cur, skip, c->n);
+            Nt, normals_dev, vrow_f(c), ldv, F, vrow_b(c), ns, (unsigned)round, vplane, sp_tab, sp_cur, skip, c->n);
         LAUNCHED(c);
     }
-    // v1 -> [hidden of variables_query | first hidden of lit_query]   (:240, :252)
-    // query (+ softplus pair) (:240);  lit_query layers 2, 3 (:252)
-    if (x3p) {
-#ifdef DSAT_WITH_TCGEN05
-        if ((rc = run_x3(c, XQ, OP_Q2))) return rc;
-        if ((rc = run_x3(c, XL1, OP_V1))) return rc;
-        if ((rc = run_x3(c, XL2, OP_L2))) return rc;
-        if ((rc = run_x3(c, XL3, OP_L3))) return rc;
-#endif
-    } else if (!tcp) {
-        if ((rc = run_linear(c, OP_V1, c->VROW.p, ldv, c->H1.p, ldh1, Nt, EPI_LRELU))) return rc;
-        if ((rc = run_linear(c, OP_Q2, c->H1.p, ldh1, c->QS.p, 3 * Q, Nt, EPI_QUERY))) return rc;
-        if ((rc = run_linear(c, OP_L2, c->H1.p + c->HQ, ldh1, c->H2.p, c->HL, Nt, EPI_LRELU))) return rc;
-        if ((rc = run_linear(c, OP_L3, c->H2.p, c->HL, c->LIT.p, 2 * Q, Nt, EPI_LINEAR))) return rc;
-    }
-#ifdef DSAT_WITH_TCGEN05
-    else {
-        if (fusedp) {
-            if ((rc = run_fused(c, 0, OP_Q2))) return rc;
-            if ((rc = run_fused(c, 1, OP_L3))) return rc;
-        } else {
-        if ((rc = run_linear_tc(c, OP_V1, Nt, tc::TC_LRELU, c->H1b.p, ldh1, true))) return rc;
-        if ((rc = run_linear_tc(c, OP_Q2, Nt, tc::TC_QUERY, c->QSb.p, 3 * Q, true))) return rc;
-        if ((rc = run_linear_tc(c, OP_L2, Nt, tc::TC_LRELU, c->H2b.p, c->HL, true))) return rc;
-        if ((rc = run_linear_tc(c, OP_L3, Nt, tc::TC_LINEAR, c->LITb.p, 2 * Q, true))) return rc;
-        }
-    }
-#endif
+    // variables_query (+ softplus pair) (:240);  lit_query (:252), which shares the first layer on the per-layer paths
+    if ((rc = run_mlp(c, 0)) || (rc = run_mlp(c, 1, true))) return rc;
     // clause side gather: clause_messages and 4*clauses_loss                    (:241, :248, :255-256)
     prof_mark(c, PROF_CLAUSE_GATHER);
     rc = dispatch_width(c, Q, [&](auto v) {
@@ -975,42 +954,20 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
         const int grid = tcp ? gather_grid(clause_gather_kernel<V, __nv_bfloat16>, Mt, GATHER_WARPS, c->sm_count)
                              : gather_grid(clause_gather_kernel<V, float>, Mt, GATHER_WARPS, c->sm_count);
         if (x3p) {
-#ifdef DSAT_WITH_TCGEN05
             if (!launch_clause_gather_smem_f32(c, g))
-#endif
-            clause_gather_kernel<V, float><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
-                g, c->chains, c->LIT.p, 2 * Q, c->QS.p, 3 * Q, Q, nullptr, ldc, F, crow_b(c), cplane, skip);
+                clause_gather_kernel<V, float><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
+                    g, c->chains, c->LIT.p, 2 * Q, c->QS.p, 3 * Q, Q, nullptr, ldc, F, crow_b(c), cplane, skip);
         } else if (!tcp)
             clause_gather_kernel<V, float><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
                 g, c->chains, c->LIT.p, 2 * Q, c->QS.p, 3 * Q, Q, c->CROW.p, ldc, F, nullptr, 0, skip);
-#ifdef DSAT_WITH_TCGEN05
         else if (!launch_clause_gather_smem(c, g))
             clause_gather_kernel<V, __nv_bfloat16><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
                 g, c->chains, c->LITb.p, 2 * Q, c->QSb.p, 3 * Q, Q, c->CROWb.p, ldc, F, nullptr, 0, skip);
-#endif
     });
     if (rc) return rc;
     LAUNCHED(c);
     // clause_update MLP                                                          (:258-261)
-    if (x3p) {
-#ifdef DSAT_WITH_TCGEN05
-        if ((rc = run_x3(c, XC, OP_C2))) return rc;
-#endif
-    } else if (!tcp) {
-        if ((rc = run_linear(c, OP_C1, c->CROW.p, ldc, c->CH.p, c->HC, Mt, EPI_LRELU))) return rc;
-        if ((rc = run_linear(c, OP_C2, c->CH.p, c->HC, c->COUT.p, Q + F, Mt, EPI_LINEAR))) return rc;
-    }
-#ifdef DSAT_WITH_TCGEN05
-    else {
-        if (fusedp) {
-            if ((rc = run_fused(c, 2, OP_C2))) return rc;
-        } else {
-        if ((rc = run_linear_tc(c, OP_C1, Mt, tc::TC_LRELU, c->CHb.p, c->HC, true))) return rc;
-        // message to literals -> bf16, new clause value -> fp32 (PairNorm input)
-        if ((rc = run_linear_tc(c, OP_C2, Mt, tc::TC_LINEAR, c->COUTb.p, Q + F, true))) return rc;
-        }
-    }
-#endif
+    if ((rc = run_mlp(c, 2))) return rc;
     // literal side gather                                                        (:245-246, :269-273)
     prof_mark(c, PROF_LITERAL_GATHER);
     rc = dispatch_width(c, Q, [&](auto v) {
@@ -1018,22 +975,18 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
         const int grid = tcp ? gather_grid(literal_gather_kernel<V, __nv_bfloat16>, Nt, GATHER_WARPS, c->sm_count)
                              : gather_grid(literal_gather_kernel<V, float>, Nt, GATHER_WARPS, c->sm_count);
         if (x3p) {  // 4*clauses_loss is read back as hi + lo from the clause rows' planes
-#ifdef DSAT_WITH_TCGEN05
             if (!launch_literal_gather_smem_f32(c, g))
-#endif
-            literal_gather_kernel<V, float><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
-                g, c->chains, nullptr, ldc, F + Q, c->COUT.p, Q + F, c->QS.p, 3 * Q, nullptr, ldv, F + DSAT_AUX_PAD,
-                vrow_b(c), vplane, crow_b(c), cplane, skip);
+                literal_gather_kernel<V, float><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
+                    g, c->chains, nullptr, ldc, F + Q, c->COUT.p, Q + F, c->QS.p, 3 * Q, nullptr, ldv, F + DSAT_AUX_PAD,
+                    vrow_b(c), vplane, crow_b(c), cplane, skip);
         } else if (!tcp)
             literal_gather_kernel<V, float><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
                 g, c->chains, c->CROW.p, ldc, F + Q, c->COUT.p, Q + F, c->QS.p, 3 * Q, c->VROW.p, ldv, F + DSAT_AUX_PAD,
                 nullptr, 0, nullptr, 0, skip);
-#ifdef DSAT_WITH_TCGEN05
         else if (!launch_literal_gather_smem(c, g))
             literal_gather_kernel<V, __nv_bfloat16><<<grid, GATHER_WARPS * 32, 0, c->stream>>>(
                 g, c->chains, c->CROWb.p, ldc, F + Q, c->COUTb.p, Q + F, c->QSb.p, 3 * Q, c->VROWb.p, ldv, F + DSAT_AUX_PAD,
                 nullptr, 0, nullptr, 0, skip);
-#endif
     });
     if (rc) return rc;
     LAUNCHED(c);
@@ -1043,90 +996,46 @@ int run_round(dsat_ctx* c, int round, const float* normals_dev, NoiseSource ns, 
         constexpr int V = decltype(v)::value;
         const int grid = c->total_graphs < c->sm_count * 8 ? c->total_graphs : c->sm_count * 8;
         if (x3p) {
-#ifdef DSAT_WITH_TCGEN05
             if (!launch_pairnorm_smem<V>(c, c->clause_seg.p, c->m, c->max_graph_clauses, c->COUT.p, Q + F, Q, crow_b(c), cplane, ldc,
                                          nullptr, 0, 0))
-#endif
-            pairnorm_kernel<V, float, float><<<grid, PN_WARPS * 32, 0, c->stream>>>(
-                c->clause_seg.p, c->n_graphs, c->m, c->total_graphs, c->COUT.p, Q + F, Q, nullptr, ldc, nullptr, 0,
-                crow_b(c), cplane, nullptr, 0, skip);
+                pairnorm_kernel<V, float, float><<<grid, PN_WARPS * 32, 0, c->stream>>>(
+                    c->clause_seg.p, c->n_graphs, c->m, c->total_graphs, c->COUT.p, Q + F, Q, nullptr, ldc, nullptr, 0,
+                    crow_b(c), cplane, nullptr, 0, skip);
         } else if (!tcp)
             pairnorm_kernel<V, float, float><<<grid, PN_WARPS * 32, 0, c->stream>>>(
                 c->clause_seg.p, c->n_graphs, c->m, c->total_graphs, c->COUT.p, Q + F, Q, c->CROW.p, ldc, nullptr, 0,
                 nullptr, 0, nullptr, 0, skip);
-#ifdef DSAT_WITH_TCGEN05
         else
             pairnorm_bf16_kernel<32 * V><<<grid, PN_WARPS * 32, 0, c->stream>>>(
                 c->clause_seg.p, c->n_graphs, c->m, c->total_graphs, c->COUTb.p, Q + F, Q, c->CROWb.p, ldc, nullptr, 0, skip);
-#endif
     });
     if (rc) return rc;
     LAUNCHED(c);
     // update_gate MLP                                                            (:277-278)
-    if (x3p) {
-#ifdef DSAT_WITH_TCGEN05
-        if ((rc = run_x3(c, XU, OP_U3))) return rc;
-#endif
-    } else if (!tcp) {
-        if ((rc = run_linear(c, OP_U1, c->VROW.p, ldv, c->U1.p, c->HU, Nt, EPI_LRELU))) return rc;
-        if ((rc = run_linear(c, OP_U2, c->U1.p, c->HU, c->U2.p, c->HU, Nt, EPI_LRELU))) return rc;
-        if ((rc = run_linear(c, OP_U3, c->U2.p, c->HU, c->UOUT.p, F, Nt, EPI_LINEAR))) return rc;
-    }
-#ifdef DSAT_WITH_TCGEN05
-    else {
-        if (fusedp) {
-            if ((rc = run_fused(c, 3, OP_U3))) return rc;
-        } else {
-        if ((rc = run_linear_tc(c, OP_U1, Nt, tc::TC_LRELU, c->U1b.p, c->HU, true))) return rc;
-        if ((rc = run_linear_tc(c, OP_U2, Nt, tc::TC_LRELU, c->U2b.p, c->HU, true))) return rc;
-        if ((rc = run_linear_tc(c, OP_U3, Nt, tc::TC_LINEAR, c->UOUTb.p, F, true))) return rc;
-        }
-    }
-#endif
+    if ((rc = run_mlp(c, 3))) return rc;
     // variables PairNorm + residual + carry                                     (:279-280, :347)
     prof_mark(c, PROF_NORM_VAR);
     rc = dispatch_width(c, F, [&](auto v) {
         constexpr int V = decltype(v)::value;
         int grid = c->total_graphs < c->sm_count * 8 ? c->total_graphs : c->sm_count * 8;
         if (x3p) {
-#ifdef DSAT_WITH_TCGEN05
             if (!launch_pairnorm_smem<V>(c, c->var_seg.p, c->n, c->max_graph_vars, c->UOUT.p, F, 0, vrow_b(c), vplane, ldv,
                                          c->SPREp.p, (size_t)Nt * F, F))
-            pairnorm_kernel<V, float, float><<<grid, PN_WARPS * 32, 0, c->stream>>>(
-                c->var_seg.p, c->n_graphs, c->n, c->total_graphs, c->UOUT.p, F, 0, nullptr, ldv, nullptr, F,
-                vrow_b(c), vplane, c->SPREp.p, (size_t)Nt * F, skip);
-#endif
+                pairnorm_kernel<V, float, float><<<grid, PN_WARPS * 32, 0, c->stream>>>(
+                    c->var_seg.p, c->n_graphs, c->n, c->total_graphs, c->UOUT.p, F, 0, nullptr, ldv, nullptr, F,
+                    vrow_b(c), vplane, c->SPREp.p, (size_t)Nt * F, skip);
         } else if (!tcp)
             pairnorm_kernel<V, float, float><<<grid, PN_WARPS * 32, 0, c->stream>>>(
                 c->var_seg.p, c->n_graphs, c->n, c->total_graphs, c->UOUT.p, F, 0, c->VROW.p, ldv, c->SPRE.p, F,
                 nullptr, 0, nullptr, 0, skip);
-#ifdef DSAT_WITH_TCGEN05
         else
             pairnorm_bf16_kernel<32 * V><<<grid, PN_WARPS * 32, 0, c->stream>>>(
                 c->var_seg.p, c->n_graphs, c->n, c->total_graphs, c->UOUTb.p, F, 0, c->VROWb.p, ldv, c->SPREb.p, F, skip);
-#endif
     });
     if (rc) return rc;
     LAUNCHED(c);
     // variables_output MLP                                                       (:283)
-    if (x3p) {
-#ifdef DSAT_WITH_TCGEN05
-        if ((rc = run_x3(c, XO, OP_O2))) return rc;
-#endif
-    } else if (!tcp) {
-        if ((rc = run_linear(c, OP_O1, c->SPRE.p, F, c->O1.p, c->HO, Nt, EPI_LRELU))) return rc;
-        if ((rc = run_linear(c, OP_O2, c->O1.p, c->HO, c->LOGITS.p, DSAT_LOGIT_PAD, Nt, EPI_LINEAR))) return rc;
-    }
-#ifdef DSAT_WITH_TCGEN05
-    else {
-        if (fusedp) {
-            if ((rc = run_fused(c, 4, OP_O2))) return rc;
-        } else {
-        if ((rc = run_linear_tc(c, OP_O1, Nt, tc::TC_LRELU, c->O1b.p, c->HO, true))) return rc;
-        if ((rc = run_linear_tc(c, OP_O2, Nt, tc::TC_LINEAR, c->LOGITS.p, DSAT_LOGIT_PAD, false))) return rc;
-        }
-    }
-#endif
+    if ((rc = run_mlp(c, 4))) return rc;
     // logit map selection, SAT check, early exit                                 (:289-338)
     prof_mark(c, PROF_HEAD);
     head_kernel<<<c->total_graphs, 128, 0, c->stream>>>(g, c->total_graphs, c->group_graphs, c->LOGITS.p,
@@ -1216,10 +1125,7 @@ extern "C" {
 int dsat_version(void) { return 2; }
 
 int dsat_build_info(void) {
-    int flags = 0;
-#ifdef DSAT_WITH_TCGEN05
-    flags |= 1;
-#endif
+    int flags = 1;      // the tcgen05 paths are always compiled in
 #ifdef DSAT_ASSERT
     flags |= 2;
 #endif
@@ -1261,13 +1167,9 @@ void dsat_destroy(dsat_ctx* c) {
     free_buffers(c);
     for (auto& op : c->ops) {
         op.w.release(); op.b.release();
-#ifdef DSAT_WITH_TCGEN05
         op.w_bf16.release();
-#endif
     }
-#ifdef DSAT_WITH_TCGEN05
     for (auto& w : c->wx) w.release();
-#endif
     c->cl_rowptr.release(); c->cl_lit.release(); c->lit_rowptr.release(); c->lit_clause.release();
     c->batch_seg.release(); c->graph_group.release(); c->row_graph.release(); c->graph_elem0.release();
     c->var_seg.release(); c->clause_seg.release(); c->deg_w.release(); c->vdeg_w.release(); c->rev_w.release(); c->var_order.release();
@@ -1313,21 +1215,17 @@ int dsat_timer_end(dsat_ctx* c, float* ms) {
 
 long long dsat_launch_count(const dsat_ctx* c) { return c ? c->launches : 0; }
 
-#ifdef DSAT_WITH_TCGEN05
 // widths the x3 kernels tile: every layer at most 256 wide, or a single layer that is a multiple of 256
 static bool x3_supported(const dsat_ctx* c) {
     auto wide_ok = [](int n) { return n <= 256 || n % 256 == 0; };
     return c->HQ <= 256 && c->HC <= 256 && c->HU <= 256 && c->HO <= 256 && c->Q + c->F <= 256 && wide_ok(c->HL) && wide_ok(2 * c->Q);
 }
-#endif
 
 int dsat_get_precision(const dsat_ctx* c) { return c ? c->precision : DSAT_ERR_ARG; }
 
 int dsat_set_precision(dsat_ctx* c, int dtype) {
     if (!c) return DSAT_ERR_ARG;
-    if (dtype == DSAT_F32) { c->precision = dtype; return DSAT_OK; }
-#ifdef DSAT_WITH_TCGEN05
-    if (dtype == DSAT_BF16 || dtype == DSAT_BF16_UNFUSED) { c->precision = dtype; return DSAT_OK; }
+    if (dtype == DSAT_F32 || dtype == DSAT_BF16 || dtype == DSAT_BF16_UNFUSED) { c->precision = dtype; return DSAT_OK; }
     if (dtype == DSAT_F32_TC) {
         if (c->has_model && !x3_supported(c)) {
             c->err = "DSAT_F32_TC needs layer widths of at most 256 (feature_maps, query_maps <= 128); use DSAT_F32";
@@ -1336,8 +1234,7 @@ int dsat_set_precision(dsat_ctx* c, int dtype) {
         c->precision = dtype;
         return DSAT_OK;
     }
-#endif
-    c->err = "precision not available in this build";
+    c->err = "unknown precision";
     return DSAT_ERR_UNSUPPORTED;
 }
 
@@ -1367,19 +1264,15 @@ int dsat_set_model(dsat_ctx* c, int n_layers, const float* const* kernels, const
     CK_CUDA(c, cudaStreamSynchronize(c->stream));
     if (c->has_buffers && (c->F != F || c->Q != Q)) release_buffers(c);
     c->generation++;        // weight buffers are re-allocated
-#ifdef DSAT_WITH_TCGEN05
     // the whole-MLP plans hold the weight pointers and their TMA descriptors: rebuild them with the next launch
     c->has_tc_buffers = false; c->has_x3_buffers = false; c->fused_ready = false; c->x3_ready = false;
-#endif
     c->F = F; c->Q = Q;
     int rc = pack_weights(c, kernels, biases, in_dims, out_dims);
     if (rc) return rc;
-#ifdef DSAT_WITH_TCGEN05
     if ((rc = tc_pack_weights(c))) return rc;
     if ((rc = x3_pack_weights(c))) return rc;
     // widths the split-precision kernels do not tile run their Dense layers on the CUDA cores instead (same fp32 results)
     if (c->precision == DSAT_F32_TC && !x3_supported(c)) c->precision = DSAT_F32;
-#endif
     c->has_model = true;
     return DSAT_OK;
 }
@@ -1991,9 +1884,6 @@ int dsat_spmm(dsat_ctx* c, int direction, const void* x_dev, void* y_dev, int fe
 // see dsat_mlp_fused.cuh.  The activations must have been produced by a previous round.
 int dsat_profile_fused(dsat_ctx* c, int which, long long* counters16) {
     if (!c || !counters16 || which < 0 || which > 6) return DSAT_ERR_ARG;
-#ifndef DSAT_WITH_TCGEN05
-    return DSAT_ERR_UNSUPPORTED;
-#else
     CK_CUDA(c, cudaSetDevice(c->device));
     if (use_x3(c)) {    // the seven x3 launches (query, lit 1, lit 2, lit 3, clause, update, output): 9 counters, see dsat_mlp_x3.cuh
         int rc = ensure_x3_buffers(c);
@@ -2027,7 +1917,6 @@ int dsat_profile_fused(dsat_ctx* c, int which, long long* counters16) {
     d.release();
     CK_CUDA(c, e);
     return DSAT_OK;
-#endif
 }
 
 int dsat_profile_classes(void) { return PROF_CLASSES; }
@@ -2065,27 +1954,52 @@ int dsat_profile_rounds(dsat_ctx* c, int rounds, uint64_t seed, float* class_ms,
 }
 
 // ----------------------------------------------------------------------------------------- debug
-static int debug_buffer(dsat_ctx* c, int id, float** p, long long* rows, int* ld) {
+// Where a debug buffer lives in the active precision.  Its rows and ld are the same in every precision; the storage is
+// fp32, bf16, or hi/lo bf16 planes (the lo plane rows*ld elements after the hi plane at p), or none for a buffer the
+// precision does not hold (hidden activations that stay on-chip).
+enum DebugStore { STORE_NONE, STORE_F32, STORE_BF16, STORE_PLANES };
+struct DebugLoc { DebugStore store; void* p; };
+struct DebugBuf { long long rows; int ld; DebugLoc at; };
+
+static int debug_buffer(dsat_ctx* c, int id, DebugBuf* d) {
     const long long Nt = c->Nt, Mt = c->Mt;
+    auto f32 = [](void* p) { return DebugLoc{STORE_F32, p}; };
+    auto b16 = [](void* p) { return DebugLoc{STORE_BF16, p}; };
+    auto planes = [](void* p) { return DebugLoc{STORE_PLANES, p}; };
+    const DebugLoc none{STORE_NONE, nullptr};
+    struct Row { long long rows; int ld; DebugLoc simt, bf16, x3; };     // DSAT_F32, DSAT_BF16(_UNFUSED), DSAT_F32_TC
+    Row r;
     switch (id) {
-        case DSAT_BUF_VROW: *p = c->VROW.p; *rows = Nt; *ld = c->ldv(); break;
-        case DSAT_BUF_CROW: *p = c->CROW.p; *rows = Mt; *ld = c->ldc(); break;
-        case DSAT_BUF_H1: *p = c->H1.p; *rows = Nt; *ld = c->ldh1(); break;
-        case DSAT_BUF_H2: *p = c->H2.p; *rows = Nt; *ld = c->HL; break;
-        case DSAT_BUF_QS: *p = c->QS.p; *rows = Nt; *ld = 3 * c->Q; break;
-        case DSAT_BUF_LIT: *p = c->LIT.p; *rows = Nt; *ld = 2 * c->Q; break;
-        case DSAT_BUF_CH: *p = c->CH.p; *rows = Mt; *ld = c->HC; break;
-        case DSAT_BUF_COUT: *p = c->COUT.p; *rows = Mt; *ld = c->Q + c->F; break;
-        case DSAT_BUF_U1: *p = c->U1.p; *rows = Nt; *ld = c->HU; break;
-        case DSAT_BUF_U2: *p = c->U2.p; *rows = Nt; *ld = c->HU; break;
-        case DSAT_BUF_UOUT: *p = c->UOUT.p; *rows = Nt; *ld = c->F; break;
-        case DSAT_BUF_SPRE: *p = c->SPRE.p; *rows = Nt; *ld = c->F; break;
-        case DSAT_BUF_O1: *p = c->O1.p; *rows = Nt; *ld = c->HO; break;
-        case DSAT_BUF_LOGITS: *p = c->LOGITS.p; *rows = Nt; *ld = DSAT_LOGIT_PAD; break;
-        case DSAT_BUF_OUT: *p = c->OUT.p; *rows = Nt; *ld = 1; break;
-        case DSAT_BUF_X: *p = reinterpret_cast<float*>(c->X.p); *rows = Nt; *ld = 2; break;
+        case DSAT_BUF_VROW: r = {Nt, c->ldv(), f32(c->VROW.p), b16(c->VROWb.p), planes(c->VROWp.p)}; break;
+        case DSAT_BUF_CROW: r = {Mt, c->ldc(), f32(c->CROW.p), b16(c->CROWb.p), planes(c->CROWp.p)}; break;
+        case DSAT_BUF_H1: r = {Nt, c->ldh1(), f32(c->H1.p), none, none}; break;
+        case DSAT_BUF_H2: r = {Nt, c->HL, f32(c->H2.p), none, planes(c->H2p.p)}; break;
+        case DSAT_BUF_QS: r = {Nt, 3 * c->Q, f32(c->QS.p), b16(c->QSb.p), f32(c->QS.p)}; break;
+        case DSAT_BUF_LIT: r = {Nt, 2 * c->Q, f32(c->LIT.p), b16(c->LITb.p), f32(c->LIT.p)}; break;
+        case DSAT_BUF_CH: r = {Mt, c->HC, f32(c->CH.p), none, none}; break;
+        case DSAT_BUF_COUT: r = {Mt, c->Q + c->F, f32(c->COUT.p), b16(c->COUTb.p), f32(c->COUT.p)}; break;
+        case DSAT_BUF_U1: r = {Nt, c->HU, f32(c->U1.p), none, none}; break;
+        case DSAT_BUF_U2: r = {Nt, c->HU, f32(c->U2.p), none, none}; break;
+        case DSAT_BUF_UOUT: r = {Nt, c->F, f32(c->UOUT.p), b16(c->UOUTb.p), f32(c->UOUT.p)}; break;
+        case DSAT_BUF_SPRE: r = {Nt, c->F, f32(c->SPRE.p), b16(c->SPREb.p), planes(c->SPREp.p)}; break;
+        case DSAT_BUF_O1: r = {Nt, c->HO, f32(c->O1.p), none, none}; break;
+        case DSAT_BUF_LOGITS: r = {Nt, DSAT_LOGIT_PAD, f32(c->LOGITS.p), f32(c->LOGITS.p), f32(c->LOGITS.p)}; break;
+        case DSAT_BUF_OUT: r = {Nt, 1, f32(c->OUT.p), f32(c->OUT.p), f32(c->OUT.p)}; break;
+        case DSAT_BUF_X: r = {Nt, 2, f32(c->X.p), f32(c->X.p), f32(c->X.p)}; break;
         default: c->err = "unknown buffer id"; return DSAT_ERR_ARG;
     }
+    *d = {r.rows, r.ld, use_x3(c) ? r.x3 : use_tc(c) ? r.bf16 : r.simt};
+    return DSAT_OK;
+}
+
+// dsat_debug_read / dsat_debug_write: the buffers of the active precision, and where buffer `id` lives there
+static int debug_access(dsat_ctx* c, int id, long long count, DebugBuf* d) {
+    CK_CUDA(c, cudaSetDevice(c->device));
+    int rc = ensure_active_buffers(c);
+    if (rc || (rc = debug_buffer(c, id, d))) return rc;
+    if (d->at.store == STORE_NONE) { c->err = "the active precision does not hold this buffer (it stays on-chip)"; return DSAT_ERR_UNSUPPORTED; }
+    CK_ARG(c, count == d->rows * d->ld, "dsat_debug_read / dsat_debug_write: count must be rows*ld");
+    CK_CUDA(c, cudaStreamSynchronize(c->stream));
     return DSAT_OK;
 }
 
@@ -2093,99 +2007,44 @@ int dsat_debug_dims(const dsat_ctx* cc, int buffer, long long* rows, int* ld) {
     dsat_ctx* c = const_cast<dsat_ctx*>(cc);
     if (!c || !rows || !ld) return DSAT_ERR_ARG;
     CK_ARG(c, c->has_model && c->has_graph, "set the model and the graph first");
-    float* p;
-    return debug_buffer(c, buffer, &p, rows, ld);
+    DebugBuf d;
+    if (int rc = debug_buffer(c, buffer, &d)) return rc;
+    *rows = d.rows; *ld = d.ld;
+    return DSAT_OK;
 }
 
 int dsat_debug_read(dsat_ctx* c, int buffer, float* host_out, long long count) {
     if (!c || !host_out) return DSAT_ERR_ARG;
-    CK_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_active_buffers(c);
-    if (rc) return rc;
-    float* p; long long rows; int ld;
-    if ((rc = debug_buffer(c, buffer, &p, &rows, &ld))) return rc;
-    CK_ARG(c, count == rows * ld, "dsat_debug_read: count must be rows*ld");
-    CK_CUDA(c, cudaStreamSynchronize(c->stream));
-#ifdef DSAT_WITH_TCGEN05
-    if (use_x3(c)) {    // MLP inputs live as hi/lo planes, the hidden activations of the fused MLPs are never materialised
-        const __nv_bfloat16* src = nullptr;
-        switch (buffer) {
-            case DSAT_BUF_VROW: src = c->VROWp.p; break;
-            case DSAT_BUF_CROW: src = c->CROWp.p; break;
-            case DSAT_BUF_SPRE: src = c->SPREp.p; break;
-            case DSAT_BUF_H2: src = c->H2p.p; break;
-            case DSAT_BUF_H1: case DSAT_BUF_CH: case DSAT_BUF_U1: case DSAT_BUF_U2: case DSAT_BUF_O1:
-                c->err = "this buffer stays on-chip on the fp32-accurate tensor-core path";
-                return DSAT_ERR_UNSUPPORTED;
-            default: break;
-        }
-        if (src) {
-            std::vector<__nv_bfloat16> tmp((size_t)count * 2);
-            CK_CUDA(c, dsat_memcpy_sync(tmp.data(), src, (size_t)count * 4, cudaMemcpyDeviceToHost));
-            for (long long i = 0; i < count; ++i) host_out[i] = __bfloat162float(tmp[i]) + __bfloat162float(tmp[count + i]);
-            return DSAT_OK;
-        }
+    DebugBuf d;
+    if (int rc = debug_access(c, buffer, count, &d)) return rc;
+    if (d.at.store == STORE_F32) {
+        CK_CUDA(c, dsat_memcpy_sync(host_out, d.at.p, (size_t)count * sizeof(float), cudaMemcpyDeviceToHost));
+        return DSAT_OK;
     }
-    if (use_tc(c)) {    // on the tensor-core path these buffers live in bf16: convert for the caller
-        const __nv_bfloat16* src = nullptr;
-        switch (buffer) {
-            case DSAT_BUF_VROW: src = c->VROWb.p; break;
-            case DSAT_BUF_CROW: src = c->CROWb.p; break;
-            case DSAT_BUF_SPRE: src = c->SPREb.p; break;
-            case DSAT_BUF_QS: src = c->QSb.p; break;
-            case DSAT_BUF_LIT: src = c->LITb.p; break;
-            case DSAT_BUF_COUT: src = c->COUTb.p; break;
-            case DSAT_BUF_UOUT: src = c->UOUTb.p; break;
-            default: break;
-        }
-        if (src) {
-            std::vector<__nv_bfloat16> tmp((size_t)count);
-            CK_CUDA(c, dsat_memcpy_sync(tmp.data(), src, (size_t)count * 2, cudaMemcpyDeviceToHost));
-            for (long long i = 0; i < count; ++i) host_out[i] = __bfloat162float(tmp[i]);
-            return DSAT_OK;
-        }
-    }
-#endif
-    CK_CUDA(c, dsat_memcpy_sync(host_out, p, (size_t)count * sizeof(float), cudaMemcpyDeviceToHost));
+    const bool split = d.at.store == STORE_PLANES;
+    std::vector<__nv_bfloat16> tmp((size_t)count * (split ? 2 : 1));
+    CK_CUDA(c, dsat_memcpy_sync(tmp.data(), d.at.p, tmp.size() * 2, cudaMemcpyDeviceToHost));
+    for (long long i = 0; i < count; ++i)
+        host_out[i] = split ? __bfloat162float(tmp[i]) + __bfloat162float(tmp[count + i]) : __bfloat162float(tmp[i]);
     return DSAT_OK;
 }
 
 int dsat_debug_write(dsat_ctx* c, int buffer, const float* host_in, long long count) {
     if (!c || !host_in) return DSAT_ERR_ARG;
-    CK_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_active_buffers(c);
-    if (rc) return rc;
-    float* p; long long rows; int ld;
-    if ((rc = debug_buffer(c, buffer, &p, &rows, &ld))) return rc;
-    CK_ARG(c, count == rows * ld, "dsat_debug_write: count must be rows*ld");
-    CK_CUDA(c, cudaStreamSynchronize(c->stream));
-#ifdef DSAT_WITH_TCGEN05
-    if (use_x3(c)) {
-        __nv_bfloat16* dst = buffer == DSAT_BUF_VROW ? c->VROWp.p : buffer == DSAT_BUF_CROW ? c->CROWp.p
-                           : buffer == DSAT_BUF_SPRE ? c->SPREp.p : nullptr;
-        if (dst) {
-            std::vector<__nv_bfloat16> tmp((size_t)count * 2);
-            for (long long i = 0; i < count; ++i) {
-                const __nv_bfloat16 hi = __float2bfloat16(host_in[i]);
-                tmp[i] = hi;
-                tmp[count + i] = __float2bfloat16(host_in[i] - __bfloat162float(hi));
-            }
-            CK_CUDA(c, dsat_memcpy_sync(dst, tmp.data(), (size_t)count * 4, cudaMemcpyHostToDevice));
-            return DSAT_OK;
-        }
-        if (p == nullptr) { c->err = "this buffer stays on-chip on the fp32-accurate tensor-core path"; return DSAT_ERR_UNSUPPORTED; }
+    DebugBuf d;
+    if (int rc = debug_access(c, buffer, count, &d)) return rc;
+    if (d.at.store == STORE_F32) {
+        CK_CUDA(c, dsat_memcpy_sync(d.at.p, host_in, (size_t)count * sizeof(float), cudaMemcpyHostToDevice));
+        return DSAT_OK;
     }
-#endif
-    CK_CUDA(c, dsat_memcpy_sync(p, host_in, (size_t)count * sizeof(float), cudaMemcpyHostToDevice));
-#ifdef DSAT_WITH_TCGEN05
-    if (use_tc(c) && (buffer == DSAT_BUF_VROW || buffer == DSAT_BUF_CROW || buffer == DSAT_BUF_SPRE)) {   // keep the bf16 mirrors in step
-        __nv_bfloat16* dst = buffer == DSAT_BUF_VROW ? c->VROWb.p : buffer == DSAT_BUF_CROW ? c->CROWb.p : c->SPREb.p;
-        const long long tot = rows * ld;
-        mirror_cols_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, c->stream>>>(p, ld, dst, ld, rows, ld);
-        LAUNCHED(c);
-        CK_CUDA(c, cudaStreamSynchronize(c->stream));
+    const bool split = d.at.store == STORE_PLANES;
+    std::vector<__nv_bfloat16> tmp((size_t)count * (split ? 2 : 1));
+    for (long long i = 0; i < count; ++i) {     // round to nearest, as the kernels' __float2bfloat16_rn
+        const __nv_bfloat16 hi = __float2bfloat16(host_in[i]);
+        tmp[i] = hi;
+        if (split) tmp[count + i] = __float2bfloat16(host_in[i] - __bfloat162float(hi));
     }
-#endif
+    CK_CUDA(c, dsat_memcpy_sync(d.at.p, tmp.data(), tmp.size() * 2, cudaMemcpyHostToDevice));
     return DSAT_OK;
 }
 
@@ -2194,10 +2053,6 @@ int dsat_debug_write(dsat_ctx* c, int buffer, const float* host_in, long long co
 int dsat_tc_linear_test(dsat_ctx* c, int rows, int K, int N, const float* a_host, const float* w_host,
                         const float* bias_host, int epi, int out_bf16, float* out_host) {
     if (!c || !a_host || !w_host || !bias_host || !out_host) return DSAT_ERR_ARG;
-#ifndef DSAT_WITH_TCGEN05
-    c->err = "built without the tcgen05 path";
-    return DSAT_ERR_UNSUPPORTED;
-#else
     CK_ARG(c, rows > 0 && K > 0 && N > 0 && K % 16 == 0 && N % 16 == 0, "dsat_tc_linear_test: K and N must be multiples of 16");
     CK_ARG(c, epi != tc::TC_QUERY || N % 32 == 0, "query epilogue needs N % 32 == 0");
     CK_CUDA(c, cudaSetDevice(c->device));
@@ -2244,7 +2099,6 @@ int dsat_tc_linear_test(dsat_ctx* c, int rows, int K, int N, const float* a_host
     da.release(); dw.release(); db.release(); dout_b.release(); dout_f.release();
     CK_CUDA(c, e);
     return DSAT_OK;
-#endif
 }
 
 // Randomized rounding of the CURRENT diffusion state X alone (dsat_debug_write of DSAT_BUF_X first): X <- one-hot sample
@@ -2304,57 +2158,7 @@ int dsat_debug_mlp(dsat_ctx* c, int which) {
     if (!c || which < 0 || which > 4) return DSAT_ERR_ARG;
     CK_CUDA(c, cudaSetDevice(c->device));
     int rc = ensure_active_buffers(c);
-    if (rc) return rc;
-    const long long Nt = c->Nt, Mt = c->Mt;
-    const int F = c->F, Q = c->Q, ldv = c->ldv(), ldc = c->ldc(), ldh1 = c->ldh1();
-    (void)Mt; (void)ldc;
-#ifdef DSAT_WITH_TCGEN05
-    if (use_x3(c)) {
-        enum { XQ = 0, XL1, XL2, XL3, XC, XU, XO };
-        switch (which) {
-            case 0: rc = run_x3(c, XQ, OP_Q2); break;
-            case 1: rc = run_x3(c, XL1, OP_V1); if (!rc) rc = run_x3(c, XL2, OP_L2); if (!rc) rc = run_x3(c, XL3, OP_L3); break;
-            case 2: rc = run_x3(c, XC, OP_C2); break;
-            case 3: rc = run_x3(c, XU, OP_U3); break;
-            default: rc = run_x3(c, XO, OP_O2); break;
-        }
-    } else if (use_tc(c) && c->precision == DSAT_BF16 && c->fused_ready) {
-        static const int cls[5] = {OP_Q2, OP_L3, OP_C2, OP_U3, OP_O2};
-        rc = run_fused(c, which, cls[which]);
-    } else if (use_tc(c)) {
-        switch (which) {
-            case 0: rc = run_linear_tc(c, OP_V1, Nt, tc::TC_LRELU, c->H1b.p, ldh1, true);
-                    if (!rc) rc = run_linear_tc(c, OP_Q2, Nt, tc::TC_QUERY, c->QSb.p, 3 * Q, true); break;
-            case 1: rc = run_linear_tc(c, OP_V1, Nt, tc::TC_LRELU, c->H1b.p, ldh1, true);
-                    if (!rc) rc = run_linear_tc(c, OP_L2, Nt, tc::TC_LRELU, c->H2b.p, c->HL, true);
-                    if (!rc) rc = run_linear_tc(c, OP_L3, Nt, tc::TC_LINEAR, c->LITb.p, 2 * Q, true); break;
-            case 2: rc = run_linear_tc(c, OP_C1, Mt, tc::TC_LRELU, c->CHb.p, c->HC, true);
-                    if (!rc) rc = run_linear_tc(c, OP_C2, Mt, tc::TC_LINEAR, c->COUTb.p, Q + F, true); break;
-            case 3: rc = run_linear_tc(c, OP_U1, Nt, tc::TC_LRELU, c->U1b.p, c->HU, true);
-                    if (!rc) rc = run_linear_tc(c, OP_U2, Nt, tc::TC_LRELU, c->U2b.p, c->HU, true);
-                    if (!rc) rc = run_linear_tc(c, OP_U3, Nt, tc::TC_LINEAR, c->UOUTb.p, F, true); break;
-            default: rc = run_linear_tc(c, OP_O1, Nt, tc::TC_LRELU, c->O1b.p, c->HO, true);
-                     if (!rc) rc = run_linear_tc(c, OP_O2, Nt, tc::TC_LINEAR, c->LOGITS.p, DSAT_LOGIT_PAD, false); break;
-        }
-    } else
-#endif
-    {
-        switch (which) {
-            case 0: rc = run_linear(c, OP_V1, c->VROW.p, ldv, c->H1.p, ldh1, Nt, EPI_LRELU);
-                    if (!rc) rc = run_linear(c, OP_Q2, c->H1.p, ldh1, c->QS.p, 3 * Q, Nt, EPI_QUERY); break;
-            case 1: rc = run_linear(c, OP_V1, c->VROW.p, ldv, c->H1.p, ldh1, Nt, EPI_LRELU);
-                    if (!rc) rc = run_linear(c, OP_L2, c->H1.p + c->HQ, ldh1, c->H2.p, c->HL, Nt, EPI_LRELU);
-                    if (!rc) rc = run_linear(c, OP_L3, c->H2.p, c->HL, c->LIT.p, 2 * Q, Nt, EPI_LINEAR); break;
-            case 2: rc = run_linear(c, OP_C1, c->CROW.p, ldc, c->CH.p, c->HC, Mt, EPI_LRELU);
-                    if (!rc) rc = run_linear(c, OP_C2, c->CH.p, c->HC, c->COUT.p, Q + F, Mt, EPI_LINEAR); break;
-            case 3: rc = run_linear(c, OP_U1, c->VROW.p, ldv, c->U1.p, c->HU, Nt, EPI_LRELU);
-                    if (!rc) rc = run_linear(c, OP_U2, c->U1.p, c->HU, c->U2.p, c->HU, Nt, EPI_LRELU);
-                    if (!rc) rc = run_linear(c, OP_U3, c->U2.p, c->HU, c->UOUT.p, F, Nt, EPI_LINEAR); break;
-            default: rc = run_linear(c, OP_O1, c->SPRE.p, F, c->O1.p, c->HO, Nt, EPI_LRELU);
-                     if (!rc) rc = run_linear(c, OP_O2, c->O1.p, c->HO, c->LOGITS.p, DSAT_LOGIT_PAD, Nt, EPI_LINEAR); break;
-        }
-    }
-    if (rc) return rc;
+    if (rc || (rc = run_mlp(c, which))) return rc;
     CK_CUDA(c, cudaStreamSynchronize(c->stream));
     return DSAT_OK;
 }

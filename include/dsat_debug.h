@@ -51,14 +51,18 @@ int dsat_profile_rounds(dsat_ctx* ctx, int rounds, uint64_t seed, float* class_m
 int dsat_tc_linear_test(dsat_ctx* ctx, int rows, int K, int N, const float* a_host, const float* w_host,
                         const float* bias_host, int epi, int out_bf16, float* out_host);
 
-/* Build flags of the loaded library: bit 0 = tcgen05 paths compiled in, bit 1 = -DDSAT_ASSERT debug build (bounds checks). */
+/* Build flags of the loaded library: bit 0 = tcgen05 paths compiled in (always 1), bit 1 = -DDSAT_ASSERT debug build
+ * (bounds checks). */
 int dsat_build_info(void);
 
 /* Randomized rounding alone: X (DSAT_BUF_X, written with dsat_debug_write) <- one-hot sample drawn with the context's
  * sampling mode from the Philox stream (seed, step). */
 int dsat_debug_rounding(dsat_ctx* ctx, uint64_t seed, int step);
 
-/* Parity hooks: run the pieces of one model call separately and read/write activation buffers. */
+/* Parity hooks: run the pieces of one model call separately and read/write activation buffers.  dsat_debug_read /
+ * dsat_debug_write convert between the caller's fp32 and the buffer's storage in the active precision (fp32, bf16, or
+ * hi + lo bf16 planes); a buffer the precision does not hold (hidden activations that stay on-chip) returns
+ * DSAT_ERR_UNSUPPORTED.  dsat_debug_dims answers for every buffer. */
 int dsat_debug_begin(dsat_ctx* ctx, float noise_scale, const float* noisy_num, const int32_t* labels);
 int dsat_debug_round(dsat_ctx* ctx, int round, const float* normals /* [N,4] host */);
 int dsat_debug_dims(const dsat_ctx* ctx, int buffer, long long* rows, int* ld);
