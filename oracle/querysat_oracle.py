@@ -16,6 +16,7 @@ function here                   reference file:line
 ``mlp``                         ``model/mlp.py:23-24,39,42-50``
 ``pair_norm``                   ``layers/normalization.py:43-71``, graph-norm matrices
                                 ``model/query_sat.py:206-211``
+``degree_weights``              ``model/query_sat.py:193-197``
 ``softplus_loss_adj``           ``loss/sat.py:125-137``
 ``train_loss``                  ``model/query_sat.py:40-53`` (+ TFP Bernoulli KL, external)
 ``distribution_at_time``        ``model/query_sat.py:66-68``
@@ -183,6 +184,19 @@ def train_loss(labels, logits, noise_scale, label_smoothing=0.01):
     return loss / (norm + 1e-4)
 
 
+def degree_weights(graph: OracleGraph, dtype):
+    """``model/query_sat.py:193-197``: literal degrees [2N,1], clause sizes [M,1], ``degree_weight`` [2N,1],
+    ``var_degree_weight`` [N,1] and ``rev_degree_weight`` [M,1]."""
+    n, m = graph.n_vars, graph.n_clauses
+    ones_e = torch.ones(graph.lit_row.shape[0], dtype=dtype)
+    lit_degree = torch.zeros(2 * n, dtype=dtype).index_add_(0, graph.lit_row, ones_e)[:, None]
+    rev_lit_degree = torch.zeros(m, dtype=dtype).index_add_(0, graph.clause, ones_e)[:, None]
+    degree_weight = torch.rsqrt(torch.clamp(lit_degree, min=1))
+    var_degree_weight = 4 * torch.rsqrt(torch.clamp(lit_degree[:n] + lit_degree[n:], min=1))
+    rev_degree_weight = torch.rsqrt(torch.clamp(rev_lit_degree, min=1))
+    return lit_degree, rev_lit_degree, degree_weight, var_degree_weight, rev_degree_weight
+
+
 def is_batch_sat(out_logits, graph: OracleGraph):
     variables = torch.round(torch.sigmoid(out_logits))          # half-to-even, as tf.round
     literals = torch.cat([variables, 1 - variables], dim=0)
@@ -214,12 +228,7 @@ def model_loop(graph: OracleGraph, w, noise_scale, noisy_num, labels, normals, r
     q = w["variables_query"][-1][0].shape[1]
     ns = torch.as_tensor(noise_scale, dtype=dtype)
 
-    ones_e = torch.ones(graph.lit_row.shape[0], dtype=dtype)
-    lit_degree = torch.zeros(2 * n, dtype=dtype).index_add_(0, graph.lit_row, ones_e)[:, None]
-    degree_weight = torch.rsqrt(torch.clamp(lit_degree, min=1))
-    var_degree_weight = 4 * torch.rsqrt(torch.clamp(lit_degree[:n] + lit_degree[n:], min=1))
-    rev_lit_degree = torch.zeros(m, dtype=dtype).index_add_(0, graph.clause, ones_e)[:, None]
-    rev_degree_weight = torch.rsqrt(torch.clamp(rev_lit_degree, min=1))
+    _, _, degree_weight, var_degree_weight, rev_degree_weight = degree_weights(graph, dtype)
 
     var_w = graph_norm_weights(graph.var_graph, g_cnt, dtype)
 

@@ -14,7 +14,7 @@ from tests import helpers as H
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("precision,tol", [(_lib.F32, 1e-3), (_lib.BF16, 8e-2)])
+@pytest.mark.parametrize("precision,tol", [(_lib.F32_TC, 1e-3), (_lib.F32, 1e-3), (_lib.BF16, 8e-2)])
 def test_uf250_shape_model_call(ctx, precision, tol):
     n_vars, m, chains, rounds = 250, 1065, 3, 4
     _, clauses = synth.random_3sat(n_vars, m, seed=250)
