@@ -59,6 +59,8 @@ _SIGNATURES = {
     "dsat_words_per_graph": (C.c_int, [_vp]),
     "dsat_hist_reduce": (C.c_int, [_vp, C.c_int, _u64p, C.POINTER(C.c_int64), C.c_int, _i32p, _i32p]),
     "dsat_hist_reduce_segments": (C.c_int, [_vp, C.c_int, _i32p, _i32p, _u64p, C.POINTER(C.c_int64), C.c_int, _i32p, _i32p]),
+    "dsat_enumerate_models": (C.c_int, [_vp, C.c_int, C.c_int, C.c_longlong, _i32p, _i32p, _u64p, C.c_longlong,
+                                        C.POINTER(C.c_longlong)]),
     "dsat_spmm": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_int]),
     "dsat_profile_classes": (C.c_int, []),
     "dsat_profile_fused": (C.c_int, [_vp, C.c_int, C.POINTER(C.c_longlong)]),
@@ -317,6 +319,24 @@ class Context:
                                                         _ptr(keys, C.c_uint64), counts.ctypes.data_as(C.POINTER(C.c_int64)),
                                                         cap, _ptr(runs, C.c_int32), C.byref(n_sat)))
         return [(keys[runs[s]:runs[s + 1]], counts[runs[s]:runs[s + 1]]) for s in range(n_seg)], int(n_sat.value)
+
+    def enumerate_models(self, n_vars: int, clauses, count_only: bool = False):
+        """Every model of the formula (``dsat_enumerate_models``): ``uint64 [K]`` ascending by the integer each encodes
+        (x1 = bit 0), or with ``count_only`` the number of models.  ``clauses``: lists of signed 1-based literals."""
+        lens = np.fromiter(map(len, clauses), dtype=np.int32, count=len(clauses))
+        flat = np.fromiter((l for c in clauses for l in c), dtype=np.int32, count=int(lens.sum(dtype=np.int64)))
+        cap = 0 if count_only else 1 << 16         # one call for up to 65536 models, a second one with the exact size above
+        while True:
+            out = np.empty(cap, dtype=np.uint64)
+            n = C.c_longlong(0)
+            rc = self._lib.dsat_enumerate_models(self._h, int(n_vars), int(lens.shape[0]), int(flat.shape[0]),
+                                                 _ptr(lens, C.c_int32), _ptr(flat, C.c_int32),
+                                                 _ptr(out, C.c_uint64) if cap else None, cap, C.byref(n))
+            if rc != 0 and cap and n.value > cap:
+                cap = n.value
+                continue
+            self._check(rc)
+            return int(n.value) if count_only else out[:n.value]
 
     def spmm(self, direction: int, x_dev_ptr: int, y_dev_ptr: int, feat: int, dtype: int, chains: int):
         self._check(self._lib.dsat_spmm(self._h, int(direction), _vp(x_dev_ptr), _vp(y_dev_ptr), int(feat), int(dtype),

@@ -20,6 +20,7 @@
 #include "dsat_graph_host.cuh"
 #include "dsat_norm_head.cuh"
 #include "dsat_hist.cuh"
+#include "dsat_models.cuh"
 #include "dsat_gemm_tc.cuh"
 #include "dsat_mlp_fused.cuh"
 #include "dsat_mlp_x3.cuh"
@@ -126,6 +127,10 @@ struct dsat_ctx {
     // histogram reduction scratch (dsat_hist.cuh)
     DevBuf<int> hist_idx, hist_run, hist_totals, hist_seg, hist_run_seg;
     DevBuf<unsigned long long> hist_keys, hist_counts;
+    // model enumeration scratch (dsat_models.cuh); no other state of the context is touched by dsat_enumerate_models
+    DevBuf<models::Clause> enum_clauses;
+    DevBuf<unsigned> enum_block_models;
+    DevBuf<unsigned long long> enum_offsets, enum_total, enum_out;
     // injected noise staging
     DevBuf<float> inj_normals, inj_uniforms, inj_noisy;
     DevBuf<int> inj_labels;
@@ -472,6 +477,8 @@ void free_buffers(dsat_ctx* c) {
     c->inj_normals.release(); c->inj_uniforms.release(); c->inj_noisy.release(); c->inj_labels.release();
     c->hist_idx.release(); c->hist_run.release(); c->hist_totals.release(); c->hist_keys.release(); c->hist_counts.release();
     c->hist_seg.release(); c->hist_run_seg.release();
+    c->enum_clauses.release(); c->enum_block_models.release(); c->enum_offsets.release(); c->enum_total.release();
+    c->enum_out.release();
     c->VROWb.release(); c->CROWb.release(); c->H1b.release(); c->H2b.release(); c->QSb.release(); c->LITb.release();
     c->CHb.release(); c->COUTb.release(); c->UOUTb.release(); c->U1b.release(); c->U2b.release(); c->SPREb.release();
     c->O1b.release();
@@ -1777,6 +1784,89 @@ int dsat_hist_reduce_segments(dsat_ctx* c, int n_segments, const int32_t* graph_
         CK_CUDA(c, cudaStreamSynchronize(c->stream));
     }
     CK_ARG(c, K <= capacity, "dsat_hist_reduce_segments: capacity too small (seg_runs[n_segments] holds the required size)");
+    return DSAT_OK;
+}
+
+// ------------------------------------------------------------------------------- model enumeration
+int dsat_enumerate_models(dsat_ctx* c, int n_vars, int n_clauses, long long nnz, const int32_t* lens, const int32_t* flat,
+                          uint64_t* models_out, long long capacity, long long* n_models) {
+    if (!c) return DSAT_ERR_ARG;
+    if (n_models) *n_models = 0;
+    CK_ARG(c, n_models && capacity >= 0 && (capacity == 0 || models_out), "dsat_enumerate_models: null output");
+    CK_ARG(c, n_vars >= 1 && n_vars <= 63, "dsat_enumerate_models: n_vars must be in 1..63");
+    CK_ARG(c, n_clauses >= 0 && nnz >= 0 && (n_clauses == 0 || lens) && (nnz == 0 || flat),
+           "dsat_enumerate_models: negative size or null clause array");
+    long long total = 0;
+    for (int j = 0; j < n_clauses; ++j) {
+        CK_ARG(c, lens[j] >= 0, "dsat_enumerate_models: negative clause length");
+        total += lens[j];
+    }
+    CK_ARG(c, total == nnz, "dsat_enumerate_models: clause lengths do not sum to nnz");
+    // values of variables 1..6 over the 64 lanes: variable v is true in the lanes whose bit v is set
+    static const unsigned long long var_lanes[6] = {0xAAAAAAAAAAAAAAAAull, 0xCCCCCCCCCCCCCCCCull, 0xF0F0F0F0F0F0F0F0ull,
+                                                    0xFF00FF00FF00FF00ull, 0xFFFF0000FFFF0000ull, 0xFFFFFFFF00000000ull};
+    std::vector<models::Clause> cls(n_clauses);
+    bool empty_clause = false;
+    for (long long j = 0, e = 0; j < n_clauses; e += lens[j], ++j) {
+        models::Clause k{0ull, 0ull, 0ull};
+        for (long long q = e; q < e + lens[j]; ++q) {
+            const int lit = flat[q];
+            const long long var = (lit < 0 ? -(long long)lit : lit) - 1;
+            if (lit == 0 || var >= n_vars) {
+                c->err = "dsat_enumerate_models: literal " + std::to_string(lit) + " of clause " + std::to_string(j) +
+                         " is 0 or beyond n_vars";
+                return DSAT_ERR_ARG;
+            }
+            if (var < 6) k.lane_sat |= lit > 0 ? var_lanes[var] : ~var_lanes[var];
+            else if (lit > 0) k.pos_hi |= 1ull << (var - 6);
+            else k.neg_hi |= 1ull << (var - 6);
+        }
+        empty_clause |= lens[j] == 0;
+        cls[j] = k;
+    }
+    if (empty_clause) return DSAT_OK;       // no assignment satisfies an empty clause (VariableAssignment.satisfiable)
+    CK_CUDA(c, cudaSetDevice(c->device));
+    const int low = n_vars < 6 ? n_vars : 6;                                // lanes that exist: 2^low
+    const unsigned long long lane_mask = low == 6 ? ~0ull : (1ull << (1 << low)) - 1;
+    const unsigned long long h_count = 1ull << (n_vars - low), h_chunk = 1ull << (models::CHUNK_LOG2 - 6);
+    const unsigned long long max_blocks = ((h_count < h_chunk ? h_count : h_chunk) + models::H_PER_BLOCK - 1) / models::H_PER_BLOCK;
+    CK_CUDA(c, c->enum_clauses.alloc(n_clauses > 0 ? n_clauses : 1));
+    CK_CUDA(c, c->enum_block_models.alloc(max_blocks));
+    CK_CUDA(c, c->enum_offsets.alloc(max_blocks));
+    CK_CUDA(c, c->enum_total.alloc(1));
+    if (n_clauses > 0)
+        CK_CUDA(c, cudaMemcpyAsync(c->enum_clauses.p, cls.data(), n_clauses * sizeof(models::Clause), cudaMemcpyHostToDevice,
+                                   c->stream));
+    unsigned long long found = 0, written = 0;
+    for (unsigned long long h0 = 0; h0 < h_count; h0 += h_chunk) {
+        const unsigned long long h_end = h_count - h0 < h_chunk ? h_count : h0 + h_chunk;
+        const unsigned blocks = (unsigned)((h_end - h0 + models::H_PER_BLOCK - 1) / models::H_PER_BLOCK);
+        models::count_kernel<<<blocks, models::THREADS, 0, c->stream>>>(c->enum_clauses.p, n_clauses, lane_mask, h0, h_end,
+                                                                        c->enum_block_models.p);
+        LAUNCHED(c);
+        models::scan_kernel<<<1, models::SCAN_THREADS, 0, c->stream>>>(c->enum_block_models.p, (int)blocks, c->enum_offsets.p,
+                                                                        c->enum_total.p);
+        LAUNCHED(c);
+        unsigned long long chunk_models = 0;
+        CK_CUDA(c, cudaMemcpyAsync(&chunk_models, c->enum_total.p, sizeof(chunk_models), cudaMemcpyDeviceToHost, c->stream));
+        CK_CUDA(c, cudaStreamSynchronize(c->stream));
+        const unsigned long long room = (unsigned long long)capacity - written;
+        const unsigned long long take = chunk_models < room ? chunk_models : room;
+        if (take > 0) {
+            CK_CUDA(c, c->enum_out.alloc(take));
+            models::emit_kernel<<<blocks, models::THREADS, 0, c->stream>>>(c->enum_clauses.p, n_clauses, lane_mask, h0, h_end,
+                                                                           c->enum_offsets.p, take, c->enum_out.p);
+            LAUNCHED(c);
+            CK_CUDA(c, cudaMemcpyAsync(models_out + written, c->enum_out.p, take * sizeof(uint64_t), cudaMemcpyDeviceToHost,
+                                       c->stream));
+            CK_CUDA(c, cudaStreamSynchronize(c->stream));
+            written += take;
+        }
+        found += chunk_models;
+    }
+    *n_models = (long long)found;
+    CK_ARG(c, found <= (unsigned long long)capacity || (capacity == 0 && !models_out),
+           "dsat_enumerate_models: capacity too small (n_models holds the required size)");
     return DSAT_OK;
 }
 

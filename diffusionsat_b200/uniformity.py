@@ -1,12 +1,41 @@
-"""Uniformity statistics of a sample histogram (host side, scipy).
+"""Uniformity statistics of a sample histogram (host side, scipy) and the exact model set they compare against.
 
 Mirror of reference ``utils/chi_square.py:7-36`` (``chi_square_likelihood``) and of the comparison made in
-``diffusion_metrics.py:111,130-147`` (histogram against the ideal ``k`` samples per solution).
+``diffusion_metrics.py:111,130-147`` (histogram against the ideal ``k`` samples per solution).  The model set comes from
+:func:`enumerate_models` (GPU brute force, ``dsat_enumerate_models``), which replaces the reference's unigen/approxmc
+counting (``utils/AllSolutions.py:44-68``).
 """
 
 from __future__ import annotations
 
 from scipy import stats
+
+MAX_ENUMERATION_VARS = 63
+
+
+def _models_call(n_vars, clauses, count_only, context, device):
+    if not 1 <= int(n_vars) <= MAX_ENUMERATION_VARS:
+        raise ValueError("exact model enumeration takes 1..%d variables, got %d" % (MAX_ENUMERATION_VARS, n_vars))
+    from . import _lib
+    ctx = context if context is not None else _lib.Context(device)
+    try:
+        return ctx.enumerate_models(int(n_vars), [list(c) for c in clauses], count_only=count_only)
+    finally:
+        if context is None:
+            ctx.close()
+
+
+def enumerate_models(n_vars: int, clauses, *, context=None, device: int = 0):
+    """Every model of a formula over ``n_vars <= 63`` variables as ``uint64`` integers in the reference encoding (x1 = bit
+    0), ascending; the same list as ``synth.enumerate_solutions`` for any size the GPU can go through (2^n assignments).
+    ``context``: a ``_lib.Context`` to run on (its model, graph and sampling state are left as they are); otherwise a
+    context on ``device`` is created for the call."""
+    return _models_call(n_vars, clauses, False, context, device)
+
+
+def count_models(n_vars: int, clauses, *, context=None, device: int = 0) -> int:
+    """Number of models of the formula (:func:`enumerate_models` without writing them out)."""
+    return _models_call(n_vars, clauses, True, context, device)
 
 
 def chi_square_likelihood(observed: dict, expected: dict) -> float:

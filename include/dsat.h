@@ -170,6 +170,18 @@ int dsat_hist_reduce(dsat_ctx* ctx, int chain_limit, uint64_t* keys_out, int64_t
 int dsat_hist_reduce_segments(dsat_ctx* ctx, int n_segments, const int32_t* graph_seg, const int32_t* limit,
                               uint64_t* keys_out, int64_t* counts_out, int capacity, int32_t* seg_runs, int32_t* n_sat);
 
+/* Every model of a formula over n_vars <= 63 variables, in ascending order of the integer it encodes (x1 = bit 0), by brute
+ * force over all 2^n_vars assignments on the device (at most 2^36 per launch).  Clauses are given as in dsat_graph_build:
+ * lens[j] signed 1-based literals for clause j, laid end to end in flat; an empty clause leaves no model, repeated literals
+ * and tautologies count as in utils/VariableAssignment.py:79-90, and a variable in no clause is free.
+ * models_out == NULL with capacity 0 counts only.  *n_models = number of models; when capacity is too small, the first
+ * capacity models are written and the call returns DSAT_ERR_ARG with *n_models = the required capacity (as dsat_hist_reduce
+ * does).  Every argument is checked before any device work (a literal of magnitude 0 or > n_vars, n_vars outside 1..63, lens
+ * that do not sum to nnz, a null output).  Leaves the context's model, graph, precision and sampling state untouched.
+ * Replaces the unigen/approxmc counting of utils/AllSolutions.py:44-68. */
+int dsat_enumerate_models(dsat_ctx* ctx, int n_vars, int n_clauses, long long nnz, const int32_t* lens,
+                          const int32_t* flat, uint64_t* models_out, long long capacity, long long* n_models);
+
 #ifdef __cplusplus
 }
 #endif
