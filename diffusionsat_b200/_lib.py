@@ -61,6 +61,8 @@ _SIGNATURES = {
     "dsat_hist_reduce_segments": (C.c_int, [_vp, C.c_int, _i32p, _i32p, _u64p, C.POINTER(C.c_int64), C.c_int, _i32p, _i32p]),
     "dsat_enumerate_models": (C.c_int, [_vp, C.c_int, C.c_int, C.c_longlong, _i32p, _i32p, _u64p, C.c_longlong,
                                         C.POINTER(C.c_longlong)]),
+    "dsat_enumerate_models_search": (C.c_int, [_vp, C.c_int, C.c_int, C.c_longlong, _i32p, _i32p, _u64p, C.c_longlong,
+                                               C.POINTER(C.c_longlong)]),
     "dsat_spmm": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_int]),
     "dsat_profile_classes": (C.c_int, []),
     "dsat_profile_fused": (C.c_int, [_vp, C.c_int, C.POINTER(C.c_longlong)]),
@@ -332,6 +334,26 @@ class Context:
             rc = self._lib.dsat_enumerate_models(self._h, int(n_vars), int(lens.shape[0]), int(flat.shape[0]),
                                                  _ptr(lens, C.c_int32), _ptr(flat, C.c_int32),
                                                  _ptr(out, C.c_uint64) if cap else None, cap, C.byref(n))
+            if rc != 0 and cap and n.value > cap:
+                cap = n.value
+                continue
+            self._check(rc)
+            return int(n.value) if count_only else out[:n.value]
+
+    def enumerate_models_search(self, n_vars: int, clauses, count_only: bool = False):
+        """Every model of the formula by ordered search (``dsat_enumerate_models_search``, 1 <= n_vars <= 1024):
+        ``uint64 [K, ceil(n_vars / 64)]``, word 0 = variables 1..64, ascending by the integer each encodes, or with
+        ``count_only`` the number of models.  A count above 2^63 - 1 raises DsatError."""
+        lens = np.fromiter(map(len, clauses), dtype=np.int32, count=len(clauses))
+        flat = np.fromiter((l for c in clauses for l in c), dtype=np.int32, count=int(lens.sum(dtype=np.int64)))
+        words = (max(int(n_vars), 1) + 63) // 64
+        cap = 0 if count_only else 1 << 16         # one call for up to 65536 models, a second one with the exact size above
+        while True:
+            out = np.empty((cap, words), dtype=np.uint64)
+            n = C.c_longlong(0)
+            rc = self._lib.dsat_enumerate_models_search(self._h, int(n_vars), int(lens.shape[0]), int(flat.shape[0]),
+                                                        _ptr(lens, C.c_int32), _ptr(flat, C.c_int32),
+                                                        _ptr(out, C.c_uint64) if cap else None, cap, C.byref(n))
             if rc != 0 and cap and n.value > cap:
                 cap = n.value
                 continue

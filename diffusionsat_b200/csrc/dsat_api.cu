@@ -21,6 +21,7 @@
 #include "dsat_norm_head.cuh"
 #include "dsat_hist.cuh"
 #include "dsat_models.cuh"
+#include "dsat_model_search.cuh"
 #include "dsat_gemm_tc.cuh"
 #include "dsat_mlp_fused.cuh"
 #include "dsat_mlp_x3.cuh"
@@ -131,6 +132,11 @@ struct dsat_ctx {
     DevBuf<models::Clause> enum_clauses;
     DevBuf<unsigned> enum_block_models;
     DevBuf<unsigned long long> enum_offsets, enum_total, enum_out;
+    // model search scratch (dsat_model_search.cuh); no other state of the context is touched by dsat_enumerate_models_search
+    DevBuf<int> search_off;
+    DevBuf<unsigned short> search_lit;
+    DevBuf<unsigned long long> search_frontier[2], search_counts, search_offsets, search_total, search_out;
+    DevBuf<unsigned> search_flags;      // [0] node cursor of the search kernels, [1] branching nodes of a level
     // injected noise staging
     DevBuf<float> inj_normals, inj_uniforms, inj_noisy;
     DevBuf<int> inj_labels;
@@ -479,6 +485,9 @@ void free_buffers(dsat_ctx* c) {
     c->hist_seg.release(); c->hist_run_seg.release();
     c->enum_clauses.release(); c->enum_block_models.release(); c->enum_offsets.release(); c->enum_total.release();
     c->enum_out.release();
+    c->search_off.release(); c->search_lit.release(); c->search_frontier[0].release(); c->search_frontier[1].release();
+    c->search_counts.release(); c->search_offsets.release(); c->search_total.release(); c->search_out.release();
+    c->search_flags.release();
     c->VROWb.release(); c->CROWb.release(); c->H1b.release(); c->H2b.release(); c->QSb.release(); c->LITb.release();
     c->CHb.release(); c->COUTb.release(); c->UOUTb.release(); c->U1b.release(); c->U2b.release(); c->SPREb.release();
     c->O1b.release();
@@ -1867,6 +1876,156 @@ int dsat_enumerate_models(dsat_ctx* c, int n_vars, int n_clauses, long long nnz,
     *n_models = (long long)found;
     CK_ARG(c, found <= (unsigned long long)capacity || (capacity == 0 && !models_out),
            "dsat_enumerate_models: capacity too small (n_models holds the required size)");
+    return DSAT_OK;
+}
+
+int dsat_enumerate_models_search(dsat_ctx* c, int n_vars, int n_clauses, long long nnz, const int32_t* lens,
+                                 const int32_t* flat, uint64_t* models_out, long long capacity, long long* n_models) {
+    if (!c) return DSAT_ERR_ARG;
+    if (n_models) *n_models = 0;
+    CK_ARG(c, n_models && capacity >= 0 && (capacity == 0 || models_out), "dsat_enumerate_models_search: null output");
+    CK_ARG(c, n_vars >= 1 && n_vars <= msearch::MAX_VARS, "dsat_enumerate_models_search: n_vars must be in 1..1024");
+    CK_ARG(c, n_clauses >= 0 && nnz >= 0 && (n_clauses == 0 || lens) && (nnz == 0 || flat),
+           "dsat_enumerate_models_search: negative size or null clause array");
+    long long total = 0;
+    for (int j = 0; j < n_clauses; ++j) {
+        CK_ARG(c, lens[j] >= 0, "dsat_enumerate_models_search: negative clause length");
+        total += lens[j];
+    }
+    CK_ARG(c, total == nnz, "dsat_enumerate_models_search: clause lengths do not sum to nnz");
+    // Normalise: a clause holds when one of its literals does (utils/VariableAssignment.py:79-90), so repeated literals
+    // are kept once and a clause with x and not x, which holds everywhere, is dropped.
+    std::vector<int> off(1, 0);
+    std::vector<unsigned short> lits;
+    std::vector<unsigned char> seen(2 * (size_t)n_vars, 0);
+    bool empty_clause = false;
+    for (long long j = 0, e = 0; j < n_clauses; e += lens[j], ++j) {
+        const size_t start = lits.size();
+        bool tautology = false;
+        for (long long q = e; q < e + lens[j]; ++q) {
+            const int lit = flat[q];
+            const long long var = (lit < 0 ? -(long long)lit : lit) - 1;
+            if (lit == 0 || var >= n_vars) {
+                c->err = "dsat_enumerate_models_search: literal " + std::to_string(lit) + " of clause " + std::to_string(j) +
+                         " is 0 or beyond n_vars";
+                return DSAT_ERR_ARG;
+            }
+            const unsigned code = (unsigned)var << 1 | (lit < 0);
+            tautology |= seen[code ^ 1u] != 0;
+            if (!seen[code]) { seen[code] = 1; lits.push_back((unsigned short)code); }
+        }
+        for (size_t q = start; q < lits.size(); ++q) seen[lits[q]] = 0;
+        empty_clause |= lens[j] == 0;
+        if (tautology) lits.resize(start);
+        else if (lits.size() > start) off.push_back((int)lits.size());
+    }
+    if (empty_clause) return DSAT_OK;       // no assignment satisfies an empty clause (VariableAssignment.satisfiable)
+    CK_CUDA(c, cudaSetDevice(c->device));
+    const int m = (int)off.size() - 1, words = (n_vars + 63) / 64, node_words = 2 * words;
+    const long long lit_count = (long long)lits.size();
+    const long long clause_bytes = msearch::clause_smem_bytes(m, lit_count);
+    const int stage = clause_bytes <= msearch::CLAUSE_SMEM_MAX;
+    const size_t smem = (size_t)(stage ? clause_bytes : 0) + (size_t)msearch::WARPS * msearch::warp_smem_bytes(n_vars);
+    CK_CUDA(c, cudaFuncSetAttribute(msearch::expand_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK_CUDA(c, cudaFuncSetAttribute(msearch::expand_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK_CUDA(c, cudaFuncSetAttribute(msearch::search_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK_CUDA(c, cudaFuncSetAttribute(msearch::search_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    CK_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, msearch::search_kernel<false>, msearch::THREADS, smem));
+    const int resident_blocks = (per_sm > 0 ? per_sm : 1) * c->sm_count;
+    const int frontier_cap = 2 * msearch::FRONTIER_TARGET;
+    CK_CUDA(c, c->search_off.alloc(off.size()));
+    CK_CUDA(c, c->search_lit.alloc(lits.empty() ? 1 : lits.size()));
+    CK_CUDA(c, c->search_frontier[0].alloc((size_t)frontier_cap * node_words));
+    CK_CUDA(c, c->search_frontier[1].alloc((size_t)frontier_cap * node_words));
+    CK_CUDA(c, c->search_counts.alloc(frontier_cap));
+    CK_CUDA(c, c->search_offsets.alloc(frontier_cap));
+    CK_CUDA(c, c->search_total.alloc(1));
+    CK_CUDA(c, c->search_flags.alloc(2));
+    CK_CUDA(c, cudaMemcpyAsync(c->search_off.p, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    if (!lits.empty())
+        CK_CUDA(c, cudaMemcpyAsync(c->search_lit.p, lits.data(), lits.size() * sizeof(unsigned short), cudaMemcpyHostToDevice,
+                                   c->stream));
+    // the root: nothing assigned; the bits of `set` at and above n_vars are 1 so that they never count as unassigned
+    std::vector<unsigned long long> root(node_words, 0ull);
+    for (int w = 0; w < words; ++w) {
+        const int lo = w * 64;
+        root[w] = n_vars >= lo + 64 ? 0ull : ~0ull << (n_vars - lo);
+    }
+    CK_CUDA(c, cudaMemcpyAsync(c->search_frontier[0].p, root.data(), node_words * sizeof(unsigned long long),
+                               cudaMemcpyHostToDevice, c->stream));
+    const msearch::Formula F{c->search_off.p, c->search_lit.p, m, n_vars, words};
+    auto blocks_for = [&](long long nodes) {
+        const long long b = (nodes + msearch::WARPS - 1) / msearch::WARPS;
+        return (unsigned)(b < resident_blocks ? b : resident_blocks);
+    };
+
+    // 1. breadth-first frontier, in depth-first order when the models are written out (a count needs no order)
+    const int ordered = capacity > 0;
+    int cur = 0, n_nodes = 1;
+    for (int level = 0; level < msearch::MAX_LEVELS && n_nodes < msearch::FRONTIER_TARGET; ++level) {
+        CK_CUDA(c, cudaMemsetAsync(c->search_flags.p, 0, 2 * sizeof(unsigned), c->stream));
+        msearch::expand_kernel<false><<<blocks_for(n_nodes), msearch::THREADS, smem, c->stream>>>(
+            F, stage, lit_count, ordered, c->search_frontier[cur].p, n_nodes, c->search_counts.p, c->search_flags.p + 1,
+            nullptr, nullptr, 0);
+        LAUNCHED(c);
+        msearch::scan_kernel<<<1, msearch::SCAN_THREADS, 0, c->stream>>>(c->search_counts.p, n_nodes, c->search_offsets.p,
+                                                                         c->search_total.p);
+        LAUNCHED(c);
+        unsigned long long kids = 0;
+        unsigned branching = 0;
+        CK_CUDA(c, cudaMemcpyAsync(&kids, c->search_total.p, sizeof(kids), cudaMemcpyDeviceToHost, c->stream));
+        CK_CUDA(c, cudaMemcpyAsync(&branching, c->search_flags.p + 1, sizeof(branching), cudaMemcpyDeviceToHost, c->stream));
+        CK_CUDA(c, cudaStreamSynchronize(c->stream));
+        if (branching == 0) break;          // no node branches (leaves, kept nodes, a conflicting root): the frontier stays
+        msearch::expand_kernel<true><<<blocks_for(n_nodes), msearch::THREADS, smem, c->stream>>>(
+            F, stage, lit_count, ordered, c->search_frontier[cur].p, n_nodes, nullptr, nullptr, c->search_offsets.p,
+            c->search_frontier[cur ^ 1].p, frontier_cap);
+        LAUNCHED(c);
+        cur ^= 1;
+        n_nodes = (int)kids;                // at most twice a frontier below FRONTIER_TARGET
+        if (n_nodes == 0) break;
+    }
+
+    // 2. depth-first search below each frontier node, CHUNK_NODES nodes per launch
+    unsigned long long found = 0, written = 0;
+    for (int n0 = 0; n0 < n_nodes; n0 += msearch::CHUNK_NODES) {
+        const int cnt = n_nodes - n0 < msearch::CHUNK_NODES ? n_nodes - n0 : msearch::CHUNK_NODES;
+        const unsigned long long* nodes = c->search_frontier[cur].p + (size_t)n0 * node_words;
+        CK_CUDA(c, cudaMemsetAsync(c->search_flags.p, 0, sizeof(unsigned), c->stream));
+        msearch::search_kernel<false><<<blocks_for(cnt), msearch::THREADS, smem, c->stream>>>(
+            F, stage, lit_count, nodes, cnt, c->search_flags.p, c->search_counts.p, nullptr, 0, nullptr);
+        LAUNCHED(c);
+        msearch::scan_kernel<<<1, msearch::SCAN_THREADS, 0, c->stream>>>(c->search_counts.p, cnt, c->search_offsets.p,
+                                                                         c->search_total.p);
+        LAUNCHED(c);
+        unsigned long long chunk_models = 0;
+        CK_CUDA(c, cudaMemcpyAsync(&chunk_models, c->search_total.p, sizeof(chunk_models), cudaMemcpyDeviceToHost, c->stream));
+        CK_CUDA(c, cudaStreamSynchronize(c->stream));
+        found = msearch::sat_add(found, chunk_models);
+        if (found == msearch::SAT) {
+            *n_models = -1;
+            c->err = "dsat_enumerate_models_search: more than 2^63 - 1 models";
+            return DSAT_ERR_UNSUPPORTED;
+        }
+        const unsigned long long room = (unsigned long long)capacity - written;
+        const unsigned long long take = chunk_models < room ? chunk_models : room;
+        if (take > 0) {
+            CK_CUDA(c, c->search_out.alloc(take * words));
+            CK_CUDA(c, cudaMemsetAsync(c->search_flags.p, 0, sizeof(unsigned), c->stream));
+            msearch::search_kernel<true><<<blocks_for(cnt), msearch::THREADS, smem, c->stream>>>(
+                F, stage, lit_count, nodes, cnt, c->search_flags.p, c->search_counts.p, c->search_offsets.p, take,
+                c->search_out.p);
+            LAUNCHED(c);
+            CK_CUDA(c, cudaMemcpyAsync(models_out + written * words, c->search_out.p, take * words * sizeof(uint64_t),
+                                       cudaMemcpyDeviceToHost, c->stream));
+            CK_CUDA(c, cudaStreamSynchronize(c->stream));
+            written += take;
+        }
+    }
+    *n_models = (long long)found;
+    CK_ARG(c, found <= (unsigned long long)capacity || (capacity == 0 && !models_out),
+           "dsat_enumerate_models_search: capacity too small (n_models holds the required size)");
     return DSAT_OK;
 }
 

@@ -38,6 +38,35 @@ def count_models(n_vars: int, clauses, *, context=None, device: int = 0) -> int:
     return _models_call(n_vars, clauses, True, context, device)
 
 
+MAX_SEARCH_VARS = 1024
+
+
+def _search_call(n_vars, clauses, count_only, context, device):
+    if not 1 <= int(n_vars) <= MAX_SEARCH_VARS:
+        raise ValueError("model search takes 1..%d variables, got %d" % (MAX_SEARCH_VARS, n_vars))
+    from . import _lib
+    ctx = context if context is not None else _lib.Context(device)
+    try:
+        return ctx.enumerate_models_search(int(n_vars), [list(c) for c in clauses], count_only=count_only)
+    finally:
+        if context is None:
+            ctx.close()
+
+
+def enumerate_models_by_search(n_vars: int, clauses, *, context=None, device: int = 0):
+    """Every model of a formula over ``n_vars <= 1024`` variables by ordered search on the GPU
+    (``dsat_enumerate_models_search``): ``uint64 [K, ceil(n_vars / 64)]``, word 0 = variables 1..64 (the layout of the
+    sampler's keys; ``dist.keys_to_ints`` turns them into ints), ascending.  For ``n_vars <= 63`` the same models as
+    :func:`enumerate_models`.  Its cost follows the search tree (which skips every subtree with a failed clause), not
+    2^n.  ``context`` and ``device`` as in :func:`enumerate_models`."""
+    return _search_call(n_vars, clauses, False, context, device)
+
+
+def count_models_by_search(n_vars: int, clauses, *, context=None, device: int = 0) -> int:
+    """Number of models of the formula (:func:`enumerate_models_by_search` without writing them out)."""
+    return _search_call(n_vars, clauses, True, context, device)
+
+
 def chi_square_likelihood(observed: dict, expected: dict) -> float:
     """p-value of the chi-square test of ``observed`` against ``expected`` (dicts id -> count).
     Ids missing on one side count as zero there; a single shared id is reported as p = 1."""

@@ -182,6 +182,20 @@ int dsat_hist_reduce_segments(dsat_ctx* ctx, int n_segments, const int32_t* grap
 int dsat_enumerate_models(dsat_ctx* ctx, int n_vars, int n_clauses, long long nnz, const int32_t* lens,
                           const int32_t* flat, uint64_t* models_out, long long capacity, long long* n_models);
 
+/* The models dsat_enumerate_models finds, in the same ascending order, for 1 <= n_vars <= 1024, by a search on the device
+ * instead of the brute force: it branches on the highest unassigned variable, 0 before 1, propagates unit clauses and
+ * skips every subtree with a clause that fails, so its cost follows the search tree rather than 2^n_vars.  Counting does not
+ * branch on variables that no open clause holds (a variable in no clause among them): they multiply the count, so count-only
+ * calls and overflows stay fast; writing the models out branches on them, at a cost that follows the models written.
+ * Each model is `words` = ceil(n_vars / 64) 64-bit words, word 0 = variables 1..64 (the layout of dsat_sample's packed and
+ * dsat_hist_reduce's keys); models_out is [capacity, words].  Clauses, count-only mode (models_out == NULL, capacity 0), the
+ * capacity rule and the argument checks are those of dsat_enumerate_models, with n_vars outside 1..1024 refused.  A count
+ * above 2^63 - 1 returns DSAT_ERR_UNSUPPORTED with *n_models = -1.  Leaves the context's model, graph, precision and sampling
+ * state untouched. */
+int dsat_enumerate_models_search(dsat_ctx* ctx, int n_vars, int n_clauses, long long nnz, const int32_t* lens,
+                                 const int32_t* flat, uint64_t* models_out /* [capacity, words] */, long long capacity,
+                                 long long* n_models);
+
 #ifdef __cplusplus
 }
 #endif

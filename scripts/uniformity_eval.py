@@ -1,5 +1,6 @@
 """Uniformity evaluation of the sampler on one formula (SURVEY.md section 8f-2): exact model set on the GPU
-(uniformity.enumerate_models, in place of the reference's unigen/approxmc counting, utils/AllSolutions.py:44-68), `k`
+(uniformity.enumerate_models up to 63 variables, uniformity.enumerate_models_by_search above, in place of the reference's
+unigen/approxmc counting, utils/AllSolutions.py:44-68), `k`
 samples per model as in diffusion_metrics.py:111, chi-square against the ideal uniform histogram (utils/chi_square.py).
 
   python scripts/uniformity_eval.py formula.cnf [weights.npz] [k] [--precision fp32|fp32_simt|bf16]
@@ -12,7 +13,9 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 from diffusionsat_b200.dimacs import DimacsFile
 from diffusionsat_b200.sampler import DiffusionSampler
-from diffusionsat_b200.uniformity import chi_square_likelihood, chi_square_vs_ideal, enumerate_models
+from diffusionsat_b200.dist import keys_to_ints
+from diffusionsat_b200.uniformity import (MAX_ENUMERATION_VARS, chi_square_likelihood, chi_square_vs_ideal, enumerate_models,
+                                          enumerate_models_by_search)
 
 
 def main():
@@ -25,7 +28,11 @@ def main():
     df = DimacsFile(filename=args.cnf)
     df.load()
     sampler = DiffusionSampler(args.weights, args.cnf, precision=args.precision)
-    models = enumerate_models(df.number_of_vars(), df.clauses(), context=sampler.ctx).tolist()
+    n = df.number_of_vars()
+    if n <= MAX_ENUMERATION_VARS:
+        models = enumerate_models(n, df.clauses(), context=sampler.ctx).tolist()
+    else:       # the histogram's keys are ints of the same packed words (sampler.samples -> dist.keys_to_ints)
+        models = keys_to_ints(enumerate_models_by_search(n, df.clauses(), context=sampler.ctx), n)
     print("models:", len(models))
     hist = sampler.samples(len(models) * args.k)
     model_set = set(models)
